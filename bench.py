@@ -2,6 +2,7 @@
 """Headline benchmark of the B200 retrieval core (contract: see the task statement / DESIGN.md section 6).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-knn] [--no-c4] [--no-c5]
+                  [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic input at BASELINE.json configs[1]
 (C2): quantise 1,000,000 SIFT-like 128-D descriptors against a k=4096 codebook (fused tcgen05
@@ -475,6 +476,22 @@ def run_c5(args, torch, dist, dev, rank, world, barrier, max_over_ranks, ops, P)
 # ----------------------------------------------------------------------------------------------
 # GPU arm
 # ----------------------------------------------------------------------------------------------
+DUMP_ROWS = 1024         # image rows of the step's [10k x 4096] float64 result that --dump-outputs keeps: 32 MiB
+
+
+def dump_outputs(out_dir, tf, codebook):
+    """Writes what the last timed step returned, for comparing two builds output for output: the same DUMP_ROWS image
+    rows (fixed seed, ascending) of the Okapi tf matrix, whose 328 MB are too many to keep whole, and the codebook the
+    step quantised against.  The codebook is trained on the device during set-up, so a difference there explains a
+    difference in the rows."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    rows = np.sort(np.random.default_rng(7).choice(tf.shape[0], DUMP_ROWS, replace=False))
+    sample = tf.index_select(0, torch.from_numpy(rows).to(tf.device)).cpu().numpy()
+    np.save(os.path.join(out_dir, "okapi_tf_rows.npy"), sample)
+    np.save(os.path.join(out_dir, "codebook.npy"), np.asarray(codebook, dtype=np.float32))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -566,12 +583,16 @@ def run_ours(args):
     kernel_events.clear()
     t_start, t_end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t_start.record()
-    for i in range(args.steps):
+    for _ in range(args.steps - 1):
         device_step()
+    last = device_step()
     t_end.record()
     barrier()
     launches = ops.launches() - l0
     ms_step = max_over_ranks(t_start.elapsed_time(t_end) / args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last, km.cluster_centers_)
+    del last
     # all gemm_select launches of a step (main launch + any fallback re-run) count towards the kernel time
     kern_ms = float(np.sum([a.elapsed_time(b) for a, b in kernel_events]) / args.steps)
     assign_stats = ops.search_stats()
@@ -960,7 +981,13 @@ def main():
     ap.add_argument("--no-c4", action="store_true")
     ap.add_argument("--no-c5", action="store_true")
     ap.add_argument("--c4-iters", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (rank 0, --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
