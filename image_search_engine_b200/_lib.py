@@ -72,6 +72,19 @@ PROTOTYPES = {
                                 _c_void_p, _c_void_p, _i64, _c_void_p, _c_void_p,
                                 _i64, _i64, _int, _int, _i64, _c_void_p, _int,
                                 _c_void_p, _c_void_p, _c_void_p, _c_void_p]),
+    "ise_range_seed": (_int, [_c_void_p, _c_void_p, _c_void_p, _c_void_p, _c_void_p, _i64, _int, _int, C.c_float,
+                              _c_void_p, _c_void_p]),
+    "ise_range_count": (_int, [_c_void_p, _c_void_p, _int, _i64, _c_void_p, _i64, _i64, _i64, _int, _int, C.c_float,
+                               _i64, _c_void_p, _c_void_p, _int, _c_void_p, _c_void_p, _c_void_p, _c_void_p, _c_void_p]),
+    "ise_range_lims_workspace_bytes": (_size, [_c_void_p, _i64]),
+    "ise_range_lims": (_int, [_c_void_p, _c_void_p, _i64, _i64, _c_void_p, _c_void_p, _size, _c_void_p]),
+    "ise_range_fill": (_int, [_c_void_p, _i64, _int, _c_void_p, _c_void_p, _c_void_p, _c_void_p, _c_void_p, _c_void_p,
+                              _c_void_p, _c_void_p]),
+    "ise_range_sort_workspace_bytes": (_size, [_c_void_p, _i64, _i64]),
+    "ise_range_sort": (_int, [_c_void_p, _i64, _c_void_p, _i64, _c_void_p, _c_void_p, _c_void_p, _size, _c_void_p]),
+    "ise_scores_range_workspace_bytes": (_size, [_c_void_p, _i64, _i64]),
+    "ise_scores_range": (_int, [_c_void_p, _c_void_p, _i64, _i64, _int, C.c_float, _i64, _i64, _c_void_p, _c_void_p,
+                                _c_void_p, _c_void_p, _size, _c_void_p]),
     "ise_topk_merge": (_int, [_c_void_p, _c_void_p, _c_void_p, _int, _i64, _int, _int, _c_void_p, _c_void_p,
                               _c_void_p]),
     "ise_kmeans_accumulate": (_int, [_c_void_p, _c_void_p, _int, _i64, _int, _i64, _c_void_p, _c_void_p,

@@ -190,6 +190,30 @@ class IndexFlat:
             D, I = Dp, Ip
         return D, I
 
+    def range_search(self, x, radius: float):
+        """faiss IndexFlat::range_search: every stored vector scoring better than ``radius`` (IP: > radius, L2: squared
+        distance < radius; strict, in FP32).  Returns (lims [nq + 1], D, I): the results of query i are
+        D[lims[i]:lims[i+1]] / I[...] in ascending id.  NumPy input gives NumPy output (lims uint64, like Faiss's
+        size_t array); CUDA tensors give CUDA tensors (lims int64)."""
+        q, was_cuda = _to_device(x)
+        if q.shape[1] != self.d:
+            raise AssertionError(f"range_search: expected (n, {self.d}) array")
+        lims, D, I = self._range_search_device(q, radius)
+        if was_cuda:
+            return lims, D, I
+        return lims.cpu().numpy().astype(np.uint64), D.cpu().numpy(), I.cpu().numpy()
+
+    def _range_search_device(self, q: torch.Tensor, radius: float):
+        nq = q.shape[0]
+        if self._ntotal == 0 or nq == 0:
+            return ops._range_empty(nq, q.device)
+        if nq < distance_compute_blas_threshold:
+            qf = q if q.dtype == torch.float32 else q.to(torch.float32)
+            return ops.range_search_exact(qf.contiguous(), self._database(), self.metric_type, radius)
+        b = self._operand()
+        a = ops.prepare_operand(q, rows=True)
+        return ops.range_search(q, a, self._database(), b, self.metric_type, radius)
+
     def assign(self, x, k: int = 1):
         return self.search(x, k)[1]
 

@@ -501,6 +501,178 @@ def search_topk(q_raw: torch.Tensor, a_op: Operand, db_raw: torch.Tensor, b_op: 
     return D, I
 
 
+# ------------------------------------------------------------------------------------------
+# range search (Faiss IndexFlat::range_search)
+# ------------------------------------------------------------------------------------------
+RANGE_CAP = 256                   # candidate slots per query of the first collect; rows beyond it are re-run
+RANGE_BUDGET_BYTES = 1 << 30      # candidate buffers (m x cap x 12 B) of one query chunk / one overflow batch
+
+
+def _rows_slice(op: Operand, r0: int, r1: int) -> Operand:
+    """Rows [r0, r1) of an operand as views (no copy)."""
+    return Operand(op.hi[r0:r1], None if op.lo is None else op.lo[r0:r1], op.norms[r0:r1], op.meta, r1 - r0, op.d,
+                   op.ldp, row_inv=None if op.row_inv is None else op.row_inv[r0:r1])
+
+
+def _range_lims(kept: torch.Tensor, m: int, base: int = 0) -> torch.Tensor:
+    """lims [m + 1] int64 = base + exclusive scan of kept [m + 1] (kept[m] == 0)."""
+    lib, ctx = _lib.load(), _lib.ctx(_dev(kept))
+    lims = torch.empty((m + 1,), dtype=torch.int64, device=kept.device)
+    ws = torch.empty((int(lib.ise_range_lims_workspace_bytes(ctx, m)),), dtype=torch.uint8, device=kept.device)
+    _lib.check(lib.ise_range_lims(ctx, _ptr(kept), m, int(base), _ptr(lims), _ptr(ws), ws.numel(), _stream()))
+    _count()
+    return lims
+
+
+def _range_candidates(q_raw, db_raw, a: Operand, b: Operand, metric: int, radius: float, seed, cap: int, id_base: int):
+    """Collect over the hi planes + exact filter.  Returns (cand_val, cand_idx, row_count, kept [m + 1])."""
+    cv, ci, rc = gemm_collect(a.hi_only(), b.hi_only(), metric, seed, cap, id_base)
+    kept = torch.empty((a.n + 1,), dtype=torch.int64, device=cv.device)
+    _lib.check(_lib.load().ise_range_count(
+        _lib.ctx(_dev(cv)), _ptr(q_raw), DTYPE_F32 if q_raw.dtype == torch.float32 else DTYPE_U8, q_raw.stride(0),
+        _ptr(db_raw), db_raw.stride(0), a.n, db_raw.shape[0], a.d, int(metric), radius, int(id_base), _ptr(a.norms),
+        _ptr(b.norms), int(cap), _ptr(rc), _ptr(cv), _ptr(ci), _ptr(kept), _stream()))
+    _count()
+    return cv, ci, rc, kept
+
+
+def _range_fill(m, cap, rc, cv, ci, row_map, lims, D, I):
+    _lib.check(_lib.load().ise_range_fill(_lib.ctx(_dev(cv)), m, int(cap), _ptr(rc), _ptr(cv), _ptr(ci), _ptr(row_map),
+                                          _ptr(lims), _ptr(D), _ptr(I), _stream()))
+    _count()
+
+
+def _range_concat(parts, nq: int, device):
+    """Joins per-chunk (kept [m + 1], lims [m + 1], D, I) results (chunks in query order)."""
+    if len(parts) == 1:
+        _, lims, D, I = parts[0]
+        return lims, D, I
+    kept = torch.cat([p[0][:-1] for p in parts] + [torch.zeros((1,), dtype=torch.int64, device=device)])
+    return _range_lims(kept, nq), torch.cat([p[2] for p in parts]), torch.cat([p[3] for p in parts])
+
+
+def _range_empty(nq: int, device):
+    return (torch.zeros((nq + 1,), dtype=torch.int64, device=device), torch.empty((0,), dtype=torch.float32, device=device),
+            torch.empty((0,), dtype=torch.int64, device=device))
+
+
+def range_search(q_raw: torch.Tensor, a_op: Operand, db_raw: torch.Tensor, b_op: Operand, metric: int, radius: float,
+                 id_base: int = 0, _cap: int = RANGE_CAP):
+    """Every database row whose exact FP32 score beats ``radius`` (IP: > radius, L2: squared distance < radius), for
+    every query row (the tensor-core path, nq >= 20).  Returns (lims int64 [nq + 1], D float32 [lims[nq]],
+    I int64 [lims[nq]]) on the device; the results of query i are D / I[lims[i]:lims[i+1]], in ascending id.
+
+    One coarse product over the FP16 hi planes collects every column that beats the radius loosened by the rigorous
+    coarse error bound (ise_range_seed), so the candidate set is complete by construction; the candidates are
+    re-scored exactly in FP32 and filtered with the strict test.  The per-query candidate counts are read back once;
+    queries with more than ``_cap`` candidates are collected again with a buffer sized to their count."""
+    nq = a_op.n
+    dev = q_raw.device
+    radius = float(np.float32(radius))
+    if q_raw.dtype not in (torch.float32, torch.uint8) or q_raw.stride(1) != 1:
+        raise IseError("range_search: query rows must be float32 or uint8, row-major")
+    if db_raw.dtype != torch.float32 or db_raw.stride(1) != 1:
+        raise IseError("range_search: database rows must be float32, row-major")
+    if a_op.d != b_op.d:
+        raise IseError(f"dimension mismatch {a_op.d} vs {b_op.d}")
+    if nq == 0 or b_op.n == 0:
+        last_search_stats.update(mode="range", rows=nq, candidates=0, overflow_rows=0, results=0, fallback_rows=0)
+        return _range_empty(nq, dev)
+    lib, ctx = _lib.load(), _lib.ctx(_dev(q_raw))
+    seed = torch.empty((nq,), dtype=torch.float32, device=dev)
+    _lib.check(lib.ise_range_seed(ctx, _ptr(a_op.meta), _ptr(a_op.norms), _ptr(a_op.row_inv), _ptr(b_op.meta), nq,
+                                  a_op.d, int(metric), radius, _ptr(seed), _stream()))
+    _count()
+    chunk = max(1, RANGE_BUDGET_BYTES // (12 * _cap))
+    parts, n_cand, n_over = [], 0, 0
+    for q0 in range(0, nq, chunk):
+        q1 = min(nq, q0 + chunk)
+        m = q1 - q0
+        cv, ci, rc, kept = _range_candidates(q_raw[q0:q1], db_raw, _rows_slice(a_op, q0, q1), b_op, metric, radius,
+                                             seed[q0:q1], _cap, id_base)
+        rc_h = rc[:m].cpu().numpy().astype(np.int64)          # the one readback of the candidate counts
+        over = np.nonzero(rc_h > _cap)[0]
+        n_cand += int(np.minimum(rc_h, _cap).sum())
+        n_over += int(over.size)
+        reruns = []
+        if over.size:
+            # overflowing queries again, largest first, in batches whose buffers fit the budget (cap = largest count)
+            over = over[np.argsort(-rc_h[over], kind="stable")]
+            i0 = 0
+            while i0 < over.size:
+                cap2 = int(rc_h[over[i0]])
+                i1 = min(over.size, i0 + max(1, RANGE_BUDGET_BYTES // (12 * cap2)))
+                sel = torch.from_numpy(over[i0:i1]).to(dev)
+                gsel = sel + q0
+                cv2, ci2, rc2, kept2 = _range_candidates(q_raw.index_select(0, gsel), db_raw, a_op.rows(gsel), b_op,
+                                                         metric, radius, seed.index_select(0, gsel), cap2, id_base)
+                got = int(rc2.max().item())
+                if got > cap2:
+                    raise IseError(f"range_search: a re-run query found {got} candidates, more than the {cap2} its "
+                                   "first pass counted")
+                kept.index_copy_(0, sel, kept2[:-1])
+                n_cand += int(rc_h[over[i0:i1]].sum())
+                reruns.append((sel, cap2, rc2, cv2, ci2))
+                i0 = i1
+        lims = _range_lims(kept, m)
+        total = int(lims[m].item())
+        D = torch.empty((total,), dtype=torch.float32, device=dev)
+        I = torch.empty((total,), dtype=torch.int64, device=dev)
+        if total:
+            _range_fill(m, _cap, rc, cv, ci, None, lims, D, I)
+            for sel, cap2, rc2, cv2, ci2 in reruns:
+                _range_fill(sel.numel(), cap2, rc2, cv2, ci2, sel, lims, D, I)
+            ws = torch.empty((int(lib.ise_range_sort_workspace_bytes(ctx, m, total)),), dtype=torch.uint8, device=dev)
+            _lib.check(lib.ise_range_sort(ctx, m, _ptr(lims), total, _ptr(D), _ptr(I), _ptr(ws), ws.numel(), _stream()))
+            _count(2)
+        parts.append((kept, lims, D, I))
+    lims, D, I = _range_concat(parts, nq, dev)
+    last_search_stats.update(mode="range", rows=nq, candidates=n_cand, overflow_rows=n_over, results=int(D.numel()),
+                             fallback_rows=0)
+    return lims, D, I
+
+
+def range_search_exact(q: torch.Tensor, db: torch.Tensor, metric: int, radius: float, id_base: int = 0,
+                       max_score_bytes: int = 1 << 30):
+    """Range search with Faiss's direct per-pair formulas (its nq < 20 regime): exact FP32 pair scores of a query chunk
+    (ise_pair_scores), then counts, offsets and the results in column order (ise_scores_range).  Same return as
+    range_search."""
+    if q.dtype != torch.float32 or db.dtype != torch.float32 or not q.is_contiguous() or not db.is_contiguous():
+        raise IseError("range_search_exact needs contiguous float32 tensors")
+    nq, d = q.shape
+    nb = db.shape[0]
+    radius = float(np.float32(radius))
+    if nq == 0 or nb == 0:
+        last_search_stats.update(mode="range-exact", rows=nq, results=0, fallback_rows=0)
+        return _range_empty(nq, q.device)
+    lib, ctx = _lib.load(), _lib.ctx(_dev(q))
+    chunk = int(max(1, min(nq, 65535, max_score_bytes // (4 * nb))))
+    parts, base = [], 0
+    for q0 in range(0, nq, chunk):
+        qs = q[q0:q0 + chunk]
+        n = qs.shape[0]
+        scores = torch.empty((n, nb), dtype=torch.float32, device=q.device)
+        _lib.check(lib.ise_pair_scores(ctx, _ptr(qs), n, _ptr(db), nb, d, int(metric), _ptr(scores), _stream()))
+        ws = torch.empty((int(lib.ise_scores_range_workspace_bytes(ctx, n, nb)),), dtype=torch.uint8, device=q.device)
+        lims = torch.empty((n + 1,), dtype=torch.int64, device=q.device)
+        _lib.check(lib.ise_scores_range(ctx, _ptr(scores), n, nb, int(metric), radius, int(id_base), base, _ptr(lims),
+                                        None, None, _ptr(ws), ws.numel(), _stream()))
+        total = int(lims[n].item()) - base
+        D = torch.empty((total,), dtype=torch.float32, device=q.device)
+        I = torch.empty((total,), dtype=torch.int64, device=q.device)
+        if total:
+            _lib.check(lib.ise_scores_range(ctx, _ptr(scores), n, nb, int(metric), radius, int(id_base), base,
+                                            _ptr(lims), _ptr(D), _ptr(I), _ptr(ws), ws.numel(), _stream()))
+        _count(6 if total else 4)
+        parts.append((lims, D, I))
+        base += total
+    lims = parts[0][0] if len(parts) == 1 else torch.cat([p[0][:-1] for p in parts] + [parts[-1][0][-1:]])
+    D = parts[0][1] if len(parts) == 1 else torch.cat([p[1] for p in parts])
+    I = parts[0][2] if len(parts) == 1 else torch.cat([p[2] for p in parts])
+    last_search_stats.update(mode="range-exact", rows=nq, results=int(D.numel()), fallback_rows=0)
+    return lims, D, I
+
+
 def flat_search_exact(q: torch.Tensor, db: torch.Tensor, metric: int, topk: int, id_base: int = 0):
     """Exact FP32 CUDA-core search (Faiss's n < 20 path)."""
     if q.dtype != torch.float32 or db.dtype != torch.float32 or not q.is_contiguous() or not db.is_contiguous():

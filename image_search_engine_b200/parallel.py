@@ -153,6 +153,14 @@ class DeviceOps:
     def merge(self, D_parts, I_parts, metric):
         return ops.topk_merge(D_parts, I_parts, metric)
 
+    def range_search(self, q, q_op, db, b_op, metric, radius, id_base):
+        """local range search -> (lims int64 [nq + 1], D, I) with global ids, ascending within a query; fewer than 20
+        queries take the direct-formula path like the unsharded IndexFlat"""
+        if q.shape[0] < 20:
+            qf = q if q.dtype == torch.float32 else q.to(torch.float32)
+            return ops.range_search_exact(qf.contiguous(), db, metric, radius, id_base=id_base)
+        return ops.range_search(q, q_op, db, b_op, metric, radius, id_base=id_base)
+
 
 def _world(group):
     if not dist.is_available() or not dist.is_initialized():
@@ -457,3 +465,47 @@ class ShardedIndexFlat:
         D_out = full[:nq, :, 2].contiguous().view(torch.float32)
         self.last_exchange_bytes = int(send.numel() * 4 * (world - 1) // world + full.numel() * 4 * (world - 1) // world)
         return D_out, I_out
+
+    def range_search(self, q, radius):
+        """q replicated on every rank.  Returns (lims int64 [nq + 1], D, I) identical on every rank and equal to the
+        unsharded IndexFlat.range_search: each query's results are rank 0's, then rank 1's, ... -- shards are contiguous
+        and ascending, so ids stay ascending.
+
+        Exchange: one all-gather of the per-query result counts ([world, nq] int64), then one all-gather of every
+        rank's packed (id, dis) results, padded to the largest rank's total."""
+        rank, world = _world(self.group)
+        qd = self.lops.to_local(q)
+        nq = int(qd.shape[0])
+        dev = qd.device
+        if self._local is None or self._local.shape[0] == 0 or nq == 0:
+            # a rank that owns no rows still takes part in the exchange, with no results
+            lims = torch.zeros((nq + 1,), dtype=torch.int64, device=dev)
+            D = torch.empty((0,), dtype=torch.float32, device=dev)
+            I = torch.empty((0,), dtype=torch.int64, device=dev)
+        else:
+            lims, D, I = self.lops.range_search(qd, self.lops.prepare(qd, rows=True), self._local, self._b_op,
+                                                self.metric_type, radius, self.id_base)
+        if world == 1:
+            return lims, D, I
+        counts = torch.empty((world * nq,), dtype=torch.int64, device=dev)
+        dist.all_gather_into_tensor(counts, (lims[1:] - lims[:-1]).contiguous(), group=self.group)
+        C = counts.cpu().numpy().reshape(world, nq)
+        totals = C.sum(axis=1)
+        pad = max(int(totals.max()), 1)
+        send = torch.zeros((pad, 3), dtype=torch.int32, device=dev)
+        n_mine = int(D.shape[0])
+        send[:n_mine, :2] = I.contiguous().view(torch.int32).view(n_mine, 2)
+        send[:n_mine, 2] = D.contiguous().view(torch.int32)
+        full = torch.empty((world * pad, 3), dtype=torch.int32, device=dev)
+        dist.all_gather_into_tensor(full, send, group=self.group)
+        # payload order is (rank, query, id); a stable sort by query gives (query, rank, id)
+        query_of = np.concatenate([np.repeat(np.arange(nq, dtype=np.int64), C[r]) for r in range(world)])
+        src = np.concatenate([r * pad + np.arange(totals[r], dtype=np.int64) for r in range(world)])
+        src = torch.from_numpy(src[np.argsort(query_of, kind="stable")]).to(dev)
+        out = full.index_select(0, src)
+        lims_h = np.zeros(nq + 1, dtype=np.int64)
+        np.cumsum(C.sum(axis=0), out=lims_h[1:])
+        I_out = out[:, :2].contiguous().view(torch.int64).view(-1)
+        D_out = out[:, 2].contiguous().view(torch.float32)
+        self.last_exchange_bytes = int(counts.numel() * 8 * (world - 1) // world + full.numel() * 4 * (world - 1) // world)
+        return torch.from_numpy(lims_h).to(dev), D_out, I_out

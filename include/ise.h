@@ -252,6 +252,47 @@ int ise_rescore_select(ise_ctx* ctx, const void* a, int a_dtype, int64_t lda, co
                        const float* cand_val, const int64_t* cand_idx,
                        float* out_val, int64_t* out_idx, int32_t* flag_rows, int32_t* flag_count, void* stream);
 
+/* ---- range search over the flat index (faiss/IndexFlat.cpp IndexFlat::range_search ->
+ * faiss/utils/distances.cpp range_search_inner_product / range_search_L2sqr) ------------------------------
+ * Every column whose exact FP32 score beats `radius` (IP: dis > radius, L2: squared dis < radius; strict).
+ * Results of a row are in ascending id.  Tensor-core path (nq >= 20), no host round trip inside a step:
+ *   ise_range_seed:  row_seed[m] for ise_gemm_collect = radius loosened by the rigorous coarse bound of the hi-plane
+ *                    product (eps for IP, 2 eps for L2) plus the FP32 re-score's rounding and a few ulps, so that the
+ *                    collect over hi-only planes appends EVERY column whose exact score can qualify.  Operands and
+ *                    their meta / norms / row_inv as prepared for the collect (a_row_inv nullable).
+ *   ise_gemm_collect (unchanged; hi planes only, cap slots per row);
+ *   ise_range_count: exact FP32 re-score of the first min(row_count, cap) candidates of every row (rescore formulas:
+ *                    <a,b>, or max(0, |a|^2 + |b|^2 - 2<a,b>)); passes get the exact score in cand_val, failures id -1
+ *                    in cand_idx.  kept[m + 1] int64: kept per row, 0 for overflowing rows (row_count > cap: the
+ *                    caller re-runs them with a larger cap), kept[m] = 0.  a: f32 or u8 rows, b: f32 rows.
+ *   ise_range_lims:  lims[m + 1] = base + exclusive scan of kept[m + 1].
+ *   ise_range_fill:  kept pairs of candidate row i -> out[lims[row_map ? row_map[i] : i] ...] (slot order); rows with
+ *                    row_count > cap are skipped.
+ *   ise_range_sort:  sorts every segment [lims[r], lims[r+1]) of (ids, dis) by id, in place (lims[0] = 0,
+ *                    total < 2^31). */
+int ise_range_seed(ise_ctx* ctx, const float* a_meta, const float* a_norms, const float* a_row_inv,
+                   const float* b_meta, int64_t m, int d, int metric, float radius, float* row_seed, void* stream);
+int ise_range_count(ise_ctx* ctx, const void* a, int a_dtype, int64_t lda, const float* b, int64_t ldb,
+                    int64_t m, int64_t n, int d, int metric, float radius, int64_t id_base,
+                    const float* a_norms, const float* b_norms, int cap, const int32_t* row_count,
+                    float* cand_val, int64_t* cand_idx, int64_t* kept, void* stream);
+size_t ise_range_lims_workspace_bytes(ise_ctx* ctx, int64_t m);
+int ise_range_lims(ise_ctx* ctx, const int64_t* kept, int64_t m, int64_t base, int64_t* lims,
+                   void* workspace, size_t workspace_bytes, void* stream);
+int ise_range_fill(ise_ctx* ctx, int64_t m, int cap, const int32_t* row_count, const float* cand_val,
+                   const int64_t* cand_idx, const int64_t* row_map, const int64_t* lims, float* out_dis,
+                   int64_t* out_ids, void* stream);
+size_t ise_range_sort_workspace_bytes(ise_ctx* ctx, int64_t m, int64_t total);
+int ise_range_sort(ise_ctx* ctx, int64_t m, const int64_t* lims, int64_t total, float* dis, int64_t* ids,
+                   void* workspace, size_t workspace_bytes, void* stream);
+/* Exact path (nq < 20, Faiss's direct per-pair formulas): range search over scores[nq, nb] of ise_pair_scores.
+ * Writes lims[nq + 1] (= base + offsets) always and, when out_dis / out_ids are given (length lims[nq] - base),
+ * the qualifying (score, id_base + column) pairs in column order. */
+size_t ise_scores_range_workspace_bytes(ise_ctx* ctx, int64_t nq, int64_t nb);
+int ise_scores_range(ise_ctx* ctx, const float* scores, int64_t nq, int64_t nb, int metric, float radius,
+                     int64_t id_base, int64_t base, int64_t* lims, float* out_dis, int64_t* out_ids,
+                     void* workspace, size_t workspace_bytes, void* stream);
+
 /* Merge g sorted top-k lists per row ([g, m, topk] each) into one; canonical (score, id) order.
  * Used for column-split partial results and for the cross-GPU merge of a sharded index. */
 int ise_topk_merge(ise_ctx* ctx, const float* val_parts, const int64_t* idx_parts, int g, int64_t m,
