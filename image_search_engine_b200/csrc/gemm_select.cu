@@ -13,8 +13,6 @@
 //                           or thread-local lists while the next tile's MMAs run
 // Replaces Faiss knn_inner_product / knn_L2sqr (sgemm + result handler) behind
 // reference call sites kmeans_faiss.py:41,49 and engine.py:55.
-#include <stdlib.h>
-
 #include <algorithm>
 #include <vector>
 
@@ -22,12 +20,6 @@
 #include "sm100_ptx.cuh"
 #include "topk_list.cuh"
 #include "rows_convert.cuh"
-
-// epilogue variants (A/B-tested on the B200, see profiles/r01_findings.md)
-#ifndef ISE_EPI_PREFETCH
-#define ISE_EPI_PREFETCH 0   // 1 = issue the next chunk's tcgen05.ld before scanning the current one
-                             // (measured SLOWER: C2 assign 1.53 vs 1.41 ms split, 1.32 vs 1.01 ms coarse)
-#endif
 
 namespace gs {
 
@@ -38,27 +30,18 @@ constexpr int UMMA_K = 16;
 constexpr int A_TILE_BYTES = BLOCK_M * BLOCK_K * 2;  // 16 KiB
 constexpr int B_TILE_BYTES = BLOCK_N * BLOCK_K * 2;  // 32 KiB
 constexpr int EPI_WARP0 = 4;
-// One epilogue warp per TMEM lane quadrant.  Two warps per quadrant (each scanning half of a tile's columns) is a
-// build-time option for the coarse top-1 kernels only (-DISE_EPI_HALVES_COARSE_TOP1=2): measured at the d = 128 C2
-// shape it moves the split products from 1.43 to 1.57-1.67 ms (MMA-bound: nothing to gain, a hand-over to pay) and
-// the one-product coarse pass from 1.07 to 0.99 ms (bound by the L2 -> shared-memory feed, not by the epilogue's TMEM
-// reads: profiles/r01_findings.md section 8), so the default stays at one.
-#ifndef ISE_EPI_HALVES_COARSE_TOP1
-#define ISE_EPI_HALVES_COARSE_TOP1 1
-#endif
+// One epilogue warp per TMEM lane quadrant.  Two warps per quadrant (each scanning half of a tile's columns) measured
+// slower for the coarse top-1 kernels at the d = 128 C2 shape: the split products are MMA-bound (nothing to gain, a
+// hand-over to pay) and the one-product coarse pass is bound by the L2 -> shared-memory feed, not by the epilogue's
+// TMEM reads (profiles/r01_findings.md section 8).
 // The resident-row-tile kernels (ARES: the verified one-product assign at d <= 128) are bound by their epilogue, not by
 // the tensor pipe: a single warp per scheduler runs the dependent max / select chains at ~0.27 IPC (ncu, profiles/
 // r02_findings.md), so they get two warps per quadrant to interleave.
-#ifndef ISE_EPI_HALVES_ARES
-#define ISE_EPI_HALVES_ARES 2
-#endif
-__host__ __device__ constexpr int epi_halves(int ksel, int pa, int pb, bool ares = false) {
-    return ares ? ISE_EPI_HALVES_ARES : ((ksel == 1 && pa == 1 && pb == 1) ? ISE_EPI_HALVES_COARSE_TOP1 : 1);
-}
+__host__ __device__ constexpr int epi_halves(bool ares) { return ares ? 2 : 1; }
 // conv: four extra warps that convert the NEXT work item's float32 rows into FP16 planes while the current item is
 // being multiplied (fused assign, see the CONV template parameter)
-__host__ __device__ constexpr int num_threads(int ksel, int pa, int pb, int mt = 1, bool conv = false, bool ares = false) {
-    return 128 + 128 * epi_halves(ksel, pa, pb, ares) * mt + (conv ? 128 : 0);
+__host__ __device__ constexpr int num_threads(int mt = 1, bool conv = false, bool ares = false) {
+    return 128 + 128 * epi_halves(ares) * mt + (conv ? 128 : 0);
 }
 constexpr int TMEM_COLS = 512;  // 2 accumulator stages x BLOCK_N fp32 columns
 constexpr int AUX_BYTES = 8192;
@@ -184,15 +167,14 @@ template <> struct SelList<32> { using type = RegList32; };
 //   one-product coarse pass at d = 128 needs 96 KB of operands per 1024 MMA cycles when A travels with every stage --
 //   more than L2 feeds one SM -- and 32 KB (CTA pairs) with A resident.
 template <int PA, int PB, bool L2, int KSEL, bool VERIFY, int CG, int MT = 1, bool CONV = false, int CL = 1, bool ARES = false>
-__global__ void __launch_bounds__(num_threads(KSEL, PA, PB, MT, CONV, ARES), 1)
+__global__ void __launch_bounds__(num_threads(MT, CONV, ARES), 1)
 gemm_select_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
                    const __grid_constant__ CUtensorMap tm_b_hi, const __grid_constant__ CUtensorMap tm_b_lo,
                    const Params p) {
-    static_assert(MT == 1 || (CG == 1 && epi_halves(KSEL, PA, PB, ARES) == 1), "two row tiles per CTA: single CTA, one warp per quadrant and tile");
+    static_assert(MT == 1 || (CG == 1 && epi_halves(ARES) == 1), "two row tiles per CTA: single CTA, one warp per quadrant and tile");
     static_assert(!CONV || (PA == 1 && KSEL == 1 && MT == 1), "fused conversion: top-1, hi plane of A");
-    static_assert(epi_halves(KSEL, PA, PB, ARES) == 1 || epi_halves(KSEL, PA, PB, ARES) == 2 || epi_halves(KSEL, PA, PB, ARES) == 4, "column slices per tile");
     static_assert(!ARES || (PA == 1 && MT == 1 && CL == 1), "resident row tile: hi plane of A, one row tile per CTA, no multicast");
-    static_assert(CL == 1 || (CG == 2 && MT == 1 && !CONV && (CL == 2 || CL == 4)), "multicast clusters are made of CTA pairs");
+    static_assert(CL == 1 || (CG == 2 && MT == 1 && !CONV && CL == 2), "multicast clusters are made of CTA pairs");
     // uniform over the whole grid, before any barrier / TMEM state exists
     if (!CONV && p.skip_if_a_exact && __ldcg(p.a_meta + META_LO_NONZERO) == 0.f) return;
     if (p.gate != nullptr && __ldcg(p.gate) == 0) return;
@@ -213,7 +195,7 @@ gemm_select_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_con
     constexpr int B_LOAD_ROWS = BLOCK_N / CG;
     constexpr int B_ISSUE_ROWS = B_LOAD_ROWS / CL;    // ... of which it fetches this many rows itself (CL > 1: multicast)
     constexpr int B_ISSUE_BYTES = B_LOAD_BYTES / CL;
-    constexpr int HALVES = epi_halves(KSEL, PA, PB, ARES);
+    constexpr int HALVES = epi_halves(ARES);
     constexpr int NUM_EPI_THREADS = 128 * HALVES * MT;
     constexpr int COLS_PER_HALF = BLOCK_N / HALVES;
     static_assert(STAGES >= 2 && STAGES <= 8, "pipeline depth");
@@ -518,15 +500,10 @@ gemm_select_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_con
                 const int c_end = min(c_begin + COLS_PER_HALF, ncols);
                 // ROLLED loop over 32-column chunks: one copy of the scan / insertion code (I-cache)
                 uint32_t r[32];
-#if ISE_EPI_PREFETCH
-                if (c_begin < c_end) ptx::tmem_ld_32x32b_x32(taddr + c_begin, r);
-#endif
 #pragma unroll 1
                 for (int c = c_begin; c < c_end; c += 32) {
                     {
-#if !ISE_EPI_PREFETCH
                         ptx::tmem_ld_32x32b_x32(taddr + c, r);
-#endif
                         ptx::tmem_ld_wait();
                         float v[32];
 #pragma unroll
@@ -535,9 +512,6 @@ gemm_select_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_con
                             // maximise 2<a,b> - |b|^2  ==  minimise |a|^2 + |b|^2 - 2<a,b>
                             if (L2) v[j] = fmaf(v[j], two_inv, -aux->bnorm[tile & 1][c + j]);
                         }
-#if ISE_EPI_PREFETCH
-                        if (c + 32 < c_end) ptx::tmem_ld_32x32b_x32(taddr + c + 32, r);
-#endif
                         if (c + 32 > ncols) {
 #pragma unroll
                             for (int j = 0; j < 32; ++j)
@@ -842,45 +816,20 @@ struct Plan {
 // Measured on the B200 (profiles/r01_findings.md section 7): with the lo planes in play a stage is 48-64 KB per
 // CTA and carries 8-12 MMAs, and pairs win 4-6 % (C2 assign 1.36 vs 1.41 ms, C3 split top-1 92 vs 98 ms);
 // for the coarse pass (hi planes only, 4 MMAs per 32 KB stage) the cross-CTA signalling round trip is
-// exposed and pairs lose 3-20 %, so the coarse pass stays single-CTA.
-static int pick_cg(int64_t m, bool split_products, int d = 0, int topk = 1) {
-#ifdef ISE_FORCE_CG1
-    return 1;
-#endif
-#ifdef ISE_FORCE_CG2
-    split_products = true;
-#endif
-    // coarse top-k / collect passes at large d: with the soft lock-step keeping the column range in L2, halving the
-    // B bytes per MMA cycle pays (C3 seeded top-32 35.5 -> 33.0 ms); ISE_CG2_COARSE=0 / 1 overrides
-    if (!split_products && topk != 1) {
-        const char* e = getenv("ISE_CG2_COARSE");
-        if (e ? e[0] == '1' : d >= 1024) split_products = true;
-    }
-    return (split_products && ceil_div64(m, BLOCK_M) >= 4) ? 2 : 1;
+// exposed and pairs lose 3-20 %, so the coarse top-1 pass stays single-CTA.
+// Coarse top-k / collect passes at large d: with the soft lock-step keeping the column range in L2, halving the
+// B bytes per MMA cycle pays (C3 seeded top-32 35.5 -> 33.0 ms), so they use pairs too.
+static int pick_cg(int64_t m, bool split_products, int d, int topk) {
+    const bool pairs = split_products || (topk != 1 && d >= 1024);
+    return (pairs && ceil_div64(m, BLOCK_M) >= 4) ? 2 : 1;
 }
-
-// Optional cap on the bytes of B one work item streams (0 = off).  The CTAs that walk the same column range share
-// every B tile through L2 only while they stay within L2's reach of each other, and ncu showed 30 GB and 104 GB of
-// DRAM reads for the same C3 launch on two boxes.  Capping an item at 32 MB (123 column splits instead of 7) did not
-// help when measured back to back on one box: coarse top-1 36.3 vs 36.4 ms, seeded top-32 41.0 vs 37.8 ms (the extra
-// partial lists cost more than any reuse gained), so the cap stays off (profiles/r01_findings.md section 12).
-constexpr int64_t kL2BytesPerItem = 0;   // 0 = no cap (see below)
 
 // Two row tiles per CTA (MT = 2) for the coarse TOP-1 pass (hi planes only) when the MMAs of a tile pair outlast its
 // epilogue by a wide margin (d >= 1024: >= 16 k MMA cycles against ~2 k of scan) and there are enough row tiles to go
 // round: C3-shaped top-1 30.9 vs 35.5 ms.  The top-k list epilogues lose with it (seeded top-32 40.8 vs 35.4 ms,
 // profiles/r01_findings.md section 13), so they keep one row tile and double-buffered accumulators.
-// ISE_MT2=0 / 1 overrides (A/B measurements).
 static int pick_mt(int64_t m, int d, bool split_products, int topk) {
-    if (split_products) return 1;
-    if (topk != 1) {     // A/B only (ISE_MT2_TOPK=1): two row tiles per CTA for the list epilogues, measured slower
-        const char* et = getenv("ISE_MT2_TOPK");
-        return (et && et[0] == '1' && d >= 1024 && ceil_div64(m, BLOCK_M) >= 2) ? 2 : 1;
-    }
-    const char* e = getenv("ISE_MT2");
-    if (e && e[0] == '0') return 1;
-    const bool forced = e && e[0] == '1';
-    return ((forced || d >= 1024) && ceil_div64(m, BLOCK_M) >= 2) ? 2 : 1;
+    return (!split_products && topk == 1 && d >= 1024 && ceil_div64(m, BLOCK_M) >= 2) ? 2 : 1;
 }
 
 // The launch variant (CTAs per MMA, row tiles per CTA) is decided in ONE place: the tensor maps (B box height), the
@@ -890,7 +839,6 @@ struct Variant {
 };
 // Pairs per multicast cluster (CL) for the coarse top-k / collect pass at large d, where CTA pairs are used and the pass
 // is bound by the L2 -> shared-memory feed: 2 pairs (clusters of 4 CTAs) when there are enough row tiles.
-// ISE_CLUSTER_PAIRS = 1 | 2 | 4 overrides (A/B measurements).
 // Measured on the C3 coarse pass (10 k x 1 M x 2048, ncu, profiles/r02_findings.md): clusters of 2 pairs read 11.7 GB
 // from DRAM instead of 31.9 GB (L2 traffic 263 vs 380 GB) in the same 30.8 ms; 4 pairs 7.0 GB but 3 % slower (only 15
 // clusters of 8 whole-SM CTAs are co-resident: 120 of 148 SMs).  Small column sets (the 1/64 sample pre-pass) keep plain
@@ -898,11 +846,7 @@ struct Variant {
 static int pick_cl(int64_t m, int64_t n, int d, bool split_products, int topk, int cg) {
     if (cg != 2 || split_products || topk == 1) return 1;
     if (n * (int64_t)d * 2 < (256ll << 20)) return 1;                    // B plane below 256 MB
-    const char* e = getenv("ISE_CLUSTER_PAIRS");
-    int cl = e ? atoi(e) : 2;
-    if (cl != 1 && cl != 2 && cl != 4) cl = 1;
-    while (cl > 1 && ceil_div64(m, BLOCK_M) < 2 * 2 * cl) cl >>= 1;     // at least two clusters' worth of row tiles
-    return cl;
+    return ceil_div64(m, BLOCK_M) >= 2 * 2 * 2 ? 2 : 1;                  // at least two clusters' worth of row tiles
 }
 static Variant pick_variant(int64_t m, int64_t n, int d, bool split_products, int topk) {
     Variant v;
@@ -912,35 +856,28 @@ static Variant pick_variant(int64_t m, int64_t n, int d, bool split_products, in
     return v;
 }
 
-// co-resident clusters of `csize` whole-SM CTAs (clusters of 4 / 8 do not tile every GPC: 33 / 15 on the B200 instead
-// of 37 / 18); the answer is the same for every gemm_select instantiation (one CTA per SM), so one of them is asked once
+// co-resident clusters of `csize` (1, 2 or 4) whole-SM CTAs (clusters of 4 do not tile every GPC: 33 on the B200
+// instead of 37); the answer is the same for every gemm_select instantiation (one CTA per SM), so one of them is asked
+// once
 static int cluster_slots(const ise_ctx* ctx, int csize) {
-    static int cached[9] = {0};
     if (csize <= 2) return std::max(1, ctx->sm_count / csize);
-    if (cached[csize] == 0) {
+    static int cached = 0;
+    if (cached == 0) {
         int got = 0;
-        if (csize == 4 || csize == 8) {
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3((unsigned)(csize * (ctx->sm_count / csize)));
-            cfg.blockDim = dim3((unsigned)num_threads(32, 1, 1));
-            cfg.dynamicSmemBytes = (size_t)(num_stages(1, 1, 2) * stage_bytes(1, 1, 2) + AUX_BYTES + 1024);
-            cudaLaunchAttribute attr[1];
-            attr[0].id = cudaLaunchAttributeClusterDimension;
-            attr[0].val.clusterDim.x = csize; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-            cfg.attrs = attr; cfg.numAttrs = 1;
-            if (csize == 4) {
-                auto kern = gemm_select_kernel<1, 1, false, 32, false, 2, 1, false, 2>;
-                cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.dynamicSmemBytes);
-                cudaOccupancyMaxActiveClusters(&got, kern, &cfg);
-            } else {
-                auto kern = gemm_select_kernel<1, 1, false, 32, false, 2, 1, false, 4>;
-                cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.dynamicSmemBytes);
-                cudaOccupancyMaxActiveClusters(&got, kern, &cfg);
-            }
-        }
-        cached[csize] = got > 0 ? got : std::max(1, ctx->sm_count / csize);
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = dim3((unsigned)(csize * (ctx->sm_count / csize)));
+        cfg.blockDim = dim3((unsigned)num_threads());
+        cfg.dynamicSmemBytes = (size_t)(num_stages(1, 1, 2) * stage_bytes(1, 1, 2) + AUX_BYTES + 1024);
+        cudaLaunchAttribute attr[1];
+        attr[0].id = cudaLaunchAttributeClusterDimension;
+        attr[0].val.clusterDim.x = csize; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+        cfg.attrs = attr; cfg.numAttrs = 1;
+        auto kern = gemm_select_kernel<1, 1, false, 32, false, 2, 1, false, 2>;
+        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.dynamicSmemBytes);
+        cudaOccupancyMaxActiveClusters(&got, kern, &cfg);
+        cached = got > 0 ? got : std::max(1, ctx->sm_count / csize);
     }
-    return cached[csize];
+    return cached;
 }
 
 static Plan make_plan(const ise_ctx* ctx, int64_t m, int64_t n, int d, int topk, bool single_split = false,
@@ -958,15 +895,10 @@ static Plan make_plan(const ise_ctx* ctx, int64_t m, int64_t n, int d, int topk,
     int64_t want = ceil_div64((int64_t)4 * slots, std::max(1, groups));
     int64_t max_by_tiles = std::max<int64_t>(1, pl.n_ntiles / 8);
     int64_t s_hi = std::max<int64_t>(1, std::min<int64_t>(std::min<int64_t>(2 * want, max_by_tiles), 256));
-    // L2 reach: at least this many splits (when more than one row group shares the columns at all)
-    const int64_t tile_bytes = (int64_t)BLOCK_N * ((d + BLOCK_K - 1) / BLOCK_K * BLOCK_K) * 2 * (split_products ? 2 : 1);
-    const int64_t tiles_cap = kL2BytesPerItem > 0 ? std::max<int64_t>(8, kL2BytesPerItem / tile_bytes) : pl.n_ntiles;
-    int64_t s_lo = groups > 1 ? std::min<int64_t>(256, ceil_div64(pl.n_ntiles, tiles_cap)) : 1;
-    s_hi = std::max(s_hi, s_lo);
-    if (single_split) s_lo = s_hi = 1;  // top-1 verification keeps one runner-up per row, so columns are not split
+    if (single_split) s_hi = 1;  // top-1 verification keeps one runner-up per row, so columns are not split
     // pick the split count with the smallest makespan = waves x column tiles per item
-    int64_t best_s = s_lo, best_cost = -1;
-    for (int64_t s = s_lo; s <= s_hi; ++s) {
+    int64_t best_s = 1, best_cost = -1;
+    for (int64_t s = 1; s <= s_hi; ++s) {
         const int64_t tps = ceil_div64(pl.n_ntiles, s);
         const int64_t ns = ceil_div64(pl.n_ntiles, tps);
         const int64_t waves = ceil_div64((int64_t)groups * ns, slots);
@@ -985,13 +917,10 @@ static void setup_sync(const ise_ctx* ctx, Params& p, int d, bool split_products
     p.sync_cnt = nullptr;
     p.sync_every = 0;
     p.sync_ncp = 0;
-    const char* e = getenv("ISE_LOCKSTEP");
-    if (!ctx->sync_buf || (e && e[0] == '0')) return;
+    if (!ctx->sync_buf) return;
     const int64_t tile_bytes = (int64_t)BLOCK_N * ((d + BLOCK_K - 1) / BLOCK_K * BLOCK_K) * 2 * (split_products ? 2 : 1);
-    if (tile_bytes * p.tiles_per_split < (24ll << 20) && !(e && e[0] == '1')) return;
-    const char* e_mb = getenv("ISE_LOCKSTEP_MB");                                 // A/B: check-in interval in MB of B
-    const int64_t sync_bytes = (int64_t)((e_mb && atoi(e_mb) > 0) ? atoi(e_mb) : 16) << 20;
-    const int every = (int)std::max<int64_t>(1, sync_bytes / tile_bytes);          // ~16 MB of B between check-ins
+    if (tile_bytes * p.tiles_per_split < (24ll << 20)) return;
+    const int every = (int)std::max<int64_t>(1, (16ll << 20) / tile_bytes);         // ~16 MB of B between check-ins
     const int ncp = (p.tiles_per_split + every - 1) / every;
     const int grp = cg * mt;
     const int n_mgroups = (p.n_mtiles + grp - 1) / grp;
@@ -1020,7 +949,7 @@ static int launch_cg(const ise_ctx* ctx, const CUtensorMap* maps, const Params& 
     int slots = std::max(1, ctx->sm_count / CSIZE);
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)(CSIZE * slots));
-    cfg.blockDim = dim3((unsigned)num_threads(KSEL, PA, PB, MT, CONV, ARES));
+    cfg.blockDim = dim3((unsigned)num_threads(MT, CONV, ARES));
     cfg.dynamicSmemBytes = (size_t)smem;
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
@@ -1040,17 +969,19 @@ static int launch_cg(const ise_ctx* ctx, const CUtensorMap* maps, const Params& 
 template <int PA, int PB, bool L2, int KSEL, bool VERIFY = false>
 static int launch(const ise_ctx* ctx, const CUtensorMap* maps, const Params& p, cudaStream_t st) {
     const Variant var = pick_variant(p.m, p.n, p.d, PB == 2, KSEL == 1 ? 1 : 0);
-    if constexpr ((KSEL == 1 || KSEL == 32) && PA == 1 && PB == 1 && epi_halves(KSEL, PA, PB) == 1) {
-        if (var.mt == 2) return launch_cg<PA, PB, L2, KSEL, VERIFY, 1, 2>(ctx, maps, p, st);
+    if constexpr (KSEL == 1 && PA == 1 && PB == 1) {        // coarse top-1: single CTAs, one or two row tiles each
+        if (var.cg != 1) ISE_FAIL("internal: CTA pairs picked for the coarse top-1 pass");
+        return var.mt == 2 ? launch_cg<PA, PB, L2, KSEL, VERIFY, 1, 2>(ctx, maps, p, st)
+                           : launch_cg<PA, PB, L2, KSEL, VERIFY, 1>(ctx, maps, p, st);
+    } else {
+        if (var.mt != 1) ISE_FAIL("internal: two-row-tile variant picked for a kernel that has none");
+        if constexpr (PA == 1 && PB == 1) {       // coarse top-k / collect: multicast clusters of CTA pairs
+            if (var.cg == 2 && var.cl == 2) return launch_cg<PA, PB, L2, KSEL, VERIFY, 2, 1, false, 2>(ctx, maps, p, st);
+        }
+        if (var.cl != 1) ISE_FAIL("internal: multicast cluster picked for a kernel that has none");
+        return var.cg == 2 ? launch_cg<PA, PB, L2, KSEL, VERIFY, 2>(ctx, maps, p, st)
+                           : launch_cg<PA, PB, L2, KSEL, VERIFY, 1>(ctx, maps, p, st);
     }
-    if (var.mt != 1) ISE_FAIL("internal: two-row-tile variant picked for a kernel that has none");
-    if constexpr (KSEL != 1 && PA == 1 && PB == 1) {       // coarse top-k / collect: multicast clusters of CTA pairs
-        if (var.cg == 2 && var.cl == 2) return launch_cg<PA, PB, L2, KSEL, VERIFY, 2, 1, false, 2>(ctx, maps, p, st);
-        if (var.cg == 2 && var.cl == 4) return launch_cg<PA, PB, L2, KSEL, VERIFY, 2, 1, false, 4>(ctx, maps, p, st);
-    }
-    if (var.cl != 1) ISE_FAIL("internal: multicast cluster picked for a kernel that has none");
-    return var.cg == 2 ? launch_cg<PA, PB, L2, KSEL, VERIFY, 2>(ctx, maps, p, st)
-                       : launch_cg<PA, PB, L2, KSEL, VERIFY, 1>(ctx, maps, p, st);
 }
 
 template <int PA, int PB, bool L2>
@@ -1073,10 +1004,19 @@ static int dispatch_metric(const ise_ctx* ctx, const CUtensorMap* maps, const Pa
                                    : dispatch_k<PA, PB, false>(ctx, maps, p, st);
 }
 
-static void clear_conv(Params& p) {
-    p.a_raw = nullptr; p.lda_raw = 0; p.a_hi_w = nullptr; p.a_lo_w = nullptr; p.lda_w = 0; p.a_norms_w = nullptr;
-    p.a_row_inv_w = nullptr; p.a_lo_skipped = nullptr; p.a_meta_w = nullptr; p.skip_if_a_exact = 0;
-    p.gate = nullptr; p.m_dev = nullptr; p.row_map = nullptr;
+// the parameters of a plain launch under plan `pl`: every field not set here (the optional inputs and outputs, the
+// fused-conversion operand, the verified-pipeline controls) starts zero / null
+static Params make_params(const Plan& pl, int64_t m, int64_t n, int d, int topk, int64_t id_base, const float* a_meta,
+                          const float* a_norms, const float* a_row_inv, const float* b_meta, const float* b_norms,
+                          float* out_val, int64_t* out_idx) {
+    Params p{};
+    p.m = m; p.n = n; p.d = d;
+    p.n_mtiles = pl.n_mtiles; p.n_ntiles = pl.n_ntiles;
+    p.tiles_per_split = pl.tiles_per_split; p.n_splits = pl.n_splits;
+    p.topk = topk; p.id_base = id_base;
+    p.a_meta = a_meta; p.a_norms = a_norms; p.a_row_inv = a_row_inv; p.b_meta = b_meta; p.b_norms = b_norms;
+    p.out_val = out_val; p.out_idx = out_idx;
+    return p;
 }
 
 }  // namespace gs
@@ -1141,17 +1081,9 @@ ISE_EXPORT int ise_gemm_collect(ise_ctx* ctx, const void* a_hi, const void* a_lo
     if (metric == ISE_METRIC_L2) ISE_CHECK_ARG(a_norms && b_norms);
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
-    gs::Plan pl = gs::make_plan(ctx, m, n, d, 0, false, b_lo != nullptr);
-    gs::Params p;
-    p.m = m; p.n = n; p.d = d;
-    p.n_mtiles = pl.n_mtiles; p.n_ntiles = pl.n_ntiles;
-    p.tiles_per_split = pl.tiles_per_split; p.n_splits = pl.n_splits;
-    p.topk = cap; p.id_base = id_base;
-    p.a_meta = a_meta; p.b_meta = b_meta; p.a_norms = a_norms; p.b_norms = b_norms;
-    p.a_row_inv = a_row_inv;
-    p.row_seed = row_seed; p.row_count = row_count; p.flag_rows = nullptr; p.flag_count = nullptr;
-    gs::clear_conv(p);
-    p.out_val = cand_val; p.out_idx = cand_idx;
+    const gs::Plan pl = gs::make_plan(ctx, m, n, d, 0, false, b_lo != nullptr);
+    gs::Params p = gs::make_params(pl, m, n, d, cap, id_base, a_meta, a_norms, a_row_inv, b_meta, b_norms, cand_val, cand_idx);
+    p.row_seed = row_seed; p.row_count = row_count;
     // empty slots read as id -1 / count 0
     ISE_CUDA(cudaMemsetAsync(cand_idx, 0xFF, (size_t)m * cap * sizeof(int64_t), st));
     ISE_CUDA(cudaMemsetAsync(row_count, 0, (size_t)m * sizeof(int32_t), st));
@@ -1185,18 +1117,10 @@ static int gemm_select_impl(ise_ctx* ctx, const void* a_hi, const void* a_lo, in
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
 
-    gs::Plan pl = gs::make_plan(ctx, m, n, d, topk, flag_count != nullptr, b_lo != nullptr);
-    gs::Params p;
-    p.m = m; p.n = n; p.d = d;
-    p.n_mtiles = pl.n_mtiles; p.n_ntiles = pl.n_ntiles;
-    p.tiles_per_split = pl.tiles_per_split; p.n_splits = pl.n_splits;
-    p.topk = topk; p.id_base = id_base;
-    p.a_meta = a_meta; p.b_meta = b_meta; p.a_norms = a_norms; p.b_norms = b_norms;
-    p.a_row_inv = a_row_inv;
-    gs::clear_conv(p);
+    const gs::Plan pl = gs::make_plan(ctx, m, n, d, topk, flag_count != nullptr, b_lo != nullptr);
+    gs::Params p = gs::make_params(pl, m, n, d, topk, id_base, a_meta, a_norms, a_row_inv, b_meta, b_norms, out_val, out_idx);
     p.skip_if_a_exact = skip_if_a_exact;
     p.row_seed = row_seed;
-    p.row_count = nullptr;
     p.flag_rows = flag_rows;
     p.flag_count = flag_count;
     if (flag_count) {
@@ -1212,8 +1136,6 @@ static int gemm_select_impl(ise_ctx* ctx, const void* a_hi, const void* a_lo, in
         wi = reinterpret_cast<int64_t*>(workspace);  // int64 first keeps both arrays aligned
         wv = reinterpret_cast<float*>(wi + cnt);
         p.out_val = wv; p.out_idx = wi;
-    } else {
-        p.out_val = out_val; p.out_idx = out_idx;
     }
 
     const int pa = a_lo ? 2 : 1, pb = b_lo ? 2 : 1;
@@ -1309,7 +1231,6 @@ static VerifiedWs verified_ws(void* base, int64_t m, int64_t lda) {
 // covered: up to two 64-column k-blocks (the resident row tile), enough column tiles to cycle the stage ring within an
 // item, and enough row tiles that one unsplit column range fills the machine
 static bool verified_covers(const ise_ctx* ctx, int64_t m, int64_t n, int d, int64_t lda) {
-    if (getenv("ISE_NO_VERIFIED_ASSIGN")) return false;
     const int num_kb = (d + BLOCK_K - 1) / BLOCK_K;
     if (d > 128 || lda > 128 || n < 2) return false;
     if (ceil_div64(n, BLOCK_N) * num_kb < 8) return false;
@@ -1327,14 +1248,12 @@ static int verified_launches(ise_ctx* ctx, Params p, const float* x, int64_t ldx
     const bool rerun_lo = !conv && a_lo != nullptr;          // prepared rows that may carry a lo plane
     const float* a_norms = p.a_norms;
     const float* a_row_inv = p.a_row_inv;
-    clear_conv(p);                                           // the re-runs are plain launches
     ISE_CUDA(cudaMemsetAsync(w.ctrl, 0, 16, st));
     CUtensorMap maps[4];
+    Variant pair; pair.cg = 2; pair.mt = 1; pair.cl = 1;   // every launch of the pipeline runs CTA pairs
     // ---- 1. one product per tile, exact runner-up, rows that are not provably decided are listed
     {
-        const char* e = getenv("ISE_VERIFIED_CG");
-        Variant var; var.cg = (e && e[0] == '1') ? 1 : 2; var.mt = 1; var.cl = 1;
-        if (setup_maps_var(ctx, a_hi, nullptr, lda, b_hi, nullptr, ldb, m, n, d, var, maps)) return 1;
+        if (setup_maps_var(ctx, a_hi, nullptr, lda, b_hi, nullptr, ldb, m, n, d, pair, maps)) return 1;
         Params q = p;
         q.flag_rows = w.flag_rows; q.flag_count = w.ctrl;
         if (conv) {
@@ -1342,11 +1261,8 @@ static int verified_launches(ise_ctx* ctx, Params p, const float* x, int64_t ldx
             q.a_norms_w = const_cast<float*>(a_norms); q.a_row_inv_w = const_cast<float*>(a_row_inv);
             q.a_lo_skipped = a_lo_skipped; q.a_meta_w = a_meta_w;
         }
-        int rc;
-        if (conv) rc = var.cg == 2 ? launch_cg<1, 1, L2, 1, true, 2, 1, true, 1, true>(ctx, maps, q, st)
-                                   : launch_cg<1, 1, L2, 1, true, 1, 1, true, 1, true>(ctx, maps, q, st);
-        else rc = var.cg == 2 ? launch_cg<1, 1, L2, 1, true, 2, 1, false, 1, true>(ctx, maps, q, st)
-                              : launch_cg<1, 1, L2, 1, true, 1, 1, false, 1, true>(ctx, maps, q, st);
+        const int rc = conv ? launch_cg<1, 1, L2, 1, true, 2, 1, true, 1, true>(ctx, maps, q, st)
+                            : launch_cg<1, 1, L2, 1, true, 2, 1, false, 1, true>(ctx, maps, q, st);
         if (rc) return rc;
     }
     // ---- 2. compact the listed rows
@@ -1356,7 +1272,6 @@ static int verified_launches(ise_ctx* ctx, Params p, const float* x, int64_t ldx
             a_row_inv, w.g_hi, w.g_lo, w.g_norms, w.g_row_inv, w.ctrl + 1, w.ctrl + 2);
         ISE_LAUNCH_CHECK();
     }
-    Variant pair; pair.cg = 2; pair.mt = 1; pair.cl = 1;
     // ---- 3. split products over the compacted rows (row count read on the device), results scattered back
     {
         Params q = p;
@@ -1411,17 +1326,8 @@ ISE_EXPORT int ise_assign_verified(ise_ctx* ctx, const void* a_hi, const void* a
     const gs::VerifiedWs w = gs::verified_ws(workspace, m, lda);
     if (workspace_bytes < w.bytes) ISE_FAIL("workspace too small: need " + std::to_string(w.bytes));
     DeviceGuard guard(ctx->device);
-    gs::Plan pl = gs::make_plan(ctx, m, n, d, 1, true, false);
-    gs::Params p;
-    p.m = m; p.n = n; p.d = d;
-    p.n_mtiles = pl.n_mtiles; p.n_ntiles = pl.n_ntiles;
-    p.tiles_per_split = pl.tiles_per_split; p.n_splits = pl.n_splits;
-    p.topk = 1; p.id_base = id_base;
-    p.a_meta = a_meta; p.b_meta = b_meta; p.a_norms = a_norms; p.b_norms = b_norms; p.a_row_inv = a_row_inv;
-    p.row_seed = nullptr; p.row_count = nullptr; p.flag_rows = nullptr; p.flag_count = nullptr;
-    p.sync_cnt = nullptr; p.sync_every = 0; p.sync_ncp = 0;
-    p.out_val = out_val; p.out_idx = out_idx;
-    gs::clear_conv(p);
+    const gs::Plan pl = gs::make_plan(ctx, m, n, d, 1, true, false);
+    const gs::Params p = gs::make_params(pl, m, n, d, 1, id_base, a_meta, a_norms, a_row_inv, b_meta, b_norms, out_val, out_idx);
     return metric == ISE_METRIC_L2
                ? gs::verified_launches<true>(ctx, p, nullptr, 0, const_cast<void*>(a_hi), const_cast<void*>(a_lo), lda, nullptr, nullptr, b_hi, b_lo, ldb, w, (cudaStream_t)stream)
                : gs::verified_launches<false>(ctx, p, nullptr, 0, const_cast<void*>(a_hi), const_cast<void*>(a_lo), lda, nullptr, nullptr, b_hi, b_lo, ldb, w, (cudaStream_t)stream);
@@ -1448,21 +1354,11 @@ ISE_EXPORT int ise_assign_fused(ise_ctx* ctx, const float* x, int64_t ldx, int64
     gs::Plan pl = gs::make_plan(ctx, m, n, d, 1, false, b_lo != nullptr);
     // covered: 16-byte aligned float32 rows of at most 128 columns (every keypoint descriptor type: SIFT 128, BRISK 64,
     // ORB 32), an unsplit column range (enough row tiles to fill the machine)
-    if (d % 4 != 0 || ldx % 4 != 0 || lda > 128 || !al16 || pl.n_splits != 1 || getenv("ISE_NO_FUSED_ASSIGN")) return 2;
+    if (d % 4 != 0 || ldx % 4 != 0 || lda > 128 || !al16 || pl.n_splits != 1) return 2;
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
     ISE_CUDA(cudaMemsetAsync(a_meta, 0, META_FLOATS * sizeof(float), st));
-    gs::Params p;
-    p.m = m; p.n = n; p.d = d;
-    p.n_mtiles = pl.n_mtiles; p.n_ntiles = pl.n_ntiles;
-    p.tiles_per_split = pl.tiles_per_split; p.n_splits = pl.n_splits;
-    p.topk = 1; p.id_base = id_base;
-    p.a_meta = a_meta; p.b_meta = b_meta; p.a_norms = a_norms; p.b_norms = b_norms; p.a_row_inv = a_row_inv;
-    p.row_seed = nullptr; p.row_count = nullptr; p.flag_rows = nullptr; p.flag_count = nullptr;
-    p.out_val = out_val; p.out_idx = out_idx;
-    gs::clear_conv(p);
-    p.a_raw = x; p.lda_raw = ldx; p.a_hi_w = (__half*)a_hi; p.a_lo_w = (__half*)a_lo; p.lda_w = lda;
-    p.a_norms_w = a_norms; p.a_row_inv_w = a_row_inv; p.a_lo_skipped = a_lo_skipped; p.a_meta_w = a_meta;
+    gs::Params p = gs::make_params(pl, m, n, d, 1, id_base, a_meta, a_norms, a_row_inv, b_meta, b_norms, out_val, out_idx);
     const bool l2 = metric == ISE_METRIC_L2;
     int rc;
     if (workspace != nullptr && b_lo != nullptr && gs::verified_covers(ctx, m, n, d, lda)) {
@@ -1471,7 +1367,6 @@ ISE_EXPORT int ise_assign_fused(ise_ctx* ctx, const float* x, int64_t ldx, int64
         ISE_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 15) == 0);
         const gs::VerifiedWs w = gs::verified_ws(workspace, m, lda);
         if (workspace_bytes < w.bytes) ISE_FAIL("workspace too small: need " + std::to_string(w.bytes));
-        p.sync_cnt = nullptr; p.sync_every = 0; p.sync_ncp = 0;
         rc = l2 ? gs::verified_launches<true>(ctx, p, x, ldx, a_hi, a_lo, lda, a_lo_skipped, a_meta, b_hi, b_lo, ldb, w, st)
                 : gs::verified_launches<false>(ctx, p, x, ldx, a_hi, a_lo, lda, a_lo_skipped, a_meta, b_hi, b_lo, ldb, w, st);
         if (rc) return rc;
@@ -1484,13 +1379,20 @@ ISE_EXPORT int ise_assign_fused(ise_ctx* ctx, const float* x, int64_t ldx, int64
     }
     CUtensorMap maps[4];
     if (setup_maps(ctx, a_hi, nullptr, lda, b_hi, b_lo, ldb, m, n, d, 1, maps)) return 1;
+    p.a_raw = x; p.lda_raw = ldx; p.a_hi_w = (__half*)a_hi; p.a_lo_w = (__half*)a_lo; p.lda_w = lda;
+    p.a_norms_w = a_norms; p.a_row_inv_w = a_row_inv; p.a_lo_skipped = a_lo_skipped; p.a_meta_w = a_meta;
     const int cg = gs::pick_variant(m, n, d, b_lo != nullptr, 1).cg;
-#define ISE_CONV_LAUNCH(PB, L2V)                                                                                       \
-    (cg == 2 ? gs::launch_cg<1, PB, L2V, 1, false, 2, 1, true>(ctx, maps, p, st)                                       \
-             : gs::launch_cg<1, PB, L2V, 1, false, 1, 1, true>(ctx, maps, p, st))
-    if (b_lo) rc = l2 ? ISE_CONV_LAUNCH(2, true) : ISE_CONV_LAUNCH(2, false);
-    else rc = l2 ? ISE_CONV_LAUNCH(1, true) : ISE_CONV_LAUNCH(1, false);
-#undef ISE_CONV_LAUNCH
+    if (b_lo == nullptr) {      // no split products: CTA pairs are never picked
+        if (cg != 1) ISE_FAIL("internal: CTA pairs picked for the fused assign without a B lo plane");
+        rc = l2 ? gs::launch_cg<1, 1, true, 1, false, 1, 1, true>(ctx, maps, p, st)
+                : gs::launch_cg<1, 1, false, 1, false, 1, 1, true>(ctx, maps, p, st);
+    } else if (cg == 2) {
+        rc = l2 ? gs::launch_cg<1, 2, true, 1, false, 2, 1, true>(ctx, maps, p, st)
+                : gs::launch_cg<1, 2, false, 1, false, 2, 1, true>(ctx, maps, p, st);
+    } else {
+        rc = l2 ? gs::launch_cg<1, 2, true, 1, false, 1, 1, true>(ctx, maps, p, st)
+                : gs::launch_cg<1, 2, false, 1, false, 1, 1, true>(ctx, maps, p, st);
+    }
     if (rc) return rc;
     if (a_lo) {
         // the tensor was NOT exact in its hi plane (device-side flag): complete the lo plane of the rows that skipped

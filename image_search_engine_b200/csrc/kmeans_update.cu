@@ -5,8 +5,6 @@
 // reductions (red.global.add.v4.f32) into the FP32 [k, d] sum matrix that lives in L2.
 // Sums are accumulated in FP32 like Faiss; the order differs (atomics vs Faiss's data order),
 // which stays inside the 1e-4 relative centroid tolerance of the parity contract.
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace {
@@ -82,164 +80,6 @@ __global__ void accumulate_kernel(const T* __restrict__ x, int64_t n, int d, int
     if (threadIdx.x == 0 && obj) {
         double t = 0.0;
         for (int i = 0; i < kWarps; ++i) t += s_obj[i];
-        if (t != 0.0) atomicAdd(obj, t);
-    }
-}
-
-// Shared-memory-privatised variant (small k * d, i.e. the codebook's sum matrix can be tiled over the SMs):
-// CTA (range, part) owns the centroids [range * R, range * R + R) -- their FP32 sums and counts live in ITS
-// shared memory -- and scans the ids of row partition `part`.  Shared-memory float atomics are CAS loops on this
-// architecture (ATOMS.CAST.SPIN), so ownership goes one level further: warp w owns the centroids with
-// (local id % 32 == w).  Per chunk of ids the CTA (1) scans the ids and queues every hit (row, centroid) with its
-// owner warp (native integer atomics), (2) each warp drains its queue: rows are gathered with 128-bit loads, four
-// in flight per lane, and added to the warp's own centroids with plain read-modify-writes.  The slice is flushed
-// to the global [k, d] matrix once at the end: global atomics drop from n * d / 4 to parts * k * d / 4
-// (C2: 32 M -> 1.7 M), which is what bound the plain kernel (0.28 of HBM peak).
-// Layout of a row's sums in shared memory: column 4 l + j of a 128-column block sits at j * 32 + l, so the four
-// accesses of a lane's float4 hit 32 distinct banks.
-constexpr int kPrivThreads = 1024;
-constexpr int kPrivWarps = kPrivThreads / 32;
-constexpr int kPrivUnroll = 4;
-constexpr int kPrivQCap = 128;             // queue entries per warp per chunk
-
-template <typename T> struct Vec4Load;
-template <> struct Vec4Load<float> {
-    static __device__ __forceinline__ float4 ld(const float* row, int c) { return __ldg(reinterpret_cast<const float4*>(row) + c); }
-};
-template <> struct Vec4Load<uint8_t> {
-    static __device__ __forceinline__ float4 ld(const uint8_t* row, int c) {
-        const uchar4 u = __ldg(reinterpret_cast<const uchar4*>(row) + c);
-        return make_float4((float)u.x, (float)u.y, (float)u.z, (float)u.w);
-    }
-};
-
-__device__ __forceinline__ int priv_slot(int c4, int j) {   // column 4 * c4 + j of a row -> slot in the row's smem tile
-    return (c4 >> 5) * 128 + j * 32 + (c4 & 31);
-}
-
-template <typename T>
-__global__ void __launch_bounds__(kPrivThreads, 1)
-accumulate_priv_kernel(const T* __restrict__ x, int64_t n, int d, int64_t ldx, const int64_t* __restrict__ assign,
-                       const float* __restrict__ cent, int metric, int64_t k, int R, int n_ranges, int parts,
-                       int chunk, float* __restrict__ sums, float* __restrict__ counts, double* __restrict__ obj) {
-    extern __shared__ float s_sum[];                    // [R][dpad] sums | [R] counts | queues | queue lengths
-    __shared__ double s_obj[kPrivWarps];
-    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-    const int d4 = d >> 2;
-    const int dpad = (d4 + 31) / 32 * 128;              // floats per row tile (whole 128-column blocks)
-    float* s_cnt = s_sum + (size_t)R * dpad;
-    uint32_t* s_q = reinterpret_cast<uint32_t*>(s_cnt + R);          // [kPrivWarps][kPrivQCap]: (row in chunk) << 12 | local id
-    int* s_qn = reinterpret_cast<int*>(s_q + kPrivWarps * kPrivQCap);
-    const int range = blockIdx.x % n_ranges, part = blockIdx.x / n_ranges;
-    const int64_t c0 = (int64_t)range * R, c1 = min(k, c0 + R);
-    const int64_t r_begin = n * part / parts, r_end = n * (part + 1) / parts;
-    for (int i = threadIdx.x; i < R * dpad + R; i += kPrivThreads) s_sum[i] = 0.f;
-    if (threadIdx.x < kPrivWarps) s_qn[threadIdx.x] = 0;
-    __syncthreads();
-    double my_obj = 0.0;
-    for (int64_t base = r_begin; base < r_end; base += chunk) {
-        // (1) scan this chunk's ids, queue the hits with their owner warps
-        for (int i = threadIdx.x; i < chunk; i += kPrivThreads) {
-            const int64_t r = base + i;
-            if (r >= r_end) break;
-            const int64_t a = __ldg(assign + r);
-            if (a < c0 || a >= c1) continue;
-            const int cl = (int)(a - c0);
-            const int pos = atomicAdd(&s_qn[cl & 31], 1);
-            if (pos < kPrivQCap) {
-                s_q[(cl & 31) * kPrivQCap + pos] = ((uint32_t)i << 12) | (uint32_t)cl;
-            } else {
-                // queue overflow (heavily skewed assignment): this thread adds the row straight to the global
-                // accumulators -- slow, correct, and never taken on balanced data
-                const T* row = x + r * ldx;
-                float acc = 0.f;
-                for (int c = 0; c < d; ++c) {
-                    const float v = (float)row[c];
-                    atomicAdd(sums + a * (int64_t)d + c, v);
-                    if (cent) {
-                        const float y = __ldg(cent + a * (int64_t)d + c);
-                        if (metric == ISE_METRIC_IP) acc = fmaf(v, y, acc);
-                        else { const float e = v - y; acc = fmaf(e, e, acc); }
-                    }
-                }
-                atomicAdd(counts + a, 1.0f);
-                my_obj += (double)acc;
-            }
-        }
-        __syncthreads();
-        // (2) drain: this warp's centroids are touched by nobody else
-        const int qn = min(s_qn[wib], kPrivQCap);
-        const uint32_t* q = s_q + wib * kPrivQCap;
-        for (int e0 = 0; e0 < qn; e0 += kPrivUnroll) {
-            int cl[kPrivUnroll];
-            const T* row[kPrivUnroll];
-#pragma unroll
-            for (int u = 0; u < kPrivUnroll; ++u) {
-                const uint32_t e = e0 + u < qn ? q[e0 + u] : 0xFFFFFFFFu;
-                cl[u] = e == 0xFFFFFFFFu ? -1 : (int)(e & 0xFFFu);
-                row[u] = x + (base + (int64_t)(e >> 12)) * ldx;
-            }
-            float acc[kPrivUnroll];
-#pragma unroll
-            for (int u = 0; u < kPrivUnroll; ++u) acc[u] = 0.f;
-            for (int c = lane; c < d4; c += 32) {
-                float4 v[kPrivUnroll];
-#pragma unroll
-                for (int u = 0; u < kPrivUnroll; ++u)
-                    if (cl[u] >= 0) v[u] = Vec4Load<T>::ld(row[u], c);
-#pragma unroll
-                for (int u = 0; u < kPrivUnroll; ++u) {
-                    if (cl[u] < 0) continue;
-                    // consecutive entries may hit the same centroid: plain RMWs, in program order within the lane
-                    float* dst = s_sum + (size_t)cl[u] * dpad;
-                    dst[priv_slot(c, 0)] += v[u].x;
-                    dst[priv_slot(c, 1)] += v[u].y;
-                    dst[priv_slot(c, 2)] += v[u].z;
-                    dst[priv_slot(c, 3)] += v[u].w;
-                    if (cent) {
-                        const float4 y = __ldg(reinterpret_cast<const float4*>(cent + (c0 + cl[u]) * (int64_t)d) + c);
-                        if (metric == ISE_METRIC_IP) {
-                            acc[u] = fmaf(v[u].x, y.x, acc[u]); acc[u] = fmaf(v[u].y, y.y, acc[u]);
-                            acc[u] = fmaf(v[u].z, y.z, acc[u]); acc[u] = fmaf(v[u].w, y.w, acc[u]);
-                        } else {
-                            const float e0_ = v[u].x - y.x, e1 = v[u].y - y.y, e2 = v[u].z - y.z, e3 = v[u].w - y.w;
-                            acc[u] = fmaf(e0_, e0_, acc[u]); acc[u] = fmaf(e1, e1, acc[u]);
-                            acc[u] = fmaf(e2, e2, acc[u]); acc[u] = fmaf(e3, e3, acc[u]);
-                        }
-                    }
-                }
-            }
-            // objective terms stay per lane (reduced once at the end); counts by lane 0
-#pragma unroll
-            for (int u = 0; u < kPrivUnroll; ++u) {
-                if (cl[u] < 0) continue;
-                my_obj += (double)acc[u];
-                if (lane == 0) s_cnt[cl[u]] += 1.0f;
-            }
-        }
-        __syncwarp();
-        if (lane == 0) s_qn[wib] = 0;
-        __syncthreads();
-    }
-    // every thread may hold objective terms (overflow path): reduce over the warp, then the CTA
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) my_obj += __shfl_xor_sync(0xffffffffu, my_obj, o);
-    if (lane == 0) s_obj[wib] = my_obj;
-    __syncthreads();
-    // flush the slice: only centroids this CTA actually touched
-    for (int64_t cl = wib; cl < c1 - c0; cl += kPrivWarps) {
-        const float h = s_cnt[cl];
-        if (h == 0.f) continue;
-        if (lane == 0) atomicAdd(counts + c0 + cl, h);
-        const float* src = s_sum + (size_t)cl * dpad;
-        float* dst = sums + (c0 + cl) * (int64_t)d;
-        for (int c = lane; c < d4; c += 32)
-            red_add_v4(dst + 4 * c, make_float4(src[priv_slot(c, 0)], src[priv_slot(c, 1)], src[priv_slot(c, 2)],
-                                                src[priv_slot(c, 3)]));
-    }
-    if (threadIdx.x == 0 && obj && cent) {
-        double t = 0.0;
-        for (int i = 0; i < kPrivWarps; ++i) t += s_obj[i];
         if (t != 0.0) atomicAdd(obj, t);
     }
 }
@@ -519,7 +359,7 @@ __global__ void apply_splits_kernel(float* __restrict__ centroids, int d, const 
 }  // namespace
 
 ISE_EXPORT int ise_kmeans_accumulate(ise_ctx* ctx, const void* x, int dtype, int64_t n, int d, int64_t ldx,
-                                     const int64_t* assign, const float* dis, const float* centroids, int64_t k_hint,
+                                     const int64_t* assign, const float* dis, const float* centroids, int64_t /*k*/,
                                      int metric, float* sums, float* counts, double* obj, void* stream) {
     ISE_CHECK_ARG(ctx && n >= 0 && d > 0 && ldx >= d);
     ISE_CHECK_ARG(dtype == ISE_DTYPE_F32 || dtype == ISE_DTYPE_U8);
@@ -528,43 +368,6 @@ ISE_EXPORT int ise_kmeans_accumulate(ise_ctx* ctx, const void* x, int dtype, int
     ISE_CHECK_ARG(metric == ISE_METRIC_IP || metric == ISE_METRIC_L2);
     if (centroids) ISE_CHECK_ARG((reinterpret_cast<uintptr_t>(centroids) & 15) == 0);
     DeviceGuard guard(ctx->device);
-    // privatised path: needs the objective recomputed in-kernel (or no objective), 16-byte rows and a codebook whose
-    // [k, d] sums tile over at most one CTA per SM
-    if (k_hint > 0 && (centroids || !dis) && d % 4 == 0 && ldx % 4 == 0 && n >= 4096 &&
-        (dtype == ISE_DTYPE_U8 ? true : ((reinterpret_cast<uintptr_t>(x) & 15) == 0 && ldx % 4 == 0)) &&
-        (dtype == ISE_DTYPE_U8 ? (ldx % 4 == 0 && (reinterpret_cast<uintptr_t>(x) & 3) == 0) : true) &&
-        (reinterpret_cast<uintptr_t>(sums) & 15) == 0 && !getenv("ISE_ACCUMULATE_PLAIN")) {
-        const int dpad = ((d / 4) + 31) / 32 * 128;
-        const size_t q_bytes = (size_t)kPrivWarps * kPrivQCap * sizeof(uint32_t) + kPrivWarps * sizeof(int);
-        const size_t budget = 200 * 1024 - q_bytes;
-        const int64_t r_max = std::min<int64_t>(4096, (int64_t)(budget / sizeof(float)) / (dpad + 1));   // local ids: 12 bits
-        if (r_max >= 1) {
-            const int64_t n_ranges = ceil_div64(k_hint, r_max);
-            if (n_ranges <= ctx->sm_count) {
-                const int R = (int)ceil_div64(k_hint, n_ranges);
-                const int parts = std::max<int>(1, ctx->sm_count / (int)n_ranges);
-                // chunk: on average half a queue of hits per warp (hit rate ~ 1 / n_ranges), at most 2^20 rows
-                const int chunk = (int)std::max<int64_t>(1024, std::min<int64_t>((int64_t)kPrivWarps * (kPrivQCap / 2) * n_ranges, 1 << 15));
-                const size_t shm = ((size_t)R * dpad + R) * sizeof(float) + q_bytes;
-                const int grid_p = (int)n_ranges * parts;
-                if (dtype == ISE_DTYPE_F32) {
-                    auto kern = accumulate_priv_kernel<float>;
-                    ISE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shm));
-                    kern<<<grid_p, kPrivThreads, shm, (cudaStream_t)stream>>>((const float*)x, n, d, ldx, assign, centroids,
-                                                                              metric, k_hint, R, (int)n_ranges, parts, chunk,
-                                                                              sums, counts, obj);
-                } else {
-                    auto kern = accumulate_priv_kernel<uint8_t>;
-                    ISE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shm));
-                    kern<<<grid_p, kPrivThreads, shm, (cudaStream_t)stream>>>((const uint8_t*)x, n, d, ldx, assign, centroids,
-                                                                              metric, k_hint, R, (int)n_ranges, parts, chunk,
-                                                                              sums, counts, obj);
-                }
-                ISE_LAUNCH_CHECK();
-                return 0;
-            }
-        }
-    }
     const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(ceil_div64(n, kWarps), (int64_t)ctx->sm_count * 8));
     if (dtype == ISE_DTYPE_F32)
         accumulate_kernel<float><<<grid, kThreads, 0, (cudaStream_t)stream>>>((const float*)x, n, d, ldx, assign, dis,

@@ -1,7 +1,5 @@
 // Operand preparation: FP32 / uint8 rows -> scaled FP16 hi/lo planes + exact FP32 row norms,
 // and faiss.normalize_L2.  HBM-bound streaming kernels: one warp per row, 128-bit loads.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "rows_convert.cuh"
 
@@ -467,7 +465,7 @@ ISE_EXPORT int ise_prepare_rows(ise_ctx* ctx, const void* x, int dtype, int64_t 
     }
     ISE_CHECK_ARG(x && hi);
     const bool al16 = ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(hi) | reinterpret_cast<uintptr_t>(lo)) & 15) == 0;
-    if (dtype == ISE_DTYPE_F32 && d % 4 == 0 && ldx % 4 == 0 && al16 && ldp <= 512 && !getenv("ISE_PREPARE_TWO_PASS")) {
+    if (dtype == ISE_DTYPE_F32 && d % 4 == 0 && ldx % 4 == 0 && al16 && ldp <= 512) {
         ISE_CUDA(cudaMemsetAsync(meta, 0, META_FLOATS * sizeof(float), st));
         const int nv = (int)((ldp / 4 + 31) / 32);
 #define ISE_ROWS_ARGS (const float*)x, n, d, ldx, (__half*)hi, (__half*)lo, ldp, norms, row_inv, lo_skipped, meta

@@ -7,7 +7,6 @@ of the hot path is a libise kernel.  All functions take CUDA tensors and launch 
 from __future__ import annotations
 
 import ctypes as C
-import os
 import threading
 from dataclasses import dataclass
 
@@ -388,7 +387,7 @@ def rescore_select(a_raw: torch.Tensor, b_raw: torch.Tensor, a_op: Operand, b_op
 # Below this dimension a top-1 tile is bound by reading the 128 x 256 FP32 accumulator out of TMEM
 # (~2.4k cycles, measured) rather than by its MMAs (d/64 * 512 cycles per product), so dropping the lo
 # product buys nothing and the split products are used directly (profiles/r01_findings.md).
-COARSE_TOP1_MIN_D = int(os.environ.get("ISE_COARSE_TOP1_MIN_D", "512"))
+COARSE_TOP1_MIN_D = 512
 VERIFIED_MAX_K = 100   # coarse candidates: 32 per query for k <= 16, 128 for k <= 100
 
 # statistics of the last search_topk call on this process (bench.py / tests read them)

@@ -304,8 +304,7 @@ int ise_topk_merge(ise_ctx* ctx, const float* val_parts, const int64_t* idx_part
  * objective terms: with `centroids` [k,d] given they are recomputed in exact FP32 here (IP: <x,c>,
  * L2: sum (x-c)^2) from the row already in registers, otherwise dis[] is summed.
  * accum buffers must be zeroed by the caller (so several shards / ranks can add into them).
- * k = number of centroids (rows of sums): lets the library tile the sum matrix over the SMs' shared memory
- * (privatised scatter-add) when it is small enough; k <= 0 selects the plain global-atomic kernel. */
+ * One warp per row, global atomics into sums / counts.  k (number of centroids) is ignored. */
 int ise_kmeans_accumulate(ise_ctx* ctx, const void* x, int dtype, int64_t n, int d, int64_t ldx,
                           const int64_t* assign, const float* dis, const float* centroids, int64_t k, int metric,
                           float* sums, float* counts, double* obj, void* stream);

@@ -1,6 +1,6 @@
 """Where does the seeded coarse top-32 pass (C3 shape) spend its time beyond the coarse top-1 pass?  Same launch with a
 seed nothing can beat (pure scan, no insert ever), with the real seed, and the top-1 kernels for reference."""
-import os, sys
+import sys
 import torch
 sys.path.insert(0, ".")
 from image_search_engine_b200 import ops
@@ -25,15 +25,9 @@ def t(fn, n=4):
     e1.record(); torch.cuda.synchronize()
     return e0.elapsed_time(e1) / n
 for rep in range(2):
-    for name, env, fn in (
-        ("top-32, real seed, pairs              ", {"ISE_CLUSTER_PAIRS": "1"}, lambda: ops.gemm_select(a.hi_only(), b.hi_only(), METRIC_IP, 32, row_seed=seed)),
-        ("top-32, seed nothing beats, pairs     ", {"ISE_CLUSTER_PAIRS": "1"}, lambda: ops.gemm_select(a.hi_only(), b.hi_only(), METRIC_IP, 32, row_seed=never)),
-        ("top-32, seed nothing beats, single CTA", {"ISE_CLUSTER_PAIRS": "1", "ISE_CG2_COARSE": "0"}, lambda: ops.gemm_select(a.hi_only(), b.hi_only(), METRIC_IP, 32, row_seed=never)),
-        ("top-32, real seed, single CTA         ", {"ISE_CLUSTER_PAIRS": "1", "ISE_CG2_COARSE": "0"}, lambda: ops.gemm_select(a.hi_only(), b.hi_only(), METRIC_IP, 32, row_seed=seed)),
-        ("top-1, two row tiles per CTA          ", {}, lambda: ops.gemm_select(a.hi_only(), b.hi_only(), METRIC_IP, 1)),
-        ("top-1, single CTA, one row tile       ", {"ISE_MT2": "0"}, lambda: ops.gemm_select(a.hi_only(), b.hi_only(), METRIC_IP, 1)),
+    for name, fn in (
+        ("top-32, real seed          ", lambda: ops.gemm_select(a.hi_only(), b.hi_only(), METRIC_IP, 32, row_seed=seed)),
+        ("top-32, seed nothing beats ", lambda: ops.gemm_select(a.hi_only(), b.hi_only(), METRIC_IP, 32, row_seed=never)),
+        ("top-1                      ", lambda: ops.gemm_select(a.hi_only(), b.hi_only(), METRIC_IP, 1)),
     ):
-        for k_ in ("ISE_CLUSTER_PAIRS", "ISE_CG2_COARSE", "ISE_MT2"):
-            os.environ.pop(k_, None)
-        os.environ.update(env)
         print(f"{name}: {t(fn):7.2f} ms", flush=True)

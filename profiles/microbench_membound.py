@@ -51,10 +51,6 @@ def rec(name, ms, nbytes):
 rec("prepare f32, integer-valued (absmax + hi plane + norms; 10 B/element moved)", t(lambda: ops.prepare_operand(X)), n * d * 10)
 Xf = X + 0.37
 rec("prepare f32, general (absmax + hi/lo planes + norms; 12 B/element moved)", t(lambda: ops.prepare_operand(Xf)), n * d * 12)
-import os
-os.environ["ISE_PREP_ROWS"] = "4"
-rec("prepare ROWS f32, integer-valued, 4 rows in flight per warp (A/B)", t(lambda: ops.prepare_operand(X, rows=True)), n * d * 6)
-os.environ.pop("ISE_PREP_ROWS")
 rec("prepare ROWS f32, integer-valued (single pass: 4 B read + hi plane + norms; 6 B/element)", t(lambda: ops.prepare_operand(X, rows=True)), n * d * 6)
 rec("prepare ROWS f32, general (single pass: 4 B read + hi/lo planes + norms; 8 B/element)", t(lambda: ops.prepare_operand(Xf, rows=True)), n * d * 8)
 rec("prepare u8 (one plane + norms)", t(lambda: ops.prepare_operand(Xu8)), n * d * (1 + 2))
@@ -62,8 +58,6 @@ rec("histogram f64 numpy-compat + okapi", t(lambda: ops.bovw_histogram(words, of
 rec("histogram f64 bincount", t(lambda: ops.bovw_histogram(words, off, k, mode=HIST_BINCOUNT, out=out64)), n * 8 + n_img * k * 8)
 rec("histogram f32 numpy-compat + okapi", t(lambda: ops.bovw_histogram(words, off, k, mode=HIST_NUMPY_COMPAT, okapi=True, out_dtype=torch.float32, out=out32)), n * 8 + n_img * k * 4)
 rec("okapi_tf_ dense f64 in place (row sums + weights)", t(lambda: ops.okapi_tf_(out64)), n_img * k * 8 * 2)
-rec("kmeans_accumulate f32 (+ exact objective)", t(lambda: ops.kmeans_accumulate(X, words, None, sums, counts, obj, centroids=cent)), n * (4 * d + 8))
-rec("kmeans_accumulate u8", t(lambda: ops.kmeans_accumulate(Xu8, words, None, sums, counts, obj, centroids=cent)), n * (d + 8))
 ws = [None]
 def _sorted(x):
     ws[0] = ops.kmeans_accumulate_sorted(x, words, sums, counts, obj, centroids=cent, workspace=ws[0])

@@ -354,9 +354,9 @@ def test_assign_many_row_tiles(dev, metric_ip, d, kind, k):
 @pytest.mark.parametrize("metric_ip", [True, False])
 @pytest.mark.parametrize("n,d,k,kind", [(50000, 128, 4096, "sift"), (30000, 32, 512, "orb"), (20000, 64, 300, "float"),
                                           (9000, 256, 1000, "float"), (6000, 100, 64, "float"), (5000, 2048, 40, "float")])
-def test_privatised_accumulate_equals_oracle_and_plain(dev, monkeypatch, n, d, k, kind, metric_ip):
-    """Shared-memory-privatised scatter-add (sum matrix tiled over the SMs) vs the plain global-atomic kernel and
-    vs the oracle's sequential compute_centroids: counts exact, sums / objective within FP32 reassociation."""
+def test_plain_accumulate_equals_oracle(dev, n, d, k, kind, metric_ip):
+    """Global-atomic scatter-add vs the oracle's sequential compute_centroids: counts exact, sums / objective within
+    FP32 reassociation."""
     from image_search_engine_b200 import ops
     from image_search_engine_b200._lib import METRIC_IP, METRIC_L2
     from oracle import faiss_shim as fs
@@ -374,22 +374,14 @@ def test_privatised_accumulate_equals_oracle_and_plain(dev, monkeypatch, n, d, k
     c64 = cent.astype(np.float64)[assign[keep]]
     obj_ref = float((xf[keep] * c64).sum()) if metric_ip else float(((xf[keep] - c64) ** 2).sum())
     xd, ad, cd = torch.from_numpy(x).to(dev), torch.from_numpy(assign).to(dev), torch.from_numpy(cent).to(dev)
-    res = {}
-    for which in ("priv", "plain"):
-        if which == "plain":
-            monkeypatch.setenv("ISE_ACCUMULATE_PLAIN", "1")
-        else:
-            monkeypatch.delenv("ISE_ACCUMULATE_PLAIN", raising=False)
-        accum = torch.zeros(k * d + k, device=dev)
-        sums, counts = accum[:k * d].view(k, d), accum[k * d:]
-        obj = torch.zeros(1, dtype=torch.float64, device=dev)
-        ops.kmeans_accumulate(xd, ad, None, sums, counts, obj, centroids=cd,
-                              metric=METRIC_IP if metric_ip else METRIC_L2)
-        res[which] = (sums.cpu().numpy(), counts.cpu().numpy(), float(obj.item()))
-    for which, (s, c, o) in res.items():
-        assert np.array_equal(c, counts_ref), which
-        np.testing.assert_allclose(s, sums_ref, rtol=2e-5, atol=2e-5 * np.abs(sums_ref).max(), err_msg=which)
-        assert abs(o - obj_ref) <= 1e-5 * abs(obj_ref) + 1e-3, (which, o, obj_ref)
+    accum = torch.zeros(k * d + k, device=dev)
+    sums, counts = accum[:k * d].view(k, d), accum[k * d:]
+    obj = torch.zeros(1, dtype=torch.float64, device=dev)
+    ops.kmeans_accumulate(xd, ad, None, sums, counts, obj, centroids=cd, metric=METRIC_IP if metric_ip else METRIC_L2)
+    s, c, o = sums.cpu().numpy(), counts.cpu().numpy(), float(obj.item())
+    assert np.array_equal(c, counts_ref)
+    np.testing.assert_allclose(s, sums_ref, rtol=2e-5, atol=2e-5 * np.abs(sums_ref).max())
+    assert abs(o - obj_ref) <= 1e-5 * abs(obj_ref) + 1e-3, (o, obj_ref)
 
 
 def test_exact_inputs_skip_the_lo_plane_and_nobody_reads_it(dev):
