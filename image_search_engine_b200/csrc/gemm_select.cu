@@ -1347,6 +1347,8 @@ ISE_EXPORT int ise_assign_fused(ise_ctx* ctx, const float* x, int64_t ldx, int64
     if (m == 0) return 0;
     ISE_CHECK_ARG(x && a_hi && a_norms && a_row_inv && a_meta && b_hi && b_meta && out_val && out_idx);
     ISE_CHECK_ARG(a_lo == nullptr || a_lo_skipped != nullptr);
+    // rows that may be inexact need the split products, and those have no (2, 1) plane combination
+    if (a_lo != nullptr && b_lo == nullptr) ISE_FAIL("a_lo without b_lo is not supported: pass a zero b_lo plane");
     if (metric == ISE_METRIC_L2) ISE_CHECK_ARG(b_norms != nullptr);
     ISE_CHECK_ARG(lda >= d && ldb >= d && lda % 8 == 0 && ldb % 8 == 0 && ldx >= d);
     const bool al16 = ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(a_hi) | reinterpret_cast<uintptr_t>(a_lo) |
@@ -1382,7 +1384,7 @@ ISE_EXPORT int ise_assign_fused(ise_ctx* ctx, const float* x, int64_t ldx, int64
     p.a_raw = x; p.lda_raw = ldx; p.a_hi_w = (__half*)a_hi; p.a_lo_w = (__half*)a_lo; p.lda_w = lda;
     p.a_norms_w = a_norms; p.a_row_inv_w = a_row_inv; p.a_lo_skipped = a_lo_skipped; p.a_meta_w = a_meta;
     const int cg = gs::pick_variant(m, n, d, b_lo != nullptr, 1).cg;
-    if (b_lo == nullptr) {      // no split products: CTA pairs are never picked
+    if (b_lo == nullptr) {      // no split products (a_lo is NULL too): CTA pairs are never picked
         if (cg != 1) ISE_FAIL("internal: CTA pairs picked for the fused assign without a B lo plane");
         rc = l2 ? gs::launch_cg<1, 1, true, 1, false, 1, 1, true>(ctx, maps, p, st)
                 : gs::launch_cg<1, 1, false, 1, false, 1, 1, true>(ctx, maps, p, st);
@@ -1398,8 +1400,6 @@ ISE_EXPORT int ise_assign_fused(ise_ctx* ctx, const float* x, int64_t ldx, int64
         // the tensor was NOT exact in its hi plane (device-side flag): complete the lo plane of the rows that skipped
         // it and repeat the assign with the lo products; both launches return at once otherwise
         if (ise_internal_lo_fixup(ctx, a_lo, m, lda, a_lo_skipped, a_meta, stream)) return 1;
-        const void* b_lo_full = b_lo;
-        if (b_lo_full == nullptr) return 0;     // (2, 1) plane combination does not exist: hi-only result stands (documented)
         return gemm_select_impl(ctx, a_hi, a_lo, lda, a_meta, a_norms, a_row_inv, b_hi, b_lo, ldb, b_meta, b_norms, m, n, d,
                                 metric, 1, id_base, nullptr, nullptr, nullptr, out_val, out_idx, nullptr, 0, stream, 1);
     }

@@ -273,18 +273,21 @@ def assign_fused(x: torch.Tensor, b: Operand, metric: int, id_base: int = 0, ver
     lib, ctx = _lib.load(), _lib.ctx(dev)
     ldp = (d + 7) // 8 * 8
     hi = torch.empty((n, ldp), dtype=torch.float16, device=x.device)
-    lo = torch.empty((n, ldp), dtype=torch.float16, device=x.device) if b.lo is not None else None
+    # float32 rows may be inexact in their hi plane: they always get a lo plane (the repeat pass runs only when the
+    # device finds them inexact), and the split products need a b lo plane, all zero when b is exact in its hi plane
+    lo = torch.empty((n, ldp), dtype=torch.float16, device=x.device)
+    b_lo = b.lo if b.lo is not None else torch.zeros_like(b.hi)
     norms = torch.empty((n,), dtype=torch.float32, device=x.device)
     row_inv = torch.empty((n,), dtype=torch.float32, device=x.device)
-    skipped = torch.empty((n,), dtype=torch.uint8, device=x.device) if lo is not None else None
+    skipped = torch.empty((n,), dtype=torch.uint8, device=x.device)
     meta = torch.empty((8,), dtype=torch.float32, device=x.device)
     val = torch.empty((n, 1), dtype=torch.float32, device=x.device)
     idx = torch.empty((n, 1), dtype=torch.int64, device=x.device)
     ws = None
-    if verified and b.lo is not None and lib.ise_assign_verified_covers(ctx, n, b.n, d):
+    if verified and lib.ise_assign_verified_covers(ctx, n, b.n, d):
         ws = _assign_workspace(n, d, x.device)
     rc = lib.ise_assign_fused(ctx, _ptr(x), x.stride(0), n, d, _ptr(hi), _ptr(lo), ldp, _ptr(norms), _ptr(row_inv),
-                              _ptr(skipped), _ptr(meta), _ptr(b.hi), _ptr(b.lo), b.ldp, _ptr(b.meta), _ptr(b.norms), b.n,
+                              _ptr(skipped), _ptr(meta), _ptr(b.hi), _ptr(b_lo), b.ldp, _ptr(b.meta), _ptr(b.norms), b.n,
                               int(metric), int(id_base), _ptr(val), _ptr(idx), _ptr(ws), 0 if ws is None else ws.numel(),
                               _stream())
     if rc == 2:
@@ -293,10 +296,10 @@ def assign_fused(x: torch.Tensor, b: Operand, metric: int, id_base: int = 0, ver
     if ws is not None:
         ctrl = ws[:16].view(torch.int32)
         last_search_stats.update(mode="fused-verified", fallback_rows=ctrl[0], rows=n, overflow=ctrl[2])
-        _count(6 if lo is not None else 4)
+        _count(6)
     else:
         last_search_stats.update(mode="fused-split", fallback_rows=0, rows=n)
-        _count(3 if lo is not None else 1)
+        _count(3)
     return val, idx, Operand(hi, lo, norms, meta, n, d, ldp, row_inv=row_inv)
 
 

@@ -163,7 +163,8 @@ int ise_gemm_select(ise_ctx* ctx,
  * A is multiplied in the fused launch; when the rows turn out NOT to be exact in it (a_meta[2] != 0, decided on the
  * device) the lo plane is completed and the assign repeated with it by two follow-up launches that return at once
  * otherwise -- keypoint descriptors (integer SIFT, ORB / BRISK as float) are exact.  a_lo may be NULL only when the
- * caller knows that (no repeat pass then).  Returns 2 and does nothing when the shape is not covered (d % 4 != 0,
+ * caller knows that (no repeat pass then).  The repeat pass is a split product, so a_lo needs b_lo: a column operand
+ * that is exact in its hi plane gets an all-zero b_lo plane; a_lo != NULL with b_lo == NULL is an error.  Returns 2 and does nothing when the shape is not covered (d % 4 != 0,
  * d > 128, unaligned rows, or too few rows for an unsplit column range): run ise_prepare_rows + ise_gemm_select then.
  * Replaces `X.astype(np.float32)` + index.search(X, 1) of FaissKMeans.transform (kmeans_faiss.py:49). */
 int ise_assign_fused(ise_ctx* ctx, const float* x, int64_t ldx, int64_t m, int d,
