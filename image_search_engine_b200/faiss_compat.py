@@ -412,12 +412,190 @@ class IndexIVFPQ:
                 f"ntotal={self.ntotal} (HBM resident)>")
 
 
+class IndexIVFFlat:
+    """faiss.IndexIVFFlat (faiss/IndexIVFFlat.cpp, ~1.7.4): an inverted file whose lists hold the raw FP32 vectors, so
+    a search scans only the ``nprobe`` probed lists yet returns exact FP32 distances.
+
+    Training is the level-1 clustering of ``IndexIVFPQ`` (niter 10, seed 1234, spherical for inner product); vectors
+    go to their quantizer top-1 list; a search probes ``min(nprobe, nlist)`` lists through the quantizer and scans
+    them with ``ise_ivfflat_search`` (pairs grouped by list, exact FP32 scan, canonical merge).  Storage is one
+    list-sorted FP32 copy of the vectors with their ids and list offsets; rows added since the last search are merged
+    into it lazily at the next search.
+
+    Ties: among exactly equal distances the lowest ids win (the flat index's canonical (distance, id) order, SURVEY
+    Q5).  Faiss's heap keeps the first-scanned candidate when a tie falls exactly on the k-th place, which can be a
+    higher id from an earlier-probed list; this index deliberately returns the canonical order instead.
+    """
+
+    def __init__(self, quantizer, d, nlist, metric=METRIC_L2):
+        """IndexIVF::IndexIVF: the index is trained when the quantizer already holds nlist centroids."""
+        if int(metric) not in (METRIC_L2, METRIC_INNER_PRODUCT):
+            raise NotImplementedError("IndexIVFFlat supports METRIC_L2 and METRIC_INNER_PRODUCT")
+        if quantizer.d != int(d):
+            raise RuntimeError(f"quantizer dimension {quantizer.d} differs from the index dimension {int(d)}")
+        self.quantizer, self.d, self.nlist, self.metric_type = quantizer, int(d), int(nlist), int(metric)
+        self.nprobe = 1
+        self.is_trained = quantizer.ntotal == self.nlist
+        self._lock = threading.RLock()
+        self._clear()
+
+    def _clear(self) -> None:
+        self._xs = self._ids = self._off = None     # list-sorted vectors, their ids, list offsets [nlist + 1] (device)
+        self._sizes = np.zeros(self.nlist, np.int64)   # host copy of the list sizes
+        self._pending = []                              # (vectors, list numbers, ids) added since the last search
+        self._ntotal = 0
+
+    @property
+    def ntotal(self) -> int:
+        return self._ntotal
+
+    def train(self, x) -> None:
+        """Level1Quantizer::train_q1: k-means (niter 10, seed 1234, <= 256 points per centroid, spherical for inner
+        product) unless the quantizer already holds nlist centroids; the centroids replace the quantizer's content."""
+        xd, _ = _to_device(x)
+        if xd.shape[1] != self.d:
+            raise AssertionError(f"train: expected (n, {self.d}) array")
+        if self.quantizer.ntotal != self.nlist:
+            km = Kmeans(self.d, self.nlist, niter=10, seed=1234, spherical=self.metric_type == METRIC_INNER_PRODUCT)
+            km.train(xd)
+            self.quantizer.reset()
+            self.quantizer.add(km.index._database())
+        self.is_trained = True
+
+    def add(self, x) -> None:
+        """IndexIVF::add_with_ids(n, x, nullptr): ids ntotal + i, list = the quantizer's top-1 (lowest id on ties)."""
+        if not self.is_trained:
+            raise RuntimeError("Error: 'is_trained' failed")
+        xd, _ = _to_device(x)
+        if xd.shape[1] != self.d:
+            raise AssertionError(f"add: expected (n, {self.d}) array")
+        xd = xd.to(torch.float32)
+        _, assign = self.quantizer._search_device(xd, 1, need_distances=False)
+        self.add_preassigned(xd, assign.reshape(-1))
+
+    def add_preassigned(self, x, list_nos) -> None:
+        """IndexIVF::add_core with precomputed_idx: appends x (ids ntotal + i) to the given lists, in order."""
+        if not self.is_trained:
+            raise RuntimeError("Error: 'is_trained' failed")
+        xd, was_cuda = _to_device(x)
+        if xd.shape[1] != self.d:
+            raise AssertionError(f"add: expected (n, {self.d}) array")
+        xd = xd.to(torch.float32)
+        if was_cuda and xd.data_ptr() == x.data_ptr():
+            xd = xd.clone()
+        lists = torch.as_tensor(np.asarray(list_nos) if not isinstance(list_nos, torch.Tensor) else list_nos)
+        lists = lists.to(device=xd.device, dtype=torch.int64).reshape(-1)
+        if lists.shape[0] != xd.shape[0]:
+            raise AssertionError("add_preassigned: one list number per vector")
+        if lists.shape[0] and not (0 <= int(lists.min()) and int(lists.max()) < self.nlist):
+            raise AssertionError(f"add_preassigned: list numbers must lie in [0, {self.nlist})")
+        sizes = torch.bincount(lists, minlength=self.nlist).cpu().numpy()
+        with self._lock:
+            ids = torch.arange(self._ntotal, self._ntotal + xd.shape[0], dtype=torch.int64, device=xd.device)
+            self._pending.append((xd.contiguous(), lists, ids))
+            self._sizes += sizes
+            self._ntotal += xd.shape[0]
+
+    def _lists(self):
+        """Merges the pending rows into the list-sorted storage (stable by list: ids keep ascending in every list)."""
+        with self._lock:
+            if self._pending:
+                dev = self._pending[0][0].device
+                old = self._xs is not None
+                parts_l = [torch.repeat_interleave(torch.arange(self.nlist, device=dev), torch.diff(self._off))] if old else []
+                parts_l += [p[1] for p in self._pending]
+                order = torch.argsort(torch.cat(parts_l), stable=True)
+                dest = torch.empty_like(order)
+                dest[order] = torch.arange(order.shape[0], device=dev)
+                xs = torch.empty((self._ntotal, self.d), dtype=torch.float32, device=dev)
+                ids = torch.empty((self._ntotal,), dtype=torch.int64, device=dev)
+                r0 = 0
+                for rows, row_ids in ([(self._xs, self._ids)] if old else []) + [(p[0], p[2]) for p in self._pending]:
+                    pos = dest[r0:r0 + rows.shape[0]]
+                    xs.index_copy_(0, pos, rows)
+                    ids.index_copy_(0, pos, row_ids)
+                    r0 += rows.shape[0]
+                off = np.zeros(self.nlist + 1, np.int64)
+                np.cumsum(self._sizes, out=off[1:])
+                self._xs, self._ids, self._off = xs, ids, torch.from_numpy(off).to(dev)
+                self._pending = []
+            return self._xs, self._ids, self._off
+
+    def search(self, x, k: int):
+        """IndexIVF::search: probe min(nprobe, nlist) lists, exact FP32 scan (IVFFlatScanner: fvec_inner_product /
+        fvec_L2sqr), top-k in the canonical (distance, id) order; padding id -1 / -+FLT_MAX."""
+        k = int(k)
+        if k <= 0:
+            raise AssertionError("k must be positive")
+        if k > ops.MAX_TOPK:
+            raise NotImplementedError(f"IndexIVFFlat.search supports k <= {ops.MAX_TOPK}")
+        q, was_cuda = _to_device(x)
+        if q.shape[1] != self.d:
+            raise AssertionError(f"search: expected (n, {self.d}) array")
+        q = q.to(torch.float32).contiguous()
+        nq = q.shape[0]
+        if nq and self._ntotal and self.is_trained:
+            xs, ids, off = self._lists()
+            _, probes = self.quantizer._search_device(q, min(self.nprobe, self.nlist), need_distances=False)
+            D, I = ops.ivfflat_search(q, xs, ids, off, int(self._sizes.max()), probes, self.metric_type, k)
+        else:
+            pad = -_FLT_MAX if self.metric_type == METRIC_INNER_PRODUCT else _FLT_MAX
+            D = torch.full((nq, k), pad, dtype=torch.float32, device=q.device)
+            I = torch.full((nq, k), -1, dtype=torch.int64, device=q.device)
+        if was_cuda:
+            return D, I
+        return D.cpu().numpy(), I.cpu().numpy()
+
+    def reset(self) -> None:
+        with self._lock:
+            self._clear()
+
+    def get_list_size(self, list_no: int) -> int:
+        return int(self._sizes[int(list_no)])
+
+    def get_list_ids(self, list_no: int) -> np.ndarray:
+        """Ids stored in one list, in list order (InvertedLists::get_ids)."""
+        _, ids, off = self._lists() if self._ntotal else (None, None, None)
+        if ids is None:
+            return np.zeros(0, np.int64)
+        l = int(list_no)
+        return ids[int(off[l]):int(off[l + 1])].cpu().numpy()
+
+    # joblib / pickle: trained state, vectors and list numbers in insertion order (host arrays)
+    def __getstate__(self):
+        st = dict(d=self.d, nlist=self.nlist, metric_type=self.metric_type, nprobe=self.nprobe,
+                  quantizer_metric=self.quantizer.metric_type, is_trained=self.is_trained,
+                  coarse=self.quantizer.reconstruct_n(), xb=None, assign=None)
+        if self._ntotal:
+            xs, ids, off = self._lists()
+            xb = torch.empty_like(xs)
+            xb[ids] = xs
+            assign = torch.empty_like(ids)
+            assign[ids] = torch.repeat_interleave(torch.arange(self.nlist, device=ids.device), torch.diff(off))
+            st["xb"], st["assign"] = xb.cpu().numpy(), assign.cpu().numpy()
+        return st
+
+    def __setstate__(self, st):
+        quantizer = IndexFlat(st["d"], st["quantizer_metric"])
+        if st["coarse"].shape[0]:
+            quantizer.add(st["coarse"])
+        self.__init__(quantizer, st["d"], st["nlist"], st["metric_type"])
+        self.nprobe, self.is_trained = st["nprobe"], st["is_trained"]
+        if st["xb"] is not None:
+            self.add_preassigned(st["xb"], st["assign"])
+
+    def __repr__(self):
+        return (f"<image_search_engine_b200.IndexIVFFlat d={self.d} nlist={self.nlist} nprobe={self.nprobe} "
+                f"ntotal={self.ntotal} (HBM resident)>")
+
+
 # ------------------------------------------------------------------------------------------
 # flat index file format (faiss/impl/index_write.cpp), so existing models/*.faiss files open
 # ------------------------------------------------------------------------------------------
 def write_index(index: IndexFlat, fname) -> None:
-    if isinstance(index, IndexIVFPQ):
-        raise NotImplementedError("only flat indexes are written in Faiss's file format; an IndexIVFPQ can be pickled")
+    if isinstance(index, (IndexIVFPQ, IndexIVFFlat)):
+        name = type(index).__name__
+        raise NotImplementedError(f"only flat indexes are written in Faiss's file format; an {name} can be pickled")
     xb = index.reconstruct_n() if index.ntotal else np.zeros((0, index.d), np.float32)
     fourcc = b"IxFI" if index.metric_type == METRIC_INNER_PRODUCT else b"IxF2"
     with open(str(fname), "wb") as f:

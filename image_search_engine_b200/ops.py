@@ -818,6 +818,45 @@ def ivfpq_scan(q: torch.Tensor, coarse: torch.Tensor, probes: torch.Tensor, pq_c
 
 
 # ------------------------------------------------------------------------------------------
+# IVFFlat
+# ------------------------------------------------------------------------------------------
+def ivfflat_search_workspace_bytes(nq: int, nprobe: int, nlist: int, max_list_len: int, topk: int) -> int:
+    """Device scratch of one ivfflat_search call (the formula is in include/ise.h)."""
+    return int(_lib.load().ise_ivfflat_search_workspace_bytes(_lib.ctx(torch.cuda.current_device()), int(nq),
+                                                                int(nprobe), int(nlist), int(max_list_len), int(topk)))
+
+
+def ivfflat_search(q: torch.Tensor, xs: torch.Tensor, ids: torch.Tensor, list_off: torch.Tensor, max_list_len: int,
+                   probes: torch.Tensor, metric: int, topk: int):
+    """Exact FP32 top-k of every query over the vectors of its probed lists (IndexIVFFlat.search): xs / ids grouped by
+    list (list l = rows list_off[l] .. list_off[l + 1], ids ascending inside a list), probes [nq, nprobe] int64."""
+    if q.dtype != torch.float32 or xs.dtype != torch.float32 or not q.is_contiguous() or not xs.is_contiguous():
+        raise IseError("ivfflat_search needs contiguous float32 queries and vectors")
+    if ids.dtype != torch.int64 or list_off.dtype != torch.int64 or probes.dtype != torch.int64:
+        raise IseError("ivfflat_search: ids, list offsets and probes are int64")
+    if not 1 <= topk <= MAX_TOPK:
+        raise IseError(f"topk must be in [1, {MAX_TOPK}]")
+    nq, d = q.shape
+    if xs.shape[1] != d or probes.shape[0] != nq:
+        raise IseError("ivfflat_search: inconsistent shapes")
+    nprobe, nlist = probes.shape[1], list_off.shape[0] - 1
+    val = torch.empty((nq, topk), dtype=torch.float32, device=q.device)
+    idx = torch.empty((nq, topk), dtype=torch.int64, device=q.device)
+    if nq == 0:
+        return val, idx
+    lib, ctx = _lib.load(), _lib.ctx(_dev(q))
+    ws_bytes = lib.ise_ivfflat_search_workspace_bytes(ctx, nq, nprobe, nlist, int(max_list_len), int(topk))
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=q.device)
+    probes = probes.contiguous()
+    list_off = list_off.contiguous()
+    _lib.check(lib.ise_ivfflat_search(ctx, _ptr(q), nq, d, _ptr(xs), _ptr(ids.contiguous()), _ptr(list_off), nlist,
+                                      int(max_list_len), _ptr(probes), nprobe, int(metric), int(topk), _ptr(val),
+                                      _ptr(idx), _ptr(ws), ws_bytes, _stream()))
+    _count(6)
+    return val, idx
+
+
+# ------------------------------------------------------------------------------------------
 # k-means update
 # ------------------------------------------------------------------------------------------
 def kmeans_accumulate(x: torch.Tensor, assign: torch.Tensor, dis: torch.Tensor | None, sums: torch.Tensor,

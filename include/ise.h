@@ -386,6 +386,26 @@ int ise_ivfpq_scan(ise_ctx* ctx, const float* q, int64_t nq, int d, const float*
                    const int64_t* probes, int nprobe, const float* pq_centroids, int M, int ksub,
                    const uint8_t* codes, const int64_t* list_offsets, int64_t ntotal, float* dist, void* stream);
 
+/* ---- IVFFlat index (faiss/IndexIVFFlat.cpp IndexIVFFlat::search_preassigned, IVFFlatScanner) ----------------------
+ * Exact FP32 top-k over the vectors of the probed inverted lists, scored with Faiss's scanner formulas (IP: sum x*y,
+ * L2: sum (x - y)^2, no norm expansion); no [nq, ntotal] matrix is built.  q[nq, d] float32 rows; xs_sorted[ntotal, d]
+ * the vectors grouped by list, list l = rows list_off[l] .. list_off[l + 1] (list_off: int64[nlist + 1]) with ids
+ * ids_sorted[] ascending inside every list; max_list_len = the longest list (host value, sizes the workspace);
+ * probes[nq, nprobe] int64 list ids from the quantizer (-1 = none).  out[nq, topk] sorted best-first in the canonical
+ * (distance, id) order over the scanned vectors, padded with id -1 / -+FLT_MAX.  Pairs are grouped by list on the
+ * device (radix sort), scanned in (list, query block, vector chunk) work items and the partial lists merged with
+ * ise_topk_merge; no host synchronisation.  Workspace (ise_ivfflat_search_workspace_bytes) is
+ * O(nq * nprobe * topk + nlist): 12 bytes per partial-list entry, at most max(2^24, nq nprobe topk) entries plus
+ * 1/256 of that for the merge levels, 16 bytes per (query, probe) pair and 24 per list for the grouping, and CUB's
+ * sort / scan scratch.  topk <= 128, nq * nprobe < 2^31.  The reference builds no IVFFlat; IndexIVFFlat is Faiss's exact
+ * counterpart of its IndexIVFPQ (utils.py:311-325). */
+size_t ise_ivfflat_search_workspace_bytes(ise_ctx* ctx, int64_t nq, int nprobe, int64_t nlist, int64_t max_list_len,
+                                          int topk);
+int ise_ivfflat_search(ise_ctx* ctx, const float* q, int64_t nq, int d, const float* xs_sorted,
+                       const int64_t* ids_sorted, const int64_t* list_off, int64_t nlist, int64_t max_list_len,
+                       const int64_t* probes, int nprobe, int metric, int topk, float* out_val, int64_t* out_idx,
+                       void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- collectives for a single-process multi-GPU host (NCCL over NVLink, resolved with dlopen at run time) ----------
  * The two exchange steps of the sharded path (SURVEY section 8e): the per-iteration all-reduce of the k-means
  * [k*d sums | k counts] buffer and the all-gather of per-shard top-k lists before ise_topk_merge.  The Python host
