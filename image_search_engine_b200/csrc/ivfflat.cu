@@ -15,6 +15,15 @@
 // Chunking the vectors keeps a long list from serialising onto one CTA and lets a single query (nq = 1) fill more
 // than nprobe CTAs.  S is capped at 256 / nprobe (one merge level while nprobe <= 256) and so that the partial lists
 // hold at most max(2^24, nq * nprobe * topk) entries.
+//
+// Range search (faiss/IndexIVF.cpp range_search_preassigned, IVFFlatScanner::scan_codes_range) reuses the grouping and
+// the work items, and replaces the top-k with two passes over the same score tiles:
+//   ivfflat_range_count_kernel   hits of every (pair, chunk) segment, cnt[(q * nprobe + slot) * S + c] (query-major,
+//                                so one exclusive scan (ise_range_lims) gives every segment its output offset in
+//                                Faiss's order: probe rank, then list position); lims[q] = offset of segment (q, 0, 0);
+//   ivfflat_range_fill_kernel    re-runs the items with hits and writes each segment's hits in list order.
+// Every kernel scores through score_tile, so search and range search return bit-identical distances.  S is capped at
+// 256 / nprobe and so that the segment table holds at most max(2^22, nq * nprobe) entries.
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
@@ -30,7 +39,9 @@ constexpr int kCB = 64;             // vectors per score tile
 constexpr int kDK = 32;             // dimensions per shared-memory slice
 constexpr int kThreads = 128;       // 16 x 8 threads, 4 x 4 scores each
 constexpr int kMergeFanIn = 256;    // ise_topk_merge: at most 256 lists per row
+constexpr int kWarps = kThreads / 32;
 constexpr int64_t kPartialBudget = int64_t(1) << 24;
+constexpr int64_t kSegmentBudget = int64_t(1) << 22;   // range search: (pair, chunk) segments
 
 static inline size_t align256(size_t b) { return (b + 255) & ~size_t(255); }
 
@@ -48,7 +59,7 @@ __global__ void ivf_probe_keys_kernel(const int64_t* __restrict__ probes, int64_
         const bool ok = l >= 0 && l < nlist;
         keys[i] = ok ? (int32_t)l : (int32_t)nlist;
         vals[i] = (int32_t)i;
-        if (!ok)
+        if (!ok && part_idx)
             for (int c = 0; c < S; ++c) part_idx[(((i % nprobe) * S + c) * nq + i / nprobe) * topk] = -1;
     }
 }
@@ -91,6 +102,96 @@ __device__ __forceinline__ float4 load4(const float* __restrict__ row, int c, in
     return v;
 }
 
+struct Item {
+    int64_t lbase, nch, c;              // first row of the list, its chunks, this item's chunk
+    int64_t v_begin, v_end;             // the chunk's vectors, in list positions
+};
+
+// work item w of the persistent loop: its list (item_off[l] <= w < item_off[l + 1]), query block and vector chunk; the
+// block's pairs go to s_pair (-1 past the block).  The caller synchronises before reading s_pair.
+__device__ __forceinline__ Item decode_item(int64_t w, const int64_t* __restrict__ list_off, int64_t nlist,
+                                            const int32_t* __restrict__ pairs_sorted, const int32_t* __restrict__ qoff,
+                                            const int64_t* __restrict__ item_off, int S, int tid, int* s_pair) {
+    int64_t lo = 0, hi = nlist;
+    while (hi - lo > 1) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (item_off[mid] <= w) lo = mid;
+        else hi = mid;
+    }
+    const int64_t l = lo;
+    Item it;
+    it.lbase = list_off[l];
+    const int64_t len = list_off[l + 1] - it.lbase;
+    const int64_t nch = list_chunks(len, S);
+    const int64_t local = w - item_off[l];
+    const int64_t qb = local / nch;
+    it.nch = nch;
+    it.c = local % nch;
+    const int64_t p0 = qoff[l] + qb * kQB;
+    const int nqb = (int)min((int64_t)kQB, (int64_t)qoff[l + 1] - p0);
+    if (tid < kQB) s_pair[tid] = tid < nqb ? pairs_sorted[p0 + tid] : -1;
+    const int64_t cl = (len + nch - 1) / nch;
+    it.v_begin = min(len, it.c * cl);
+    it.v_end = min(len, it.v_begin + cl);
+    return it;
+}
+
+// s_s[r][j] = score of pair s_pair[r] against list vector t0 + j (r < kQB, j < nv) with the direct formulas: one
+// sequential fmaf chain over the dimensions per (query, vector), sum x*y or sum (x-y)^2, zeros past d.  The queries
+// and kCB vectors go through shared memory kDK dimensions at a time; each thread accumulates a 4 x 4 piece of the
+// tile.  Search and both range passes score through this function only, so they see the same bits.
+template <bool L2>
+__device__ __forceinline__ void score_tile(int tid, const float* __restrict__ q, int d, bool vec, int nprobe,
+                                           const int* s_pair, const float* __restrict__ xl, int64_t t0, int nv,
+                                           float (*s_q)[kQB], float (*s_x)[kCB], float (*s_s)[kCB + 1]) {
+    const int tx = tid & 15, ty = tid >> 4;
+    float acc[4][4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
+    for (int d0 = 0; d0 < d; d0 += kDK) {
+        for (int e = tid; e < kQB * (kDK / 4); e += kThreads) {
+            const int r = e / (kDK / 4), c4 = (e % (kDK / 4)) * 4;
+            const int pr = s_pair[r];
+            const float4 v = load4(pr >= 0 ? q + (int64_t)(pr / nprobe) * d : nullptr, d0 + c4, d, vec);
+            s_q[c4][r] = v.x; s_q[c4 + 1][r] = v.y; s_q[c4 + 2][r] = v.z; s_q[c4 + 3][r] = v.w;
+        }
+        for (int e = tid; e < kCB * (kDK / 4); e += kThreads) {
+            const int r = e / (kDK / 4), c4 = (e % (kDK / 4)) * 4;
+            const float4 v = load4(r < nv ? xl + (t0 + r) * d : nullptr, d0 + c4, d, vec);
+            s_x[c4][r] = v.x; s_x[c4 + 1][r] = v.y; s_x[c4 + 2][r] = v.z; s_x[c4 + 3][r] = v.w;
+        }
+        __syncthreads();
+#pragma unroll
+        for (int kk = 0; kk < kDK; ++kk) {
+            const float4 a4 = *reinterpret_cast<const float4*>(&s_q[kk][ty * 4]);
+            const float4 b4 = *reinterpret_cast<const float4*>(&s_x[kk][tx * 4]);
+            const float a[4] = {a4.x, a4.y, a4.z, a4.w}, b[4] = {b4.x, b4.y, b4.z, b4.w};
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    if (L2) {
+                        const float t = a[i] - b[j];
+                        acc[i][j] = fmaf(t, t, acc[i][j]);
+                    } else {
+                        acc[i][j] = fmaf(a[i], b[j], acc[i][j]);
+                    }
+                }
+        }
+        __syncthreads();
+    }
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) s_s[ty * 4 + i][tx * 4 + j] = acc[i][j];
+    __syncthreads();
+}
+
+template <bool L2>
+__device__ __forceinline__ bool in_range(float s, float radius) { return L2 ? s < radius : s > radius; }
+
 template <bool L2, int KMAX>
 __global__ void __launch_bounds__(kThreads) ivfflat_scan_kernel(
         const float* __restrict__ q, int64_t nq, int d, bool vec, const float* __restrict__ xs,
@@ -103,7 +204,7 @@ __global__ void __launch_bounds__(kThreads) ivfflat_scan_kernel(
     __shared__ float s_s[kQB][kCB + 1];
     __shared__ int s_pair[kQB];
     __shared__ long long s_item;
-    const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
+    const int tid = threadIdx.x;
     const int sq = tid >> 2, sub = tid & 3;          // selection: four threads per query row of the tile
     const int64_t total = item_off[nlist];
     const float pad = L2 ? 3.402823466e+38f : -3.402823466e+38f;
@@ -112,71 +213,16 @@ __global__ void __launch_bounds__(kThreads) ivfflat_scan_kernel(
         __syncthreads();
         const int64_t w = s_item;
         if (w >= total) break;
-        int64_t lo = 0, hi = nlist;                  // item_off[lo] <= w < item_off[hi]
-        while (hi - lo > 1) {
-            const int64_t mid = (lo + hi) >> 1;
-            if (item_off[mid] <= w) lo = mid;
-            else hi = mid;
-        }
-        const int64_t l = lo;
-        const int64_t lbase = list_off[l], len = list_off[l + 1] - lbase;
-        const int64_t nch = list_chunks(len, S);
-        const int64_t local = w - item_off[l];
-        const int64_t qb = local / nch, c = local % nch;
-        const int64_t p0 = qoff[l] + qb * kQB;
-        const int nqb = (int)min((int64_t)kQB, (int64_t)qoff[l + 1] - p0);
-        if (tid < kQB) s_pair[tid] = tid < nqb ? pairs_sorted[p0 + tid] : -1;
-        const int64_t cl = (len + nch - 1) / nch;
-        const int64_t v_begin = min(len, c * cl), v_end = min(len, v_begin + cl);
+        const Item it = decode_item(w, list_off, nlist, pairs_sorted, qoff, item_off, S, tid, s_pair);
+        const int64_t lbase = it.lbase, c = it.c;
         const float* xl = xs + lbase * (int64_t)d;
         __syncthreads();
 
         TopKList<KMAX> list;
         list.init(topk);
-        for (int64_t t0 = v_begin; t0 < v_end; t0 += kCB) {
-            const int nv = (int)min((int64_t)kCB, v_end - t0);
-            float acc[4][4];
-#pragma unroll
-            for (int i = 0; i < 4; ++i)
-#pragma unroll
-                for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
-            for (int d0 = 0; d0 < d; d0 += kDK) {
-                for (int e = tid; e < kQB * (kDK / 4); e += kThreads) {
-                    const int r = e / (kDK / 4), c4 = (e % (kDK / 4)) * 4;
-                    const int pr = s_pair[r];
-                    const float4 v = load4(pr >= 0 ? q + (int64_t)(pr / nprobe) * d : nullptr, d0 + c4, d, vec);
-                    s_q[c4][r] = v.x; s_q[c4 + 1][r] = v.y; s_q[c4 + 2][r] = v.z; s_q[c4 + 3][r] = v.w;
-                }
-                for (int e = tid; e < kCB * (kDK / 4); e += kThreads) {
-                    const int r = e / (kDK / 4), c4 = (e % (kDK / 4)) * 4;
-                    const float4 v = load4(r < nv ? xl + (t0 + r) * d : nullptr, d0 + c4, d, vec);
-                    s_x[c4][r] = v.x; s_x[c4 + 1][r] = v.y; s_x[c4 + 2][r] = v.z; s_x[c4 + 3][r] = v.w;
-                }
-                __syncthreads();
-#pragma unroll
-                for (int kk = 0; kk < kDK; ++kk) {
-                    const float4 a4 = *reinterpret_cast<const float4*>(&s_q[kk][ty * 4]);
-                    const float4 b4 = *reinterpret_cast<const float4*>(&s_x[kk][tx * 4]);
-                    const float a[4] = {a4.x, a4.y, a4.z, a4.w}, b[4] = {b4.x, b4.y, b4.z, b4.w};
-#pragma unroll
-                    for (int i = 0; i < 4; ++i)
-#pragma unroll
-                        for (int j = 0; j < 4; ++j) {
-                            if (L2) {
-                                const float t = a[i] - b[j];
-                                acc[i][j] = fmaf(t, t, acc[i][j]);
-                            } else {
-                                acc[i][j] = fmaf(a[i], b[j], acc[i][j]);
-                            }
-                        }
-                }
-                __syncthreads();
-            }
-#pragma unroll
-            for (int i = 0; i < 4; ++i)
-#pragma unroll
-                for (int j = 0; j < 4; ++j) s_s[ty * 4 + i][tx * 4 + j] = acc[i][j];
-            __syncthreads();
+        for (int64_t t0 = it.v_begin; t0 < it.v_end; t0 += kCB) {
+            const int nv = (int)min((int64_t)kCB, it.v_end - t0);
+            score_tile<L2>(tid, q, d, vec, nprobe, s_pair, xl, t0, nv, s_q, s_x, s_s);
             if (s_pair[sq] >= 0) {
                 // ascending column per thread: the strict insert keeps the lower position (= lower id) on ties
                 for (int j = sub; j < nv; j += 4) {
@@ -211,27 +257,161 @@ __global__ void __launch_bounds__(kThreads) ivfflat_scan_kernel(
             }
         }
         // chunk slots this list does not use: an id -1 at the head makes ise_topk_merge skip the list
-        if (sub == 0 && pair >= 0 && c == nch - 1)
-            for (int64_t c2 = nch; c2 < S; ++c2) part_idx[((slot * S + c2) * nq + qi) * topk] = -1;
+        if (sub == 0 && pair >= 0 && c == it.nch - 1)
+            for (int64_t c2 = it.nch; c2 < S; ++c2) part_idx[((slot * S + c2) * nq + qi) * topk] = -1;
         __syncthreads();
     }
 }
 
+// range pass 1: cnt[pair * S + c] = hits (strict radius test) of pair against chunk c of its list.  Segments of probe
+// -1 and chunk slots a list does not use keep the zero the caller wrote.  A warp takes rows warp, warp + kWarps, ...
+// of the tile and counts 32 columns per ballot.
+template <bool L2>
+__global__ void __launch_bounds__(kThreads) ivfflat_range_count_kernel(
+        const float* __restrict__ q, int d, bool vec, const float* __restrict__ xs,
+        const int64_t* __restrict__ list_off, int64_t nlist, const int32_t* __restrict__ pairs_sorted,
+        const int32_t* __restrict__ qoff, const int64_t* __restrict__ item_off, int nprobe, int S, float radius,
+        unsigned long long* __restrict__ counter, int64_t* __restrict__ cnt) {
+    __shared__ __align__(16) float s_q[kDK][kQB];
+    __shared__ __align__(16) float s_x[kDK][kCB];
+    __shared__ float s_s[kQB][kCB + 1];
+    __shared__ int s_pair[kQB];
+    __shared__ long long s_item;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int64_t total = item_off[nlist];
+    for (;;) {
+        if (tid == 0) s_item = (long long)atomicAdd(counter, 1ull);
+        __syncthreads();
+        const int64_t w = s_item;
+        if (w >= total) break;
+        const Item it = decode_item(w, list_off, nlist, pairs_sorted, qoff, item_off, S, tid, s_pair);
+        const float* xl = xs + it.lbase * (int64_t)d;
+        __syncthreads();
+        int hits[kQB / kWarps];
+#pragma unroll
+        for (int i = 0; i < kQB / kWarps; ++i) hits[i] = 0;
+        for (int64_t t0 = it.v_begin; t0 < it.v_end; t0 += kCB) {
+            const int nv = (int)min((int64_t)kCB, it.v_end - t0);
+            score_tile<L2>(tid, q, d, vec, nprobe, s_pair, xl, t0, nv, s_q, s_x, s_s);
+#pragma unroll
+            for (int i = 0; i < kQB / kWarps; ++i) {
+                const int r = warp + i * kWarps;
+#pragma unroll
+                for (int h = 0; h < kCB; h += 32) {
+                    const int j = h + lane;
+                    hits[i] += __popc(__ballot_sync(0xffffffffu, j < nv && in_range<L2>(s_s[r][j], radius)));
+                }
+            }
+            __syncthreads();
+        }
+        if (lane == 0) {
+#pragma unroll
+            for (int i = 0; i < kQB / kWarps; ++i) {
+                const int pair = s_pair[warp + i * kWarps];
+                if (pair >= 0) cnt[(int64_t)pair * S + it.c] = hits[i];
+            }
+        }
+        __syncthreads();
+    }
+}
+
+// range pass 2: the hits of segment (pair, c) go to out[offs[seg] .. offs[seg + 1]) in list position order.  An item
+// whose segments are all empty is skipped before any vector is loaded, and a chunk stops once every segment is full.
+// Each row has a cursor (s_cur, owned by the warp of the row); a ballot over 32 columns and popc prefixes give the
+// slots.  Writes are bounded by the segment end.
+template <bool L2>
+__global__ void __launch_bounds__(kThreads) ivfflat_range_fill_kernel(
+        const float* __restrict__ q, int d, bool vec, const float* __restrict__ xs, const int64_t* __restrict__ ids,
+        const int64_t* __restrict__ list_off, int64_t nlist, const int32_t* __restrict__ pairs_sorted,
+        const int32_t* __restrict__ qoff, const int64_t* __restrict__ item_off, int nprobe, int S, float radius,
+        unsigned long long* __restrict__ counter, const int64_t* __restrict__ offs, float* __restrict__ out_dis,
+        int64_t* __restrict__ out_ids) {
+    __shared__ __align__(16) float s_q[kDK][kQB];
+    __shared__ __align__(16) float s_x[kDK][kCB];
+    __shared__ float s_s[kQB][kCB + 1];
+    __shared__ int s_pair[kQB];
+    __shared__ long long s_item;
+    __shared__ long long s_cur[kQB], s_end[kQB];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const unsigned below = (1u << lane) - 1u;
+    const int64_t total = item_off[nlist];
+    for (;;) {
+        if (tid == 0) s_item = (long long)atomicAdd(counter, 1ull);
+        __syncthreads();
+        const int64_t w = s_item;
+        if (w >= total) break;
+        const Item it = decode_item(w, list_off, nlist, pairs_sorted, qoff, item_off, S, tid, s_pair);
+        const float* xl = xs + it.lbase * (int64_t)d;
+        const int64_t* il = ids + it.lbase;
+        __syncthreads();
+        bool left = false;
+#pragma unroll
+        for (int i = 0; i < kQB / kWarps; ++i) {
+            const int r = warp + i * kWarps;
+            const int pair = s_pair[r];
+            const int64_t seg = (int64_t)pair * S + it.c;
+            const int64_t b = pair >= 0 ? offs[seg] : 0, e = pair >= 0 ? offs[seg + 1] : 0;
+            if (lane == 0) { s_cur[r] = b; s_end[r] = e; }
+            left |= b < e;
+        }
+        if (!__syncthreads_or(left)) continue;
+        for (int64_t t0 = it.v_begin; t0 < it.v_end; t0 += kCB) {
+            const int nv = (int)min((int64_t)kCB, it.v_end - t0);
+            score_tile<L2>(tid, q, d, vec, nprobe, s_pair, xl, t0, nv, s_q, s_x, s_s);
+            left = false;
+#pragma unroll
+            for (int i = 0; i < kQB / kWarps; ++i) {
+                const int r = warp + i * kWarps;
+                int64_t cur = s_cur[r];
+                const int64_t e = s_end[r];
+                if (cur < e) {                                   // warp-uniform
+#pragma unroll
+                    for (int h = 0; h < kCB; h += 32) {
+                        const int j = h + lane;
+                        const float s = s_s[r][j];
+                        const bool hit = j < nv && in_range<L2>(s, radius);
+                        const unsigned m = __ballot_sync(0xffffffffu, hit);
+                        const int64_t pos = cur + __popc(m & below);
+                        if (hit && pos < e) {
+                            out_dis[pos] = s;
+                            out_ids[pos] = il[t0 + j];
+                        }
+                        cur += __popc(m);
+                    }
+                    if (lane == 0) s_cur[r] = cur;
+                    left |= cur < e;
+                }
+            }
+            if (!__syncthreads_or(left)) break;
+        }
+    }
+}
+
+// lims[r] = offs[r * per_query], r = 0 .. nq (the first segment of query r; lims[nq] = the total)
+__global__ void ivf_range_lims_kernel(const int64_t* __restrict__ offs, int64_t nq, int64_t per_query,
+                                      int64_t* __restrict__ lims) {
+    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r <= nq) lims[r] = offs[r * per_query];
+}
+
 struct Plan {
-    int S;                 // chunks per list (partial-list slots per probe)
-    int64_t npairs, g;     // nq * nprobe; partial lists per query = nprobe * S
+    int S;                 // chunks per list (partial-list / segment slots per probe)
+    int64_t npairs, g;     // nq * nprobe; slots per query = nprobe * S
     int end_bit;           // radix-sort key bits (list ids 0 .. nlist)
-    size_t sort_tmp, scan_tmp, pairs, lists, parts, level;
+    size_t sort_tmp, scan_tmp, pairs, lists, grouping;
+    size_t parts, level;   // search: partial lists and merge levels
+    int64_t segs;          // range: nq * nprobe * S (pair, chunk) segments
+    size_t seg, lims_tmp;  // range: one int64 per segment + 1 (counts, offsets); ise_range_lims scratch
 };
 
-static Plan make_plan(int64_t nq, int nprobe, int64_t nlist, int64_t max_list_len, int topk) {
+// the (query, probe) grouping both searches share; S covers the longest list, stays <= 256 / nprobe and <= room
+static Plan make_plan(int64_t nq, int nprobe, int64_t nlist, int64_t max_list_len, int64_t room) {
     Plan p{};
     const int64_t need = std::max<int64_t>(1, ceil_div64(max_list_len, kCB));
-    const int64_t room = std::max<int64_t>(1, kPartialBudget / std::max<int64_t>(1, nq * nprobe * (int64_t)topk));
     // a query's nprobe * S partial lists fit one merge while nprobe <= 256: beyond 256 / nprobe chunks per list the
     // (list, query block) items already fill the machine and more chunks only add merge levels
     const int64_t one_merge = std::max<int64_t>(1, kMergeFanIn / nprobe);
-    p.S = (int)std::min({need, room, one_merge});
+    p.S = (int)std::min({need, std::max<int64_t>(1, room), one_merge});
     p.npairs = nq * nprobe;
     p.g = (int64_t)nprobe * p.S;
     p.end_bit = 1;
@@ -241,10 +421,24 @@ static Plan make_plan(int64_t nq, int nprobe, int64_t nlist, int64_t max_list_le
     cub::DeviceScan::ExclusiveSum(nullptr, p.scan_tmp, (const int64_t*)nullptr, (int64_t*)nullptr, (int)(nlist + 1));
     p.pairs = align256((size_t)p.npairs * sizeof(int32_t));
     p.lists = align256((size_t)(nlist + 1) * sizeof(int64_t));
+    p.grouping = 4 * p.pairs + align256(p.sort_tmp) + 3 * p.lists + align256(p.scan_tmp) + 256;
+    return p;
+}
+
+static Plan search_plan(int64_t nq, int nprobe, int64_t nlist, int64_t max_list_len, int topk) {
+    Plan p = make_plan(nq, nprobe, nlist, max_list_len, kPartialBudget / std::max<int64_t>(1, nq * nprobe * (int64_t)topk));
     const size_t entries = (size_t)p.g * nq * topk;
     p.parts = align256(entries * sizeof(float)) + align256(entries * sizeof(int64_t));
     const size_t lv = p.g > kMergeFanIn ? (size_t)ceil_div64(p.g, kMergeFanIn) * nq * topk : 0;
     p.level = align256(lv * sizeof(float)) + align256(lv * sizeof(int64_t));
+    return p;
+}
+
+static Plan range_plan(ise_ctx* ctx, int64_t nq, int nprobe, int64_t nlist, int64_t max_list_len) {
+    Plan p = make_plan(nq, nprobe, nlist, max_list_len, kSegmentBudget / std::max<int64_t>(1, nq * nprobe));
+    p.segs = p.g * nq;
+    p.seg = align256((size_t)(p.segs + 1) * sizeof(int64_t));
+    p.lims_tmp = align256(ise_range_lims_workspace_bytes(ctx, p.segs));
     return p;
 }
 
@@ -253,13 +447,75 @@ static bool plan_args_ok(int64_t nq, int nprobe, int64_t nlist, int64_t max_list
            topk <= 128 && nq * nprobe < ((int64_t)1 << 31);
 }
 
+struct Grouping {
+    int32_t *keys, *keys_sorted, *vals, *pairs_sorted, *qoff;
+    int64_t *items, *item_off;
+    void *sort_tmp, *scan_tmp;
+    unsigned long long* counter;   // next work item of the persistent kernels
+};
+
+static uint8_t* take(uint8_t*& w, size_t bytes) {
+    uint8_t* r = w;
+    w += bytes;
+    return r;
+}
+
+// the first p.grouping bytes of a workspace
+static Grouping carve_grouping(uint8_t*& w, const Plan& p) {
+    Grouping g;
+    g.keys = reinterpret_cast<int32_t*>(take(w, p.pairs));
+    g.keys_sorted = reinterpret_cast<int32_t*>(take(w, p.pairs));
+    g.vals = reinterpret_cast<int32_t*>(take(w, p.pairs));
+    g.pairs_sorted = reinterpret_cast<int32_t*>(take(w, p.pairs));
+    g.sort_tmp = take(w, align256(p.sort_tmp));
+    g.qoff = reinterpret_cast<int32_t*>(take(w, p.lists));
+    g.items = reinterpret_cast<int64_t*>(take(w, p.lists));
+    g.item_off = reinterpret_cast<int64_t*>(take(w, p.lists));
+    g.scan_tmp = take(w, align256(p.scan_tmp));
+    g.counter = reinterpret_cast<unsigned long long*>(take(w, 256));
+    return g;
+}
+
+// groups the (query, probe slot) pairs by list and numbers the work items; zeroes the item counter.  part_idx (search
+// only, else null): the partial lists of pairs without a list are marked empty.
+static int group_pairs(ise_ctx* ctx, const Plan& p, const Grouping& g, const int64_t* probes, int64_t nq, int nprobe,
+                       int64_t nlist, const int64_t* list_off, int topk, int64_t* part_idx, cudaStream_t st) {
+    ISE_CUDA(cudaMemsetAsync(g.counter, 0, sizeof(unsigned long long), st));
+    const int grid_pairs = (int)std::min<int64_t>(ceil_div64(p.npairs, 256), (int64_t)ctx->sm_count * 8);
+    ivf_probe_keys_kernel<<<grid_pairs, 256, 0, st>>>(probes, nq, nprobe, nlist, p.S, topk, g.keys, g.vals, part_idx);
+    ISE_LAUNCH_CHECK();
+    size_t sort_bytes = p.sort_tmp;
+    ISE_CUDA(cub::DeviceRadixSort::SortPairs(g.sort_tmp, sort_bytes, g.keys, g.keys_sorted, g.vals, g.pairs_sorted,
+                                             (int)p.npairs, 0, p.end_bit, st));
+    const int grid_lists = (int)std::min<int64_t>(ceil_div64(nlist + 1, 256), (int64_t)ctx->sm_count * 8);
+    ivf_list_items_kernel<<<grid_lists, 256, 0, st>>>(g.keys_sorted, p.npairs, list_off, nlist, p.S, g.qoff, g.items);
+    ISE_LAUNCH_CHECK();
+    size_t scan_bytes = p.scan_tmp;
+    ISE_CUDA(cub::DeviceScan::ExclusiveSum(g.scan_tmp, scan_bytes, g.items, g.item_off, (int)(nlist + 1), st));
+    return 0;
+}
+
+// persistent CTAs (as many as fit) that take work items from the counter: the item count stays on the device
+template <typename Kernel, typename... Args>
+static int launch_persistent(ise_ctx* ctx, cudaStream_t st, Kernel kernel, Args... args) {
+    int per_sm = 0;
+    ISE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, 0));
+    kernel<<<ctx->sm_count * std::max(per_sm, 1), kThreads, 0, st>>>(args...);
+    ISE_LAUNCH_CHECK();
+    return 0;
+}
+
+static bool vec_rows(const float* q, const float* xs, int d) {
+    return (d % 4 == 0) && ((reinterpret_cast<uintptr_t>(q) | reinterpret_cast<uintptr_t>(xs)) & 15) == 0;
+}
+
 }  // namespace
 
 ISE_EXPORT size_t ise_ivfflat_search_workspace_bytes(ise_ctx* ctx, int64_t nq, int nprobe, int64_t nlist,
                                                      int64_t max_list_len, int topk) {
     if (!ctx || !plan_args_ok(nq, nprobe, nlist, max_list_len, topk)) return 0;
-    const Plan p = make_plan(nq, nprobe, nlist, max_list_len, topk);
-    return 4 * p.pairs + align256(p.sort_tmp) + 3 * p.lists + align256(p.scan_tmp) + 256 + p.parts + p.level;
+    const Plan p = search_plan(nq, nprobe, nlist, max_list_len, topk);
+    return p.grouping + p.parts + p.level;
 }
 
 ISE_EXPORT int ise_ivfflat_search(ise_ctx* ctx, const float* q, int64_t nq, int d, const float* xs_sorted,
@@ -278,56 +534,33 @@ ISE_EXPORT int ise_ivfflat_search(ise_ctx* ctx, const float* q, int64_t nq, int 
     if (workspace_bytes < need) ISE_FAIL("workspace too small: need " + std::to_string(need));
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
-    const Plan p = make_plan(nq, nprobe, nlist, max_list_len, topk);
+    const Plan p = search_plan(nq, nprobe, nlist, max_list_len, topk);
 
     uint8_t* w = reinterpret_cast<uint8_t*>(workspace);
-    auto take = [&w](size_t bytes) { uint8_t* r = w; w += bytes; return r; };
-    int32_t* keys = reinterpret_cast<int32_t*>(take(p.pairs));
-    int32_t* keys_sorted = reinterpret_cast<int32_t*>(take(p.pairs));
-    int32_t* vals = reinterpret_cast<int32_t*>(take(p.pairs));
-    int32_t* pairs_sorted = reinterpret_cast<int32_t*>(take(p.pairs));
-    void* sort_tmp = take(align256(p.sort_tmp));
-    int32_t* qoff = reinterpret_cast<int32_t*>(take(p.lists));
-    int64_t* items = reinterpret_cast<int64_t*>(take(p.lists));
-    int64_t* item_off = reinterpret_cast<int64_t*>(take(p.lists));
-    void* scan_tmp = take(align256(p.scan_tmp));
-    unsigned long long* counter = reinterpret_cast<unsigned long long*>(take(256));
+    const Grouping gr = carve_grouping(w, p);
     const size_t entries = (size_t)p.g * nq * topk;
-    float* part_val = reinterpret_cast<float*>(take(align256(entries * sizeof(float))));
-    int64_t* part_idx = reinterpret_cast<int64_t*>(take(align256(entries * sizeof(int64_t))));
+    float* part_val = reinterpret_cast<float*>(take(w, align256(entries * sizeof(float))));
+    int64_t* part_idx = reinterpret_cast<int64_t*>(take(w, align256(entries * sizeof(int64_t))));
     const size_t lv = p.g > kMergeFanIn ? (size_t)ceil_div64(p.g, kMergeFanIn) * nq * topk : 0;
-    float* lvl_val = reinterpret_cast<float*>(take(align256(lv * sizeof(float))));
-    int64_t* lvl_idx = reinterpret_cast<int64_t*>(take(align256(lv * sizeof(int64_t))));
+    float* lvl_val = reinterpret_cast<float*>(take(w, align256(lv * sizeof(float))));
+    int64_t* lvl_idx = reinterpret_cast<int64_t*>(take(w, align256(lv * sizeof(int64_t))));
 
     // 1. group the (query, probe slot) pairs by list
-    ISE_CUDA(cudaMemsetAsync(counter, 0, sizeof(unsigned long long), st));
-    const int grid_pairs = (int)std::min<int64_t>(ceil_div64(p.npairs, 256), (int64_t)ctx->sm_count * 8);
-    ivf_probe_keys_kernel<<<grid_pairs, 256, 0, st>>>(probes, nq, nprobe, nlist, p.S, topk, keys, vals, part_idx);
-    ISE_LAUNCH_CHECK();
-    size_t sort_bytes = p.sort_tmp;
-    ISE_CUDA(cub::DeviceRadixSort::SortPairs(sort_tmp, sort_bytes, keys, keys_sorted, vals, pairs_sorted,
-                                             (int)p.npairs, 0, p.end_bit, st));
-    const int grid_lists = (int)std::min<int64_t>(ceil_div64(nlist + 1, 256), (int64_t)ctx->sm_count * 8);
-    ivf_list_items_kernel<<<grid_lists, 256, 0, st>>>(keys_sorted, p.npairs, list_off, nlist, p.S, qoff, items);
-    ISE_LAUNCH_CHECK();
-    size_t scan_bytes = p.scan_tmp;
-    ISE_CUDA(cub::DeviceScan::ExclusiveSum(scan_tmp, scan_bytes, items, item_off, (int)(nlist + 1), st));
+    int rc = group_pairs(ctx, p, gr, probes, nq, nprobe, nlist, list_off, topk, part_idx, st);
+    if (rc) return rc;
 
-    // 2. scan: persistent CTAs take work items from a counter (the item count stays on the device)
-    const bool vec = (d % 4 == 0) && ((reinterpret_cast<uintptr_t>(q) | reinterpret_cast<uintptr_t>(xs_sorted)) & 15) == 0;
+    // 2. scan: persistent CTAs take work items from a counter
+    const bool vec = vec_rows(q, xs_sorted, d);
     const bool l2 = metric == ISE_METRIC_L2;
-    auto launch = [&](auto kernel) -> int {
-        int per_sm = 0;
-        ISE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, 0));
-        kernel<<<ctx->sm_count * std::max(per_sm, 1), kThreads, 0, st>>>(
-            q, nq, d, vec, xs_sorted, ids_sorted, list_off, nlist, pairs_sorted, qoff, item_off, nprobe, p.S, topk,
-            counter, part_val, part_idx);
-        ISE_LAUNCH_CHECK();
-        return 0;
-    };
-    int rc;
-    if (topk <= 32) rc = l2 ? launch(ivfflat_scan_kernel<true, 32>) : launch(ivfflat_scan_kernel<false, 32>);
-    else rc = l2 ? launch(ivfflat_scan_kernel<true, 128>) : launch(ivfflat_scan_kernel<false, 128>);
+#define ISE_SCAN_ARGS q, nq, d, vec, xs_sorted, ids_sorted, list_off, nlist, gr.pairs_sorted, gr.qoff, gr.item_off, \
+                      nprobe, p.S, topk, gr.counter, part_val, part_idx
+    if (topk <= 32)
+        rc = l2 ? launch_persistent(ctx, st, ivfflat_scan_kernel<true, 32>, ISE_SCAN_ARGS)
+                : launch_persistent(ctx, st, ivfflat_scan_kernel<false, 32>, ISE_SCAN_ARGS);
+    else
+        rc = l2 ? launch_persistent(ctx, st, ivfflat_scan_kernel<true, 128>, ISE_SCAN_ARGS)
+                : launch_persistent(ctx, st, ivfflat_scan_kernel<false, 128>, ISE_SCAN_ARGS);
+#undef ISE_SCAN_ARGS
     if (rc) return rc;
 
     // 3. merge the nprobe * S partial lists of every query, at most kMergeFanIn at a time
@@ -350,4 +583,99 @@ ISE_EXPORT int ise_ivfflat_search(ise_ctx* ctx, const float* q, int64_t nq, int 
         g = g2;
     }
     return ise_topk_merge(ctx, src_val, src_idx, (int)g, nq, topk, metric, out_val, out_idx, stream);
+}
+
+ISE_EXPORT size_t ise_ivfflat_range_workspace_bytes(ise_ctx* ctx, int64_t nq, int nprobe, int64_t nlist,
+                                                    int64_t max_list_len) {
+    if (!ctx || !plan_args_ok(nq, nprobe, nlist, max_list_len, 1)) return 0;
+    const Plan p = range_plan(ctx, nq, nprobe, nlist, max_list_len);
+    return p.grouping + 2 * p.seg + p.lims_tmp;
+}
+
+namespace {
+
+struct RangeWork {
+    Plan p;
+    Grouping gr;
+    int64_t *cnt, *offs;   // per (pair, chunk) segment: hits, output offset (offs[segs] = total)
+    void* lims_tmp;
+};
+
+static int range_setup(ise_ctx* ctx, const float* q, int64_t nq, int d, const float* xs_sorted,
+                       const int64_t* ids_sorted, const int64_t* list_off, int64_t nlist, int64_t max_list_len,
+                       int nprobe, int metric, void* workspace, size_t workspace_bytes, RangeWork* rw) {
+    ISE_CHECK_ARG(plan_args_ok(nq, nprobe, nlist, max_list_len, 1));
+    ISE_CHECK_ARG(metric == ISE_METRIC_IP || metric == ISE_METRIC_L2);
+    ISE_CHECK_ARG(d > 0 && q && list_off && workspace);
+    ISE_CHECK_ARG(max_list_len == 0 || (xs_sorted && ids_sorted));
+    const size_t need = ise_ivfflat_range_workspace_bytes(ctx, nq, nprobe, nlist, max_list_len);
+    if (workspace_bytes < need) ISE_FAIL("workspace too small: need " + std::to_string(need));
+    rw->p = range_plan(ctx, nq, nprobe, nlist, max_list_len);
+    uint8_t* w = reinterpret_cast<uint8_t*>(workspace);
+    rw->gr = carve_grouping(w, rw->p);
+    rw->cnt = reinterpret_cast<int64_t*>(take(w, rw->p.seg));
+    rw->offs = reinterpret_cast<int64_t*>(take(w, rw->p.seg));
+    rw->lims_tmp = take(w, rw->p.lims_tmp);
+    return 0;
+}
+
+}  // namespace
+
+ISE_EXPORT int ise_ivfflat_range_count(ise_ctx* ctx, const float* q, int64_t nq, int d, const float* xs_sorted,
+                                       const int64_t* ids_sorted, const int64_t* list_off, int64_t nlist,
+                                       int64_t max_list_len, const int64_t* probes, int nprobe, int metric,
+                                       float radius, int64_t* lims, void* workspace, size_t workspace_bytes,
+                                       void* stream) {
+    ISE_CHECK_ARG(ctx != nullptr && nq >= 0 && lims != nullptr);
+    DeviceGuard guard(ctx->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (nq == 0) {
+        ISE_CUDA(cudaMemsetAsync(lims, 0, sizeof(int64_t), st));
+        return 0;
+    }
+    ISE_CHECK_ARG(probes != nullptr);
+    RangeWork rw;
+    int rc = range_setup(ctx, q, nq, d, xs_sorted, ids_sorted, list_off, nlist, max_list_len, nprobe, metric,
+                         workspace, workspace_bytes, &rw);
+    if (rc) return rc;
+    const Plan& p = rw.p;
+    // segments no item writes (probe -1, chunk slots a list does not use) count 0; cnt[segs] = 0 ends the scan
+    ISE_CUDA(cudaMemsetAsync(rw.cnt, 0, (size_t)(p.segs + 1) * sizeof(int64_t), st));
+    rc = group_pairs(ctx, p, rw.gr, probes, nq, nprobe, nlist, list_off, 0, nullptr, st);
+    if (rc) return rc;
+    const bool vec = vec_rows(q, xs_sorted, d);
+#define ISE_COUNT_ARGS q, d, vec, xs_sorted, list_off, nlist, rw.gr.pairs_sorted, rw.gr.qoff, rw.gr.item_off, nprobe, \
+                       p.S, radius, rw.gr.counter, rw.cnt
+    rc = metric == ISE_METRIC_L2 ? launch_persistent(ctx, st, ivfflat_range_count_kernel<true>, ISE_COUNT_ARGS)
+                                 : launch_persistent(ctx, st, ivfflat_range_count_kernel<false>, ISE_COUNT_ARGS);
+#undef ISE_COUNT_ARGS
+    if (rc) return rc;
+    rc = ise_range_lims(ctx, rw.cnt, p.segs, 0, rw.offs, rw.lims_tmp, p.lims_tmp, stream);
+    if (rc) return rc;
+    ivf_range_lims_kernel<<<(unsigned)ceil_div64(nq + 1, 256), 256, 0, st>>>(rw.offs, nq, p.g, lims);
+    ISE_LAUNCH_CHECK();
+    return 0;
+}
+
+ISE_EXPORT int ise_ivfflat_range_fill(ise_ctx* ctx, const float* q, int64_t nq, int d, const float* xs_sorted,
+                                      const int64_t* ids_sorted, const int64_t* list_off, int64_t nlist,
+                                      int64_t max_list_len, int nprobe, int metric, float radius, float* out_dis,
+                                      int64_t* out_ids, void* workspace, size_t workspace_bytes, void* stream) {
+    ISE_CHECK_ARG(ctx != nullptr && nq >= 0);
+    if (nq == 0) return 0;
+    ISE_CHECK_ARG(out_dis && out_ids);
+    DeviceGuard guard(ctx->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    RangeWork rw;
+    int rc = range_setup(ctx, q, nq, d, xs_sorted, ids_sorted, list_off, nlist, max_list_len, nprobe, metric,
+                         workspace, workspace_bytes, &rw);
+    if (rc) return rc;
+    ISE_CUDA(cudaMemsetAsync(rw.gr.counter, 0, sizeof(unsigned long long), st));
+    const bool vec = vec_rows(q, xs_sorted, d);
+#define ISE_FILL_ARGS q, d, vec, xs_sorted, ids_sorted, list_off, nlist, rw.gr.pairs_sorted, rw.gr.qoff, \
+                      rw.gr.item_off, nprobe, rw.p.S, radius, rw.gr.counter, rw.offs, out_dis, out_ids
+    rc = metric == ISE_METRIC_L2 ? launch_persistent(ctx, st, ivfflat_range_fill_kernel<true>, ISE_FILL_ARGS)
+                                 : launch_persistent(ctx, st, ivfflat_range_fill_kernel<false>, ISE_FILL_ARGS);
+#undef ISE_FILL_ARGS
+    return rc;
 }

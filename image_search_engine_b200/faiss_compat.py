@@ -414,7 +414,8 @@ class IndexIVFPQ:
 
 class IndexIVFFlat:
     """faiss.IndexIVFFlat (faiss/IndexIVFFlat.cpp, ~1.7.4): an inverted file whose lists hold the raw FP32 vectors, so
-    a search scans only the ``nprobe`` probed lists yet returns exact FP32 distances.
+    a search scans only the ``nprobe`` probed lists yet returns exact FP32 distances.  ``range_search`` filters the
+    same lists by a radius (``ise_ivfflat_range_count`` / ``_fill``) and returns its results in Faiss's probe order.
 
     Training is the level-1 clustering of ``IndexIVFPQ`` (niter 10, seed 1234, spherical for inner product); vectors
     go to their quantizer top-1 list; a search probes ``min(nprobe, nlist)`` lists through the quantizer and scans
@@ -545,6 +546,30 @@ class IndexIVFFlat:
         if was_cuda:
             return D, I
         return D.cpu().numpy(), I.cpu().numpy()
+
+    def range_search(self, x, radius: float):
+        """IndexIVF::range_search: probe min(nprobe, nlist) lists as ``search`` does and return every vector of them
+        whose exact FP32 score (IVFFlatScanner's direct formulas) beats ``radius``: IP dis > radius, L2 squared
+        distance < radius, both strict, radius cast to float32.  Returns (lims [nq + 1], D, I); the results of query i
+        are D[lims[i]:lims[i+1]] / I[...] in Faiss's scan order: by probe rank (nearest list first), then by position
+        in the list (ids ascend inside a list).  This differs from IndexFlat.range_search, whose results come in
+        ascending id.  NumPy input gives NumPy output (lims uint64); CUDA tensors give CUDA tensors (lims int64).  An
+        untrained or empty index returns no results."""
+        q, was_cuda = _to_device(x)
+        if q.shape[1] != self.d:
+            raise AssertionError(f"range_search: expected (n, {self.d}) array")
+        q = q.to(torch.float32).contiguous()
+        nq = q.shape[0]
+        if nq and self._ntotal and self.is_trained:
+            xs, ids, off = self._lists()
+            _, probes = self.quantizer._search_device(q, min(self.nprobe, self.nlist), need_distances=False)
+            lims, D, I = ops.ivfflat_range_search(q, xs, ids, off, int(self._sizes.max()), probes, self.metric_type,
+                                                  radius)
+        else:
+            lims, D, I = ops._range_empty(nq, q.device)
+        if was_cuda:
+            return lims, D, I
+        return lims.cpu().numpy().astype(np.uint64), D.cpu().numpy(), I.cpu().numpy()
 
     def reset(self) -> None:
         with self._lock:

@@ -856,6 +856,50 @@ def ivfflat_search(q: torch.Tensor, xs: torch.Tensor, ids: torch.Tensor, list_of
     return val, idx
 
 
+def ivfflat_range_workspace_bytes(nq: int, nprobe: int, nlist: int, max_list_len: int) -> int:
+    """Device scratch of one ivfflat_range_search call (the formula is in include/ise.h)."""
+    return int(_lib.load().ise_ivfflat_range_workspace_bytes(_lib.ctx(torch.cuda.current_device()), int(nq),
+                                                               int(nprobe), int(nlist), int(max_list_len)))
+
+
+def ivfflat_range_search(q: torch.Tensor, xs: torch.Tensor, ids: torch.Tensor, list_off: torch.Tensor,
+                         max_list_len: int, probes: torch.Tensor, metric: int, radius: float):
+    """Every vector of a query's probed lists whose exact FP32 score beats ``radius`` (IndexIVFFlat.range_search; IP:
+    > radius, L2: squared distance < radius, strict, radius cast to float32).  Inputs as ivfflat_search.  Returns
+    (lims int64 [nq + 1], D float32, I int64) on the device; the results of query i are D / I[lims[i]:lims[i+1]] in
+    probe rank order, then list order (Faiss's order, not ascending id).  One readback: the total, lims[nq]."""
+    if q.dtype != torch.float32 or xs.dtype != torch.float32 or not q.is_contiguous() or not xs.is_contiguous():
+        raise IseError("ivfflat_range_search needs contiguous float32 queries and vectors")
+    if ids.dtype != torch.int64 or list_off.dtype != torch.int64 or probes.dtype != torch.int64:
+        raise IseError("ivfflat_range_search: ids, list offsets and probes are int64")
+    nq, d = q.shape
+    if xs.shape[1] != d or probes.shape[0] != nq:
+        raise IseError("ivfflat_range_search: inconsistent shapes")
+    nprobe, nlist = probes.shape[1], list_off.shape[0] - 1
+    radius = float(np.float32(radius))
+    if nq == 0:
+        last_search_stats.update(mode="ivf-range", rows=0, pairs=0, results=0, fallback_rows=0)
+        return _range_empty(0, q.device)
+    lib, ctx = _lib.load(), _lib.ctx(_dev(q))
+    ws_bytes = lib.ise_ivfflat_range_workspace_bytes(ctx, nq, nprobe, nlist, int(max_list_len))
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=q.device)
+    probes, list_off, ids = probes.contiguous(), list_off.contiguous(), ids.contiguous()
+    lims = torch.empty((nq + 1,), dtype=torch.int64, device=q.device)
+    _lib.check(lib.ise_ivfflat_range_count(ctx, _ptr(q), nq, d, _ptr(xs), _ptr(ids), _ptr(list_off), nlist,
+                                           int(max_list_len), _ptr(probes), nprobe, int(metric), radius, _ptr(lims),
+                                           _ptr(ws), ws_bytes, _stream()))
+    total = int(lims[nq].item())                          # the one readback: sizes D / I
+    D = torch.empty((total,), dtype=torch.float32, device=q.device)
+    I = torch.empty((total,), dtype=torch.int64, device=q.device)
+    if total:
+        _lib.check(lib.ise_ivfflat_range_fill(ctx, _ptr(q), nq, d, _ptr(xs), _ptr(ids), _ptr(list_off), nlist,
+                                              int(max_list_len), nprobe, int(metric), radius, _ptr(D), _ptr(I),
+                                              _ptr(ws), ws_bytes, _stream()))
+    _count(9 if total else 8)
+    last_search_stats.update(mode="ivf-range", rows=nq, pairs=nq * nprobe, results=total, fallback_rows=0)
+    return lims, D, I
+
+
 # ------------------------------------------------------------------------------------------
 # k-means update
 # ------------------------------------------------------------------------------------------

@@ -405,6 +405,30 @@ int ise_ivfflat_search(ise_ctx* ctx, const float* q, int64_t nq, int d, const fl
                        const int64_t* ids_sorted, const int64_t* list_off, int64_t nlist, int64_t max_list_len,
                        const int64_t* probes, int nprobe, int metric, int topk, float* out_val, int64_t* out_idx,
                        void* workspace, size_t workspace_bytes, void* stream);
+/* Range search over the probed lists (faiss/IndexIVF.cpp range_search_preassigned, IVFFlatScanner::scan_codes_range):
+ * every vector of a probed list whose direct-formula FP32 score beats the radius, IP: dis > radius, L2: dis < radius
+ * (both strict; the scores are bit-identical to ise_ivfflat_search's).  Same inputs as ise_ivfflat_search.
+ * Results of query i are out[lims[i] .. lims[i + 1]) in Faiss's order: probe rank (probes[i, 0] first; -1 skipped),
+ * then position inside the list (= ascending id) -- not the ascending-id order of the flat range search.
+ * Two calls on the same stream with the same arguments and the same workspace, untouched in between:
+ *   ise_ivfflat_range_count  groups the pairs, counts the hits of every (pair, chunk) segment, scans them into int64
+ *                            offsets (totals above 2^31 are fine) and writes lims[nq + 1] (lims[nq] = total; lims[0] =
+ *                            0 for nq == 0).  The workspace then carries the grouping and the segment offsets;
+ *   ise_ivfflat_range_fill   re-scores the work items that have hits and writes out_dis / out_ids[lims[nq]].
+ * No host synchronisation inside; the caller reads lims[nq] to size the outputs.  Workspace
+ * (ise_ivfflat_range_workspace_bytes) is O(nq * nprobe * S + nlist): 16 bytes per segment (count, offset) for the
+ * nq * nprobe * S segments, with S = min(ceil(max_list_len / 64), max(1, 256 / nprobe),
+ * max(1, 2^22 / (nq * nprobe))) chunks per list, so at most max(2^22, nq * nprobe) segments; 16 bytes per
+ * (query, probe) pair and 24 per list for the grouping; CUB's sort / scan scratch.  nq * nprobe < 2^31. */
+size_t ise_ivfflat_range_workspace_bytes(ise_ctx* ctx, int64_t nq, int nprobe, int64_t nlist, int64_t max_list_len);
+int ise_ivfflat_range_count(ise_ctx* ctx, const float* q, int64_t nq, int d, const float* xs_sorted,
+                            const int64_t* ids_sorted, const int64_t* list_off, int64_t nlist, int64_t max_list_len,
+                            const int64_t* probes, int nprobe, int metric, float radius, int64_t* lims,
+                            void* workspace, size_t workspace_bytes, void* stream);
+int ise_ivfflat_range_fill(ise_ctx* ctx, const float* q, int64_t nq, int d, const float* xs_sorted,
+                           const int64_t* ids_sorted, const int64_t* list_off, int64_t nlist, int64_t max_list_len,
+                           int nprobe, int metric, float radius, float* out_dis, int64_t* out_ids, void* workspace,
+                           size_t workspace_bytes, void* stream);
 
 /* ---- collectives for a single-process multi-GPU host (NCCL over NVLink, resolved with dlopen at run time) ----------
  * The two exchange steps of the sharded path (SURVEY section 8e): the per-iteration all-reduce of the k-means
