@@ -88,6 +88,34 @@ __device__ __forceinline__ float warp_max(float v) {
     return v;
 }
 
+// The exact FP32 score of one candidate row `brow` (global memory) against the row `s_a` staged as float32 in shared
+// memory, for the warp calling it: per-lane sequential FMAs over dimensions lane, lane + 32, ... (float4 steps when
+// d and ldb allow), then the warp tree.  IP returns <a,b>; L2 returns Faiss's IndexFlat expansion
+// an + *bn - 2<a,b> clamped at 0 (an, *bn: the squared norms; bn is read only for L2).  Every lane returns the same
+// value.  The re-score of search results and the radius test of range search both score through it, so their
+// distances agree bit for bit.
+template <bool L2>
+__device__ __forceinline__ float exact_score(const float* s_a, const float* __restrict__ brow, int d, int64_t ldb,
+                                             float an, const float* __restrict__ bn, int lane) {
+    float acc = 0.f;
+    if ((d & 3) == 0 && (ldb & 3) == 0) {
+        const float4* b4 = reinterpret_cast<const float4*>(brow);
+        const float4* a4 = reinterpret_cast<const float4*>(s_a);
+        for (int c = lane; c < d / 4; c += 32) {
+            const float4 y = __ldg(b4 + c);
+            const float4 x = a4[c];
+            acc = fmaf(x.x, y.x, acc); acc = fmaf(x.y, y.y, acc);
+            acc = fmaf(x.z, y.z, acc); acc = fmaf(x.w, y.w, acc);
+        }
+    } else {
+        for (int c = lane; c < d; c += 32) acc = fmaf(s_a[c], __ldg(brow + c), acc);
+    }
+    acc = warp_sum(acc);
+    if (!L2) return acc;
+    const float dis = an + *bn - 2.f * acc;
+    return dis < 0.f ? 0.f : dis;
+}
+
 // Canonical ordering shared by every selection kernel: `better(a, b)` is true when candidate a
 // must precede b.  LARGEST: bigger score first; ties by smaller id; id < 0 (padding) loses ties.
 template <bool LARGEST>

@@ -19,7 +19,8 @@
 // Range search (faiss/IndexIVF.cpp range_search_preassigned, IVFFlatScanner::scan_codes_range) reuses the grouping and
 // the work items, and replaces the top-k with two passes over the same score tiles:
 //   ivfflat_range_count_kernel   hits of every (pair, chunk) segment, cnt[(q * nprobe + slot) * S + c] (query-major,
-//                                so one exclusive scan (ise_range_lims) gives every segment its output offset in
+//                                so the flat range search's offsets scan, ise_internal_range_offsets in range.cu,
+//                                gives every segment its output offset in
 //                                Faiss's order: probe rank, then list position); lims[q] = offset of segment (q, 0, 0);
 //   ivfflat_range_fill_kernel    re-runs the items with hits and writes each segment's hits in list order.
 // Every kernel scores through score_tile, so search and range search return bit-identical distances.  S is capped at
@@ -387,13 +388,6 @@ __global__ void __launch_bounds__(kThreads) ivfflat_range_fill_kernel(
     }
 }
 
-// lims[r] = offs[r * per_query], r = 0 .. nq (the first segment of query r; lims[nq] = the total)
-__global__ void ivf_range_lims_kernel(const int64_t* __restrict__ offs, int64_t nq, int64_t per_query,
-                                      int64_t* __restrict__ lims) {
-    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (r <= nq) lims[r] = offs[r * per_query];
-}
-
 struct Plan {
     int S;                 // chunks per list (partial-list / segment slots per probe)
     int64_t npairs, g;     // nq * nprobe; slots per query = nprobe * S
@@ -592,6 +586,9 @@ ISE_EXPORT size_t ise_ivfflat_range_workspace_bytes(ise_ctx* ctx, int64_t nq, in
     return p.grouping + 2 * p.seg + p.lims_tmp;
 }
 
+int ise_internal_range_offsets(const int64_t* cnt, int64_t rows, int64_t per_row, int64_t base,
+                               int64_t* offs, int64_t* lims, void* tmp, size_t tmp_bytes, void* stream);   // range.cu
+
 namespace {
 
 struct RangeWork {
@@ -650,11 +647,7 @@ ISE_EXPORT int ise_ivfflat_range_count(ise_ctx* ctx, const float* q, int64_t nq,
                                  : launch_persistent(ctx, st, ivfflat_range_count_kernel<false>, ISE_COUNT_ARGS);
 #undef ISE_COUNT_ARGS
     if (rc) return rc;
-    rc = ise_range_lims(ctx, rw.cnt, p.segs, 0, rw.offs, rw.lims_tmp, p.lims_tmp, stream);
-    if (rc) return rc;
-    ivf_range_lims_kernel<<<(unsigned)ceil_div64(nq + 1, 256), 256, 0, st>>>(rw.offs, nq, p.g, lims);
-    ISE_LAUNCH_CHECK();
-    return 0;
+    return ise_internal_range_offsets(rw.cnt, nq, p.g, 0, rw.offs, lims, rw.lims_tmp, p.lims_tmp, stream);
 }
 
 ISE_EXPORT int ise_ivfflat_range_fill(ise_ctx* ctx, const float* q, int64_t nq, int d, const float* xs_sorted,

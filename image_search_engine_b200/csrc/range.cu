@@ -5,7 +5,7 @@
 // Tensor-core path (nq >= 20, Faiss's BLAS regime):
 //   ise_range_seed   per-row coarse threshold = radius loosened by the rigorous coarse bound (CoarseBound), so that
 //                    ise_gemm_collect over the hi planes appends EVERY column whose exact score can qualify;
-//   ise_range_count  exact FP32 re-score of the appended candidates (rescore.cu's formulas), strict radius test,
+//   ise_range_count  exact FP32 re-score of the appended candidates (exact_score, as rescore.cu), strict radius test,
 //                    per-row kept counts; rows whose collect buffer overflowed are left to the caller;
 //   ise_range_lims   exclusive scan of the kept counts -> lims (int64: totals can exceed 2^31);
 //   ise_range_fill   compaction of the kept (dis, id) pairs into the result arrays (unordered within a row);
@@ -29,8 +29,8 @@ static inline size_t align256(size_t b) { return (b + 255) & ~size_t(255); }
 
 // IP:  seed = radius - slack,  L2: seed = radius + 2 slack  (collect keeps coarse score > / < seed).
 // slack = CoarseBound eps (coarse hi-plane product vs the real inner product)
-//       + the rounding of the FP32 re-score (per-lane sequential FMAs over <= d/32 + 4 terms, a 5-level warp tree:
-//         <= (d/32 + 9) 2^-24 |a||b|, taken with a 2x margin)
+//       + the rounding of the FP32 re-score, exact_score in common.cuh (per-lane sequential FMAs over <= d/32 + 4
+//         terms, a 5-level warp tree: <= (d/32 + 9) 2^-24 |a||b|, taken with a 2x margin)
 //       + a few ulps of every magnitude the two comparisons round at (the collect epilogue's fma and threshold, the
 //         re-score's norm expansion), so that the strict test of the collect can never drop a column whose exact
 //         FP32 score qualifies.
@@ -83,26 +83,8 @@ __global__ void range_count_kernel(const TA* __restrict__ a, int64_t lda, const 
             const int64_t slot = row * (int64_t)cap + j;
             const long long id = cand_idx[slot];
             if (id < 0) continue;                                   // warp-uniform
-            const float* brow = b + (id - id_base) * ldb;
-            float acc = 0.f;
-            if ((d & 3) == 0 && (ldb & 3) == 0) {
-                const float4* b4 = reinterpret_cast<const float4*>(brow);
-                const float4* a4 = reinterpret_cast<const float4*>(s_a);
-                for (int c = lane; c < d / 4; c += 32) {
-                    const float4 y = __ldg(b4 + c);
-                    const float4 x = a4[c];
-                    acc = fmaf(x.x, y.x, acc); acc = fmaf(x.y, y.y, acc);
-                    acc = fmaf(x.z, y.z, acc); acc = fmaf(x.w, y.w, acc);
-                }
-            } else {
-                for (int c = lane; c < d; c += 32) acc = fmaf(s_a[c], __ldg(brow + c), acc);
-            }
-            acc = warp_sum(acc);
-            float s = acc;
-            if (L2) {
-                const float dis = an + b_norms[id - id_base] - 2.f * acc;   // x_norms[i] + y_norms[j] - 2 * ip
-                s = dis < 0.f ? 0.f : dis;
-            }
+            const int64_t col = id - id_base;
+            const float s = exact_score<L2>(s_a, b + col * ldb, d, ldb, an, b_norms + col, lane);
             const bool keep = L2 ? (s < radius) : (s > radius);
             if (lane == 0) {
                 if (keep) {
@@ -174,11 +156,11 @@ __global__ void scores_range_count_kernel(const float* __restrict__ scores, int6
     }
 }
 
-// lims[r] = offs[r * ntiles] (offs = base + exclusive scan of the tile counts), r = 0 .. nq
-__global__ void scores_range_lims_kernel(const int64_t* __restrict__ offs, int64_t nq, int64_t ntiles,
-                                         int64_t* __restrict__ lims) {
+// lims[r] = offs[r * per_row], r = 0 .. rows (the first segment of row r; lims[rows] = the total)
+__global__ void range_lims_kernel(const int64_t* __restrict__ offs, int64_t rows, int64_t per_row,
+                                  int64_t* __restrict__ lims) {
     const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (r <= nq) lims[r] = offs[r * ntiles];
+    if (r <= rows) lims[r] = offs[r * per_row];
 }
 
 template <bool L2>
@@ -230,6 +212,21 @@ static size_t sort_temp_bytes(int64_t m, int64_t total) {
 }
 
 }  // namespace
+
+// Output offsets of a range search, shared with ise_ivfflat_range_count (ivfflat.cu): offs = base + exclusive scan of
+// the rows * per_row + 1 segment counts in cnt (the last count is 0, so offs[rows * per_row] is base + the total), then
+// lims[r] = offs[r * per_row], r = 0 .. rows, unless lims is null (per_row == 1 and offs are the lims).  tmp holds the
+// scan's scratch (scan_temp_bytes(rows * per_row + 1)).
+int ise_internal_range_offsets(const int64_t* cnt, int64_t rows, int64_t per_row, int64_t base,
+                               int64_t* offs, int64_t* lims, void* tmp, size_t tmp_bytes, void* stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    ISE_CUDA(cub::DeviceScan::ExclusiveScan(tmp, tmp_bytes, cnt, offs, cub::Sum(), base, rows * per_row + 1, st));
+    if (lims) {
+        range_lims_kernel<<<(unsigned)ceil_div64(rows + 1, kThreads), kThreads, 0, st>>>(offs, rows, per_row, lims);
+        ISE_LAUNCH_CHECK();
+    }
+    return 0;
+}
 
 ISE_EXPORT int ise_range_seed(ise_ctx* ctx, const float* a_meta, const float* a_norms, const float* a_row_inv,
                               const float* b_meta, int64_t m, int d, int metric, float radius, float* row_seed,
@@ -295,10 +292,7 @@ ISE_EXPORT int ise_range_lims(ise_ctx* ctx, const int64_t* kept, int64_t m, int6
     ISE_CHECK_ARG(ctx != nullptr && m >= 0 && kept && lims && workspace);
     if (workspace_bytes < ise_range_lims_workspace_bytes(ctx, m)) ISE_FAIL("workspace too small");
     DeviceGuard guard(ctx->device);
-    size_t bytes = workspace_bytes;
-    ISE_CUDA(cub::DeviceScan::ExclusiveScan(workspace, bytes, kept, lims, cub::Sum(), base, m + 1,
-                                            (cudaStream_t)stream));
-    return 0;
+    return ise_internal_range_offsets(kept, m, 1, base, lims, nullptr, workspace, workspace_bytes, stream);
 }
 
 ISE_EXPORT int ise_range_fill(ise_ctx* ctx, int64_t m, int cap, const int32_t* row_count, const float* cand_val,
@@ -368,15 +362,13 @@ ISE_EXPORT int ise_scores_range(ise_ctx* ctx, const float* scores, int64_t nq, i
     int64_t* cnt = reinterpret_cast<int64_t*>(w);
     int64_t* offs = reinterpret_cast<int64_t*>(w + align256((size_t)items * sizeof(int64_t)));
     void* tmp = w + 2 * align256((size_t)items * sizeof(int64_t));
-    size_t tmp_bytes = scan_temp_bytes(items);
     const dim3 grid((unsigned)std::min<int64_t>(ntiles, (int64_t)ctx->sm_count * 8), (unsigned)nq);
     const bool l2 = metric == ISE_METRIC_L2;
     if (l2) scores_range_count_kernel<true><<<grid, kThreads, 0, st>>>(scores, nq, nb, ntiles, radius, cnt);
     else scores_range_count_kernel<false><<<grid, kThreads, 0, st>>>(scores, nq, nb, ntiles, radius, cnt);
     ISE_LAUNCH_CHECK();
-    ISE_CUDA(cub::DeviceScan::ExclusiveScan(tmp, tmp_bytes, cnt, offs, cub::Sum(), base, items, st));
-    scores_range_lims_kernel<<<(unsigned)ceil_div64(nq + 1, kThreads), kThreads, 0, st>>>(offs, nq, ntiles, lims);
-    ISE_LAUNCH_CHECK();
+    int rc = ise_internal_range_offsets(cnt, nq, ntiles, base, offs, lims, tmp, scan_temp_bytes(items), stream);
+    if (rc) return rc;
     if (out_dis) {
         if (l2) scores_range_fill_kernel<true><<<grid, kThreads, 0, st>>>(scores, nq, nb, ntiles, radius, id_base, offs, base, out_dis, out_ids);
         else scores_range_fill_kernel<false><<<grid, kThreads, 0, st>>>(scores, nq, nb, ntiles, radius, id_base, offs, base, out_dis, out_ids);

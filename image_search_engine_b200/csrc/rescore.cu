@@ -54,27 +54,7 @@ __global__ void rescore_kernel(const TA* __restrict__ a, int64_t lda, const floa
             float out = worst;
             if (id >= 0) {
                 const int64_t col = id - id_base;
-                const float* brow = b + col * ldb;
-                float acc = 0.f;
-                if ((d & 3) == 0 && (ldb & 3) == 0) {
-                    const float4* b4 = reinterpret_cast<const float4*>(brow);
-                    const float4* a4 = reinterpret_cast<const float4*>(s_a);
-                    for (int c = lane; c < d / 4; c += 32) {
-                        const float4 y = __ldg(b4 + c);
-                        const float4 x = a4[c];
-                        acc = fmaf(x.x, y.x, acc); acc = fmaf(x.y, y.y, acc);
-                        acc = fmaf(x.z, y.z, acc); acc = fmaf(x.w, y.w, acc);
-                    }
-                } else {
-                    for (int c = lane; c < d; c += 32) acc = fmaf(s_a[c], __ldg(brow + c), acc);
-                }
-                acc = warp_sum(acc);
-                if (L2) {
-                    float dis = an + b_norms[col] - 2.f * acc;   // x_norms[i] + y_norms[j] - 2 * ip
-                    out = dis < 0.f ? 0.f : dis;
-                } else {
-                    out = acc;
-                }
+                out = exact_score<L2>(s_a, b + col * ldb, d, ldb, an, b_norms + col, lane);
             }
             if (lane == 0) { s_v[j] = out; s_i[j] = id; }
         }
@@ -128,6 +108,8 @@ __global__ void rescore_kernel(const TA* __restrict__ a, int64_t lda, const floa
 
 // topk == 1 fast path (k-means assign / quantisation distances): one warp per row, no sorting; ROWS rows (and their
 // gathered winners) in flight per warp so the loads cover HBM latency
+// It reads A from global memory but does exact_score's arithmetic (common.cuh) whenever both step by the same width:
+// float4 steps here also need float32 A rows with lda % 4 == 0 and 16-byte alignment (uint8 rows step by one).
 template <typename TA, bool L2, int ROWS>
 __global__ void rescore_top1_kernel(const TA* __restrict__ a, int64_t lda, const float* __restrict__ b, int64_t ldb,
                                     int64_t m, int d, int64_t id_base, const float* __restrict__ a_norms,

@@ -28,10 +28,9 @@ from ._lib import METRIC_IP, METRIC_L2, IseError
 METRIC_INNER_PRODUCT = METRIC_IP
 # METRIC_L2 imported above keeps faiss's value (1)
 
-# faiss/utils/distances.cpp: below this many queries Faiss skips the BLAS expansion
-distance_compute_blas_threshold = 20
-
-_FLT_MAX = float(np.finfo(np.float32).max)
+# faiss/utils/distances.cpp: below this many queries Faiss skips the BLAS expansion (the flat searches decide on
+# ops.BLAS_THRESHOLD; this is faiss's name for the same value, read by engine.py)
+distance_compute_blas_threshold = ops.BLAS_THRESHOLD
 
 
 def _as_host_f32(x) -> np.ndarray:
@@ -155,40 +154,8 @@ class IndexFlat:
     def _search_device(self, q: torch.Tensor, k: int, need_distances: bool = True):
         """need_distances=False skips the exact FP32 re-score (callers that only use the ids, e.g.
         quantisation); the returned scores are then the tensor-core accumulator values."""
-        nq = q.shape[0]
-        largest = self.metric_type == METRIC_INNER_PRODUCT
-        pad = -_FLT_MAX if largest else _FLT_MAX
-        if self._ntotal == 0 or nq == 0:
-            D = torch.full((nq, k), pad, dtype=torch.float32, device=q.device)
-            I = torch.full((nq, k), -1, dtype=torch.int64, device=q.device)
-            return D, I
-        kk = min(k, ops.MAX_TOPK)
-        if k > ops.MAX_TOPK and self._ntotal > ops.MAX_TOPK:
-            # beyond the fused-selection limit: exact pair scores + repeated masked selection passes (any k, like Faiss)
-            qf = q if q.dtype == torch.float32 else q.to(torch.float32)
-            return ops.search_exact_any_k(qf.contiguous(), self._database(), self.metric_type, k)
-        if nq < distance_compute_blas_threshold:
-            qf = q if q.dtype == torch.float32 else q.to(torch.float32)
-            D, I = ops.flat_search_exact(qf.contiguous(), self._database(), self.metric_type, kk)
-        else:
-            b = self._operand()
-            # nearest-column queries over raw float32 descriptors (quantisation: FaissKMeans.transform): the row
-            # preparation runs inside the contraction kernel
-            fused = ops.assign_fused(q, b, self.metric_type) if (kk == 1 and q.dtype == torch.float32) else None
-            if fused is not None:
-                D, I, a = fused
-                if need_distances:
-                    ops.rescore_topk_(q, self._database(), a, b, self.metric_type, D, I)
-            else:
-                a = ops.prepare_operand(q, rows=True)
-                D, I = ops.search_topk(q, a, self._database(), b, self.metric_type, kk, precision=self.precision,
-                                       need_distances=need_distances)
-        if kk < k:
-            Dp = torch.full((nq, k), pad, dtype=torch.float32, device=q.device)
-            Ip = torch.full((nq, k), -1, dtype=torch.int64, device=q.device)
-            Dp[:, :kk], Ip[:, :kk] = D, I
-            D, I = Dp, Ip
-        return D, I
+        return ops.flat_search(q, self._database(), self.metric_type, k, operand=self._operand, precision=self.precision,
+                               need_distances=need_distances)
 
     def range_search(self, x, radius: float):
         """faiss IndexFlat::range_search: every stored vector scoring better than ``radius`` (IP: > radius, L2: squared
@@ -204,15 +171,7 @@ class IndexFlat:
         return lims.cpu().numpy().astype(np.uint64), D.cpu().numpy(), I.cpu().numpy()
 
     def _range_search_device(self, q: torch.Tensor, radius: float):
-        nq = q.shape[0]
-        if self._ntotal == 0 or nq == 0:
-            return ops._range_empty(nq, q.device)
-        if nq < distance_compute_blas_threshold:
-            qf = q if q.dtype == torch.float32 else q.to(torch.float32)
-            return ops.range_search_exact(qf.contiguous(), self._database(), self.metric_type, radius)
-        b = self._operand()
-        a = ops.prepare_operand(q, rows=True)
-        return ops.range_search(q, a, self._database(), b, self.metric_type, radius)
+        return ops.flat_range_search(q, self._database(), self.metric_type, radius, operand=self._operand)
 
     def assign(self, x, k: int = 1):
         return self.search(x, k)[1]
@@ -370,8 +329,7 @@ class IndexIVFPQ:
         if q.shape[1] != self.d:
             raise AssertionError(f"search: expected (n, {self.d}) array")
         nq = q.shape[0]
-        D = torch.full((nq, k), _FLT_MAX, dtype=torch.float32, device=q.device)
-        I = torch.full((nq, k), -1, dtype=torch.int64, device=q.device)
+        D, I = ops.topk_padding(nq, k, METRIC_L2, q.device)
         if nq and self.ntotal:
             codes, ids, off = self._lists()
             _, probes = self.quantizer._search_device(q, min(self.nprobe, self.nlist), need_distances=False)
@@ -540,9 +498,7 @@ class IndexIVFFlat:
             _, probes = self.quantizer._search_device(q, min(self.nprobe, self.nlist), need_distances=False)
             D, I = ops.ivfflat_search(q, xs, ids, off, int(self._sizes.max()), probes, self.metric_type, k)
         else:
-            pad = -_FLT_MAX if self.metric_type == METRIC_INNER_PRODUCT else _FLT_MAX
-            D = torch.full((nq, k), pad, dtype=torch.float32, device=q.device)
-            I = torch.full((nq, k), -1, dtype=torch.int64, device=q.device)
+            D, I = ops.topk_padding(nq, k, self.metric_type, q.device)
         if was_cuda:
             return D, I
         return D.cpu().numpy(), I.cpu().numpy()
@@ -566,7 +522,7 @@ class IndexIVFFlat:
             lims, D, I = ops.ivfflat_range_search(q, xs, ids, off, int(self._sizes.max()), probes, self.metric_type,
                                                   radius)
         else:
-            lims, D, I = ops._range_empty(nq, q.device)
+            lims, D, I = ops.range_empty(nq, q.device)
         if was_cuda:
             return lims, D, I
         return lims.cpu().numpy().astype(np.uint64), D.cpu().numpy(), I.cpu().numpy()

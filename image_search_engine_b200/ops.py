@@ -18,6 +18,9 @@ from ._lib import (DTYPE_F32, DTYPE_U8, HIST_BINCOUNT, HIST_NUMPY_COMPAT, METRIC
                    OUT_F64, IseError)
 
 MAX_TOPK = 128
+# faiss/utils/distances.cpp distance_compute_blas_threshold: below this many queries Faiss skips the BLAS expansion, and
+# the flat searches take the direct-formula kernels (flat_search_exact, range_search_exact)
+BLAS_THRESHOLD = 20
 CSR_MAX_BINS = 12 * 1024     # ise_bovw_histogram_csr keeps one int32 counter per bin in shared memory
 
 # kernel-launch counter (bench.py reports it as gpu_launches)
@@ -553,7 +556,8 @@ def _range_concat(parts, nq: int, device):
     return _range_lims(kept, nq), torch.cat([p[2] for p in parts]), torch.cat([p[3] for p in parts])
 
 
-def _range_empty(nq: int, device):
+def range_empty(nq: int, device):
+    """The range-search result of nq queries that found nothing: (lims zeros [nq + 1], D [0], I [0])."""
     return (torch.zeros((nq + 1,), dtype=torch.int64, device=device), torch.empty((0,), dtype=torch.float32, device=device),
             torch.empty((0,), dtype=torch.int64, device=device))
 
@@ -579,7 +583,7 @@ def range_search(q_raw: torch.Tensor, a_op: Operand, db_raw: torch.Tensor, b_op:
         raise IseError(f"dimension mismatch {a_op.d} vs {b_op.d}")
     if nq == 0 or b_op.n == 0:
         last_search_stats.update(mode="range", rows=nq, candidates=0, overflow_rows=0, results=0, fallback_rows=0)
-        return _range_empty(nq, dev)
+        return range_empty(nq, dev)
     lib, ctx = _lib.load(), _lib.ctx(_dev(q_raw))
     seed = torch.empty((nq,), dtype=torch.float32, device=dev)
     _lib.check(lib.ise_range_seed(ctx, _ptr(a_op.meta), _ptr(a_op.norms), _ptr(a_op.row_inv), _ptr(b_op.meta), nq,
@@ -646,7 +650,7 @@ def range_search_exact(q: torch.Tensor, db: torch.Tensor, metric: int, radius: f
     radius = float(np.float32(radius))
     if nq == 0 or nb == 0:
         last_search_stats.update(mode="range-exact", rows=nq, results=0, fallback_rows=0)
-        return _range_empty(nq, q.device)
+        return range_empty(nq, q.device)
     lib, ctx = _lib.load(), _lib.ctx(_dev(q))
     chunk = int(max(1, min(nq, 65535, max_score_bytes // (4 * nb))))
     parts, base = [], 0
@@ -709,12 +713,10 @@ def search_exact_any_k(q: torch.Tensor, db: torch.Tensor, metric: int, k: int, i
     lib, ctx = _lib.load(), _lib.ctx(dev)
     nq, d = q.shape
     nb = db.shape[0]
-    k_eff = min(int(k), nb)
-    pad = -3.4028234663852886e38 if metric == METRIC_IP else 3.4028234663852886e38
-    val = torch.full((nq, k), pad, dtype=torch.float32, device=q.device)
-    idx = torch.full((nq, k), -1, dtype=torch.int64, device=q.device)
     if nq == 0 or nb == 0:
-        return val, idx
+        return topk_padding(nq, k, metric, q.device)
+    val = torch.empty((nq, k), dtype=torch.float32, device=q.device)
+    idx = torch.empty((nq, k), dtype=torch.int64, device=q.device)
     chunk = int(max(1, min(nq, 65535, max_score_bytes // (4 * nb))))
     for q0 in range(0, nq, chunk):
         qs = q[q0:q0 + chunk]
@@ -730,11 +732,9 @@ def scores_topk_any_k_(scores: torch.Tensor, metric: int, k: int, id_base: int =
     """Per-row top-k of a score matrix for any k: ceil(k / 128) selection passes, masking what a pass returned
     (``scores`` is consumed).  Rows shorter than k are padded with id -1 / -+FLT_MAX like Faiss."""
     nq, nb = scores.shape
-    pad = -3.4028234663852886e38 if metric == METRIC_IP else 3.4028234663852886e38
     if k <= MAX_TOPK:
         return scores_topk(scores, metric, k, id_base)
-    val = torch.full((nq, k), pad, dtype=torch.float32, device=scores.device)
-    idx = torch.full((nq, k), -1, dtype=torch.int64, device=scores.device)
+    val, idx = topk_padding(nq, k, metric, scores.device)
     k_eff = min(int(k), nb)
     lib, ctx = _lib.load(), _lib.ctx(_dev(scores))
     for k0 in range(0, k_eff, MAX_TOPK):
@@ -746,6 +746,60 @@ def scores_topk_any_k_(scores: torch.Tensor, metric: int, k: int, id_base: int =
             _lib.check(lib.ise_scores_mask(ctx, _ptr(scores), nq, nb, _ptr(i), kk, int(id_base), int(metric), _stream()))
             _count()
     return val, idx
+
+
+def topk_padding(nq: int, k: int, metric: int, device):
+    """(D [nq, k], I [nq, k]) of empty top-k lists, padded like Faiss: id -1, score -FLT_MAX (IP) / +FLT_MAX (L2)."""
+    pad = -3.4028234663852886e38 if metric == METRIC_IP else 3.4028234663852886e38
+    return (torch.full((nq, k), pad, dtype=torch.float32, device=device),
+            torch.full((nq, k), -1, dtype=torch.int64, device=device))
+
+
+def flat_search(q: torch.Tensor, db: torch.Tensor, metric: int, k: int, *, operand, id_base: int = 0,
+                precision: str = "verified", need_distances: bool = True):
+    """Faiss's IndexFlat.search of float32 or uint8 queries over the float32 rows ``db`` (ids id_base + row), any k >= 1:
+    the one dispatch of IndexFlat and of every ShardedIndexFlat shard, so both return the same results.  ``operand()``
+    returns db's prepared operand and is called only on the tensor-core paths (nq >= BLAS_THRESHOLD): an index that only
+    sees small batches never prepares planes.  need_distances=False skips the exact FP32 re-score (callers that only use
+    the ids, e.g. quantisation); the returned scores are then the tensor-core accumulator values."""
+    nq, nb = q.shape[0], db.shape[0]
+    if nb == 0 or nq == 0:
+        return topk_padding(nq, k, metric, q.device)
+    if k > MAX_TOPK and nb > MAX_TOPK:
+        # beyond the fused-selection limit: exact pair scores + repeated masked selection passes (any k, like Faiss)
+        return search_exact_any_k(q.to(torch.float32).contiguous(), db, metric, k, id_base)
+    kk = min(k, MAX_TOPK)
+    if nq < BLAS_THRESHOLD:
+        D, I = flat_search_exact(q.to(torch.float32).contiguous(), db, metric, kk, id_base)
+    else:
+        b = operand()
+        # nearest-column queries over raw float32 rows (quantisation): the contraction kernel prepares the rows itself
+        fused = assign_fused(q, b, metric, id_base) if (kk == 1 and q.dtype == torch.float32) else None
+        if fused is not None:
+            D, I, a = fused
+            if need_distances:
+                rescore_topk_(q, db, a, b, metric, D, I, id_base)
+        else:
+            a = prepare_operand(q, rows=True)
+            D, I = search_topk(q, a, db, b, metric, kk, id_base, precision=precision, need_distances=need_distances)
+    if kk < k:
+        Dp, Ip = topk_padding(nq, k, metric, q.device)
+        Dp[:, :kk], Ip[:, :kk] = D, I
+        D, I = Dp, Ip
+    return D, I
+
+
+def flat_range_search(q: torch.Tensor, db: torch.Tensor, metric: int, radius: float, *, operand, id_base: int = 0):
+    """Faiss's IndexFlat.range_search, dispatched like flat_search: (lims int64 [nq + 1], D, I) on the device, each
+    query's results in ascending id."""
+    nq = q.shape[0]
+    if db.shape[0] == 0 or nq == 0:
+        return range_empty(nq, q.device)
+    if nq < BLAS_THRESHOLD:
+        return range_search_exact(q.to(torch.float32).contiguous(), db, metric, radius, id_base)
+    b = operand()
+    a = prepare_operand(q, rows=True)
+    return range_search(q, a, db, b, metric, radius, id_base)
 
 
 def topk_merge(val_parts: torch.Tensor, idx_parts: torch.Tensor, metric: int):
@@ -879,7 +933,7 @@ def ivfflat_range_search(q: torch.Tensor, xs: torch.Tensor, ids: torch.Tensor, l
     radius = float(np.float32(radius))
     if nq == 0:
         last_search_stats.update(mode="ivf-range", rows=0, pairs=0, results=0, fallback_rows=0)
-        return _range_empty(0, q.device)
+        return range_empty(0, q.device)
     lib, ctx = _lib.load(), _lib.ctx(_dev(q))
     ws_bytes = lib.ise_ivfflat_range_workspace_bytes(ctx, nq, nprobe, nlist, int(max_list_len))
     ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=q.device)

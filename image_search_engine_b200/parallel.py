@@ -27,7 +27,7 @@ import torch
 import torch.distributed as dist
 
 from . import ops
-from ._lib import METRIC_IP, METRIC_L2
+from ._lib import METRIC_IP, METRIC_L2, IseError
 from .faiss_compat import ClusteringParameters, IndexFlat, IndexFlatIP, IndexFlatL2
 
 
@@ -141,25 +141,18 @@ class DeviceOps:
     def normalize(self, cent):
         ops.normalize_l2_(cent)
 
-    def search(self, q, q_op, db, b_op, metric, k, id_base):
-        """local top-k (tensor cores) + exact FP32 re-score, so the cross-rank merge compares exact scores; fewer
-        than 20 queries take the direct-difference CUDA-core kernel exactly like the unsharded IndexFlat (Faiss's
-        distance_compute_blas_threshold), so near-tied neighbours cannot differ between the two"""
-        if q.shape[0] < 20:
-            qf = q if q.dtype == torch.float32 else q.to(torch.float32)
-            return ops.flat_search_exact(qf.contiguous(), db, metric, k, id_base=id_base)
-        return ops.search_topk(q, q_op, db, b_op, metric, k, id_base=id_base)
+    def search(self, q, db, b_op, metric, k, id_base):
+        """local top-k with exact FP32 scores, so the cross-rank merge compares exact scores; the unsharded IndexFlat's
+        own dispatch, so near-tied neighbours cannot differ between the two"""
+        return ops.flat_search(q, db, metric, k, operand=lambda: b_op, id_base=id_base)
 
     def merge(self, D_parts, I_parts, metric):
         return ops.topk_merge(D_parts, I_parts, metric)
 
-    def range_search(self, q, q_op, db, b_op, metric, radius, id_base):
-        """local range search -> (lims int64 [nq + 1], D, I) with global ids, ascending within a query; fewer than 20
-        queries take the direct-formula path like the unsharded IndexFlat"""
-        if q.shape[0] < 20:
-            qf = q if q.dtype == torch.float32 else q.to(torch.float32)
-            return ops.range_search_exact(qf.contiguous(), db, metric, radius, id_base=id_base)
-        return ops.range_search(q, q_op, db, b_op, metric, radius, id_base=id_base)
+    def range_search(self, q, db, b_op, metric, radius, id_base):
+        """local range search -> (lims int64 [nq + 1], D, I) with global ids, ascending within a query; the unsharded
+        IndexFlat's own dispatch"""
+        return ops.flat_range_search(q, db, metric, radius, operand=lambda: b_op, id_base=id_base)
 
 
 def _world(group):
@@ -433,17 +426,16 @@ class ShardedIndexFlat:
         all-gather of the merged slices gives every rank the full answer -- (2 - 1/world) * nq * k * 12 bytes per rank
         instead of world * nq * k * 12, and no redundant merging."""
         rank, world = _world(self.group)
-        qd = self.lops.to_local(q)
         k = int(k)
+        if not 1 <= k <= ops.MAX_TOPK:            # on every rank, before any of them enters the exchange
+            raise IseError(f"topk must be in [1, {ops.MAX_TOPK}]")
+        qd = self.lops.to_local(q)
         nq = int(qd.shape[0])
-        largest = self.metric_type == METRIC_IP
-        pad = -3.4028234663852886e38 if largest else 3.4028234663852886e38
         if self._local is None or self._local.shape[0] == 0 or nq == 0:
             # a rank that owns no rows still takes part in the exchange with empty (padded) lists
-            D = torch.full((nq, k), pad, dtype=torch.float32, device=qd.device)
-            I = torch.full((nq, k), -1, dtype=torch.int64, device=qd.device)
+            D, I = ops.topk_padding(nq, k, self.metric_type, qd.device)
         else:
-            D, I = self.lops.search(qd, self.lops.prepare(qd, rows=True), self._local, self._b_op, self.metric_type, k, self.id_base)
+            D, I = self.lops.search(qd, self._local, self._b_op, self.metric_type, k, self.id_base)
         if world == 1:
             return D, I
         per = -(-nq // world)                       # queries per merging rank (last slices padded)
@@ -479,12 +471,9 @@ class ShardedIndexFlat:
         dev = qd.device
         if self._local is None or self._local.shape[0] == 0 or nq == 0:
             # a rank that owns no rows still takes part in the exchange, with no results
-            lims = torch.zeros((nq + 1,), dtype=torch.int64, device=dev)
-            D = torch.empty((0,), dtype=torch.float32, device=dev)
-            I = torch.empty((0,), dtype=torch.int64, device=dev)
+            lims, D, I = ops.range_empty(nq, dev)
         else:
-            lims, D, I = self.lops.range_search(qd, self.lops.prepare(qd, rows=True), self._local, self._b_op,
-                                                self.metric_type, radius, self.id_base)
+            lims, D, I = self.lops.range_search(qd, self._local, self._b_op, self.metric_type, radius, self.id_base)
         if world == 1:
             return lims, D, I
         counts = torch.empty((world * nq,), dtype=torch.int64, device=dev)

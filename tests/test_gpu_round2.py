@@ -1,6 +1,6 @@
 """GPU tests of the round-2 boundary work: O(nnz) Okapi on CSR input, the opt-in corrected tf-idf mode, k beyond
-the fused-selection limit, thread safety of the cached host pipelines, and the sharded index's small-batch / empty
-shard handling.  All through the public Python surface, i.e. through the C ABI."""
+the fused-selection limit, thread safety of the cached host pipelines, and the sharded index's equality with the flat
+index and its empty shard handling.  All through the public Python surface, i.e. through the C ABI."""
 import threading
 from pathlib import Path
 
@@ -155,25 +155,63 @@ def test_concurrent_pipelined_transforms_share_one_bovw():
 
 
 def test_sharded_index_small_batches_and_empty_shard():
-    """world = 1 (no process group): fewer than 20 queries take the same exact kernel as the unsharded index, and a
-    shard without rows answers with padded lists instead of raising."""
+    """world = 1 (no process group): the sharded index runs the unsharded index's dispatch (ops.flat_search /
+    ops.flat_range_search) -- the exact kernel below 20 queries, the fused top-1 or the tensor-core path above -- so
+    both return the same bits; a shard without rows answers with padded lists instead of raising; k beyond the fused
+    limit is refused before any work."""
     from image_search_engine_b200 import faiss_compat
-    from image_search_engine_b200._lib import METRIC_L2
+    from image_search_engine_b200._lib import METRIC_IP, METRIC_L2, IseError
     from image_search_engine_b200.parallel import ShardedIndexFlat
     rng = np.random.default_rng(3)
     db = rng.standard_normal((5000, 40)).astype(np.float32)
-    q = db[:7] + 1e-4 * rng.standard_normal((7, 40)).astype(np.float32)
-    six = ShardedIndexFlat(40, METRIC_L2)
-    six.add_local(db)
-    flat = faiss_compat.IndexFlatL2(40)
-    flat.add(db)
-    D, I = six.search(q, 5)
-    Dr, Ir = flat.search(q, 5)
-    assert np.array_equal(I.cpu().numpy(), Ir) and np.array_equal(D.cpu().numpy(), Dr)   # same kernel, same bits
+    qf = db[:40] + 1e-4 * rng.standard_normal((40, 40)).astype(np.float32)
+    qu = rng.integers(0, 256, (40, 40), dtype=np.uint8)
+    for metric in (METRIC_IP, METRIC_L2):
+        six = ShardedIndexFlat(40, metric)
+        six.add_local(db)
+        flat = faiss_compat.IndexFlatIP(40) if metric == METRIC_IP else faiss_compat.IndexFlatL2(40)
+        flat.add(db)
+        for q in (qf, qu):
+            for nq in (7, 40):
+                for k in (1, 5, 10, 100):
+                    D, I = six.search(q[:nq], k)
+                    Dr, Ir = flat.search(q[:nq], k)
+                    assert np.array_equal(I.cpu().numpy(), Ir) and np.array_equal(D.cpu().numpy(), Dr), \
+                        (metric, q.dtype, nq, k)                                                # same kernels, same bits
+                radius = float(np.median(Dr[:, 50]))
+                got = six.range_search(q[:nq], radius)
+                want = flat.range_search(q[:nq], radius)
+                assert want[0][-1] > 0, (metric, q.dtype, nq)
+                for a, b in zip(got, want):
+                    a = a.cpu().numpy()
+                    assert np.array_equal(a, b.astype(a.dtype)), (metric, q.dtype, nq)
+        with pytest.raises(IseError, match=r"topk must be in \[1, 128\]"):
+            six.search(qf, 200)
     empty = ShardedIndexFlat(40, METRIC_L2)
     empty.add_local(np.zeros((0, 40), np.float32))
-    D, I = empty.search(q, 5)
+    D, I = empty.search(qf[:7], 5)
     assert (I.cpu().numpy() == -1).all() and (D.cpu().numpy() == np.finfo(np.float32).max).all()
+
+
+@pytest.mark.parametrize("metric_ip", [True, False])
+def test_flat_search_id_base_shifts_only_the_ids(metric_ip):
+    """ops.flat_search with id_base = 1000 (a shard's global ids) returns the id_base = 0 ids plus 1000 and the same
+    distances, on the direct-formula, tensor-core and fused top-1 paths."""
+    from image_search_engine_b200 import ops
+    from image_search_engine_b200._lib import METRIC_IP, METRIC_L2
+    rng = np.random.default_rng(8)
+    metric = METRIC_IP if metric_ip else METRIC_L2
+    dev = ops.require_cuda()
+    db = torch.from_numpy(rng.standard_normal((1000, 64)).astype(np.float32)).to(dev)
+    q = torch.from_numpy(rng.standard_normal((120_000, 64)).astype(np.float32)).to(dev)
+    op = ops.attach_sample(ops.prepare_operand(db))
+    for nq, k in ((7, 10), (40, 1), (40, 10), (120_000, 1)):
+        D0, I0 = ops.flat_search(q[:nq], db, metric, k, operand=lambda: op)
+        mode = ops.search_stats()["mode"]
+        D1, I1 = ops.flat_search(q[:nq], db, metric, k, operand=lambda: op, id_base=1000)
+        assert ops.search_stats()["mode"] == mode
+        assert torch.equal(I1, I0 + 1000) and torch.equal(D1, D0), (nq, k)
+    assert mode.startswith("fused"), mode
 
 
 # ---------------------------------------------------------------------------------------------------------------

@@ -53,8 +53,8 @@ class OracleOps:
     def normalize(self, cent):
         fs.normalize_L2(cent.numpy())
 
-    def search(self, q, q_op, db, b_op, metric, k, id_base):
-        D, I = fs.knn(q_op.numpy(), b_op.numpy(), k, metric)
+    def search(self, q, db, b_op, metric, k, id_base):
+        D, I = fs.knn(q.numpy(), b_op.numpy(), k, metric)
         I = np.where(I >= 0, I + id_base, -1)
         return torch.from_numpy(D), torch.from_numpy(I)
 

@@ -107,8 +107,8 @@ RADII = {fs.METRIC_INNER_PRODUCT: 9.0, fs.METRIC_L2: 12.0}
 
 
 class RangeOracleOps(OracleOps):
-    def range_search(self, q, q_op, db, b_op, metric, radius, id_base):
-        lims, D, I = range_search(q_op.numpy(), b_op.numpy(), radius, metric)
+    def range_search(self, q, db, b_op, metric, radius, id_base):
+        lims, D, I = range_search(q.numpy(), b_op.numpy(), radius, metric)
         return torch.from_numpy(lims.astype(np.int64)), torch.from_numpy(D), torch.from_numpy(I + id_base)
 
 
