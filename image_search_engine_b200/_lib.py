@@ -112,6 +112,14 @@ PROTOTYPES = {
                                        _c_void_p, _int, _int, C.c_float, _c_void_p, _c_void_p, _size, _c_void_p]),
     "ise_ivfflat_range_fill": (_int, [_c_void_p, _c_void_p, _i64, _int, _c_void_p, _c_void_p, _c_void_p, _i64, _i64,
                                       _int, _int, C.c_float, _c_void_p, _c_void_p, _c_void_p, _size, _c_void_p]),
+    "ise_binary_knn_workspace_bytes": (_size, [_c_void_p, _i64, _i64, _int, _int]),
+    "ise_binary_knn": (_int, [_c_void_p, _c_void_p, _i64, _c_void_p, _i64, _int, _i64, _int, _c_void_p, _c_void_p,
+                              _c_void_p, _size, _c_void_p]),
+    "ise_binary_range_workspace_bytes": (_size, [_c_void_p, _i64, _i64, _int]),
+    "ise_binary_range_count": (_int, [_c_void_p, _c_void_p, _i64, _c_void_p, _i64, _int, _i64, _int, _c_void_p,
+                                      _c_void_p, _size, _c_void_p]),
+    "ise_binary_range_fill": (_int, [_c_void_p, _c_void_p, _i64, _c_void_p, _i64, _int, _i64, _int, _c_void_p,
+                                     _c_void_p, _c_void_p, _size, _c_void_p]),
     "ise_okapi_csr": (_int, [_c_void_p, _c_void_p, _c_void_p, _c_void_p, _i64, _f64, _f64, _f64, _f64, _c_void_p, _int,
                              _c_void_p, _c_void_p]),
     "ise_tfidf_finish": (_int, [_c_void_p, _c_void_p, _int, _i64, _int, _c_void_p, _int, _c_void_p]),

@@ -15,6 +15,7 @@ All arithmetic runs in libise kernels; there is no CPU path.
 """
 from __future__ import annotations
 
+import operator
 import struct
 import threading
 import time
@@ -570,10 +571,141 @@ class IndexIVFFlat:
                 f"ntotal={self.ntotal} (HBM resident)>")
 
 
+def _binary_rows(x, code_size: int, what: str):
+    """uint8 code rows [n, code_size] as given (NumPy array or tensor), checked without device work: another dtype raises
+    TypeError like faiss's _check_dtype_uint8, another shape AssertionError."""
+    a = x if isinstance(x, torch.Tensor) else np.asarray(x)
+    if a.dtype != (torch.uint8 if isinstance(a, torch.Tensor) else np.uint8):
+        raise TypeError(f"{what}: binary codes must be uint8, got {a.dtype}")
+    if a.ndim != 2 or a.shape[1] != code_size:
+        raise AssertionError(f"{what}: expected (n, {code_size}) uint8 array")
+    return a
+
+
+class IndexBinaryFlat:
+    """faiss.IndexBinaryFlat (faiss/IndexBinaryFlat.cpp, faiss/utils/hamming.cpp, ~1.7.4): exhaustive search over
+    packed binary codes -- ORB (d = 256 bits), BRISK / FREAK (512), dHash (64) -- by Hamming distance.
+
+    ``d`` is in bits (a multiple of 8, at most 2048: the scan keeps a query's words in registers); ``code_size = d // 8``.
+    Codes are uint8 rows [n, code_size], NumPy or CUDA tensors, with ids ntotal + i; they live in HBM with each row
+    padded with zero bytes to a multiple of 16.  ``search`` returns (D int32, I int64) sorted by (distance, id): among
+    equal distances the lowest ids win, also when the tie falls on the k-th place.  ``range_search`` keeps every code with
+    distance < radius, in ascending id, with the same distances.  Both run ``ise_binary_knn`` /
+    ``ise_binary_range_count`` + ``_fill`` (XOR + popcount on CUDA cores, no [nq, ntotal] matrix).  Restated from
+    memory like the rest of the Faiss semantics here (tests/_binary_oracle.py); no parity run against Faiss itself.
+    """
+
+    def __init__(self, d: int):
+        d = int(d)
+        if d <= 0 or d % 8 != 0:
+            raise RuntimeError("Error: 'd % 8 == 0' failed")     # FAISS_THROW_IF_NOT in IndexBinary::IndexBinary
+        if d // 8 > ops.BINARY_MAX_CODE_SIZE:
+            raise NotImplementedError(f"IndexBinaryFlat supports d <= {8 * ops.BINARY_MAX_CODE_SIZE} bits")
+        self.d, self.code_size = d, d // 8
+        self.is_trained = True
+        self.verbose = False
+        self._lock = threading.Lock()
+        self._chunks: list[torch.Tensor] = []    # padded device rows [n, pitch], in id order
+        self._ntotal = 0
+        self._codes: torch.Tensor | None = None  # their concatenation, built at the next search
+
+    @property
+    def ntotal(self) -> int:
+        return self._ntotal
+
+    def _device_rows(self, a) -> tuple[torch.Tensor, bool]:
+        """Checked rows -> (zero-padded contiguous copy [n, pitch] on the device, input_was_cuda)."""
+        dev = ops.require_cuda()
+        was_cuda = isinstance(a, torch.Tensor) and a.is_cuda
+        t = a if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a))
+        rows = torch.zeros((t.shape[0], ops.binary_pitch(self.code_size)), dtype=torch.uint8, device=dev)
+        rows[:, :self.code_size] = t.to(dev, non_blocking=True)
+        return rows, was_cuda
+
+    def add(self, x) -> None:
+        rows, _ = self._device_rows(_binary_rows(x, self.code_size, "add"))
+        with self._lock:
+            self._chunks.append(rows)
+            self._ntotal += rows.shape[0]
+            self._codes = None
+
+    def train(self, x) -> None:
+        pass
+
+    def reset(self) -> None:
+        with self._lock:
+            self._chunks, self._ntotal, self._codes = [], 0, None
+
+    def _database(self) -> torch.Tensor:
+        with self._lock:
+            if self._codes is None:
+                if not self._chunks:
+                    dev = ops.require_cuda()
+                    self._codes = torch.zeros((0, ops.binary_pitch(self.code_size)), dtype=torch.uint8, device=dev)
+                else:
+                    self._codes = self._chunks[0] if len(self._chunks) == 1 else torch.cat(self._chunks)
+                    self._chunks = [self._codes]
+            return self._codes
+
+    def search(self, x, k: int):
+        """hammings_knn_hc: the k nearest codes of every query, (D int32 [nq, k], I int64 [nq, k]) in the canonical
+        (distance, id) order; when k > ntotal the tail is id -1 with D = 2^31 - 1 (the neutral value of Faiss's
+        CMax<int32> heap, recalled rather than checked against Faiss).  1 <= k <= 128."""
+        k = int(k)
+        if k <= 0:
+            raise AssertionError("k must be positive")
+        if k > ops.MAX_TOPK:
+            raise NotImplementedError(f"IndexBinaryFlat.search supports k <= {ops.MAX_TOPK}")
+        q, was_cuda = self._device_rows(_binary_rows(x, self.code_size, "search"))
+        db = self._database()
+        if q.shape[0] and db.shape[0]:
+            D, I = ops.binary_knn(q, db, self.code_size, k)
+        else:
+            D = torch.full((q.shape[0], k), 2**31 - 1, dtype=torch.int32, device=q.device)
+            I = torch.full((q.shape[0], k), -1, dtype=torch.int64, device=q.device)
+        if was_cuda:
+            return D, I
+        return D.cpu().numpy(), I.cpu().numpy()
+
+    def range_search(self, x, radius: int):
+        """hamming_range_search: every stored code with Hamming distance < radius (strict).  Returns (lims [nq + 1], D
+        int32, I int64); the results of query i are D[lims[i]:lims[i+1]] / I[...] in ascending id.  NumPy input gives
+        NumPy output (lims uint64, like Faiss's size_t array); CUDA tensors give CUDA tensors (lims int64)."""
+        radius = operator.index(radius)
+        q, was_cuda = self._device_rows(_binary_rows(x, self.code_size, "range_search"))
+        lims, D, I = ops.binary_range_search(q, self._database(), self.code_size, radius)
+        if was_cuda:
+            return lims, D, I
+        return lims.cpu().numpy().astype(np.uint64), D.cpu().numpy(), I.cpu().numpy()
+
+    def reconstruct(self, i: int) -> np.ndarray:
+        return self._database()[int(i), :self.code_size].cpu().numpy()
+
+    def reconstruct_n(self, i0: int = 0, ni: int = -1) -> np.ndarray:
+        if ni < 0:
+            ni = self._ntotal - i0
+        return self._database()[i0:i0 + ni, :self.code_size].cpu().numpy()
+
+    def __repr__(self):
+        return f"<image_search_engine_b200.IndexBinaryFlat d={self.d} ntotal={self.ntotal} (HBM resident)>"
+
+    # joblib / pickle: the codes as a host array
+    def __getstate__(self):
+        return {"d": self.d, "codes": self.reconstruct_n() if self._ntotal else np.zeros((0, self.code_size), np.uint8)}
+
+    def __setstate__(self, st):
+        self.__init__(st["d"])
+        if st["codes"].shape[0]:
+            self.add(st["codes"])
+
+
 # ------------------------------------------------------------------------------------------
 # flat index file format (faiss/impl/index_write.cpp), so existing models/*.faiss files open
 # ------------------------------------------------------------------------------------------
 def write_index(index: IndexFlat, fname) -> None:
+    if isinstance(index, IndexBinaryFlat):
+        raise NotImplementedError("Faiss writes binary indexes with write_index_binary (IBxF), which is not provided; "
+                                  "an IndexBinaryFlat can be pickled")
     if isinstance(index, (IndexIVFPQ, IndexIVFFlat)):
         name = type(index).__name__
         raise NotImplementedError(f"only flat indexes are written in Faiss's file format; an {name} can be pickled")

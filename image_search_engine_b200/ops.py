@@ -955,6 +955,85 @@ def ivfflat_range_search(q: torch.Tensor, xs: torch.Tensor, ids: torch.Tensor, l
 
 
 # ------------------------------------------------------------------------------------------
+# binary codes (IndexBinaryFlat)
+# ------------------------------------------------------------------------------------------
+BINARY_MAX_CODE_SIZE = 256      # bytes (2048 bits): the scan kernels keep a query's words in registers
+
+
+def binary_pitch(code_size: int) -> int:
+    """Row pitch of stored binary codes and queries: code_size rounded up to 16 bytes (the pad bytes are zero)."""
+    return (int(code_size) + 15) // 16 * 16
+
+
+def _binary_args(q: torch.Tensor, codes: torch.Tensor, code_size: int):
+    if q.dtype != torch.uint8 or codes.dtype != torch.uint8 or not q.is_contiguous() or not codes.is_contiguous():
+        raise IseError("binary search needs contiguous uint8 query and code rows")
+    pitch = binary_pitch(code_size)
+    if q.dim() != 2 or codes.dim() != 2 or q.shape[1] != pitch or codes.shape[1] != pitch:
+        raise IseError(f"binary search: rows of {pitch} bytes (code_size {code_size} padded with zeros)")
+    return pitch
+
+
+def binary_knn_workspace_bytes(nq: int, ntotal: int, code_size: int, topk: int) -> int:
+    """Device scratch of one binary_knn call (the bound is in include/ise.h)."""
+    return int(_lib.load().ise_binary_knn_workspace_bytes(_lib.ctx(torch.cuda.current_device()), int(nq), int(ntotal),
+                                                           int(code_size), int(topk)))
+
+
+def binary_knn(q: torch.Tensor, codes: torch.Tensor, code_size: int, topk: int):
+    """Exact Hamming top-k of every query row over the stored codes (IndexBinaryFlat.search): q [nq, pitch] and codes
+    [ntotal, pitch] uint8, zero past code_size.  Returns (D int32 [nq, topk], I int64 [nq, topk]) sorted by (distance,
+    id); padding is id -1 / 2^31 - 1."""
+    pitch = _binary_args(q, codes, code_size)
+    if not 1 <= topk <= MAX_TOPK:
+        raise IseError(f"topk must be in [1, {MAX_TOPK}]")
+    nq, ntotal = q.shape[0], codes.shape[0]
+    D = torch.empty((nq, topk), dtype=torch.int32, device=q.device)
+    I = torch.empty((nq, topk), dtype=torch.int64, device=q.device)
+    if nq == 0:
+        return D, I
+    lib, ctx = _lib.load(), _lib.ctx(_dev(q))
+    ws_bytes = lib.ise_binary_knn_workspace_bytes(ctx, nq, ntotal, int(code_size), int(topk))
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=q.device)
+    _lib.check(lib.ise_binary_knn(ctx, _ptr(q), nq, _ptr(codes), ntotal, int(code_size), pitch, int(topk), _ptr(D),
+                                  _ptr(I), _ptr(ws), ws_bytes, _stream()))
+    _count(3)
+    return D, I
+
+
+def binary_range_workspace_bytes(nq: int, ntotal: int, code_size: int) -> int:
+    """Device scratch of one binary_range_search call (the bound is in include/ise.h)."""
+    return int(_lib.load().ise_binary_range_workspace_bytes(_lib.ctx(torch.cuda.current_device()), int(nq),
+                                                             int(ntotal), int(code_size)))
+
+
+def binary_range_search(q: torch.Tensor, codes: torch.Tensor, code_size: int, radius: int):
+    """Every stored code within Hamming distance < radius of each query (IndexBinaryFlat.range_search).  Inputs as
+    binary_knn.  Returns (lims int64 [nq + 1], D int32, I int64) on the device; the results of query i are
+    D / I[lims[i]:lims[i+1]] in ascending id.  One readback: the total, lims[nq]."""
+    pitch = _binary_args(q, codes, code_size)
+    nq, ntotal = q.shape[0], codes.shape[0]
+    if nq == 0 or ntotal == 0:
+        lims, D, I = range_empty(nq, q.device)
+        return lims, D.to(torch.int32), I
+    radius = min(max(int(radius), 0), 1 << 30)           # every distance is in [0, 2048]: the result is the same
+    lib, ctx = _lib.load(), _lib.ctx(_dev(q))
+    ws_bytes = lib.ise_binary_range_workspace_bytes(ctx, nq, ntotal, int(code_size))
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=q.device)
+    lims = torch.empty((nq + 1,), dtype=torch.int64, device=q.device)
+    _lib.check(lib.ise_binary_range_count(ctx, _ptr(q), nq, _ptr(codes), ntotal, int(code_size), pitch, radius,
+                                          _ptr(lims), _ptr(ws), ws_bytes, _stream()))
+    total = int(lims[nq].item())                          # the one readback: sizes D / I
+    D = torch.empty((total,), dtype=torch.int32, device=q.device)
+    I = torch.empty((total,), dtype=torch.int64, device=q.device)
+    if total:
+        _lib.check(lib.ise_binary_range_fill(ctx, _ptr(q), nq, _ptr(codes), ntotal, int(code_size), pitch, radius,
+                                             _ptr(D), _ptr(I), _ptr(ws), ws_bytes, _stream()))
+    _count(5 if total else 4)                             # count, the offsets scan (two CUB kernels), lims, fill
+    return lims, D, I
+
+
+# ------------------------------------------------------------------------------------------
 # k-means update
 # ------------------------------------------------------------------------------------------
 def kmeans_accumulate(x: torch.Tensor, assign: torch.Tensor, dis: torch.Tensor | None, sums: torch.Tensor,

@@ -430,6 +430,42 @@ int ise_ivfflat_range_fill(ise_ctx* ctx, const float* q, int64_t nq, int d, cons
                            int nprobe, int metric, float radius, float* out_dis, int64_t* out_ids, void* workspace,
                            size_t workspace_bytes, void* stream);
 
+/* ---- binary flat index (faiss/IndexBinaryFlat.cpp, faiss/utils/hamming.cpp) ---------------------------------------
+ * Exact Hamming distances between packed binary codes (ORB 256-bit, BRISK 512-bit, dHash 64-bit, ...): q[nq] and
+ * codes[ntotal] are uint8 rows of code_size bytes (1 <= code_size <= 256, i.e. d <= 2048 bits) stored with a row pitch
+ * `pitch` (a multiple of 16, 16-byte aligned base) whose bytes past code_size are ZERO in both operands.  Ids are row
+ * numbers.  Rows are scanned as 64-bit XOR + popcount words on CUDA cores; no [nq, ntotal] matrix is built and there is
+ * no host synchronisation inside a call.  The reference searches ORB / BRISK descriptors only as uint8 float rows
+ * (descriptors.py:216-258, indexer.py:34-37) and compares dHashes with a NumPy Hamming distance (utils.py:65-88).
+ *
+ * ise_binary_knn (hammings_knn_hc): out_dis[nq, topk] int32 distances and out_idx[nq, topk] int64 ids, sorted by
+ * (distance, id) ascending -- among equal distances the lowest ids win; padding (topk > ntotal) is id -1 with distance
+ * 2^31 - 1.  1 <= topk <= 128, ntotal < 2^31.  The database is cut into S <= 256 column chunks whose partial lists are
+ * joined with ise_topk_merge.  Workspace (ise_binary_knn_workspace_bytes) is 12 bytes per partial-list entry for the
+ * nq * S * topk entries, S chosen so that there are at most max(2^24, nq * topk) of them, plus 4 bytes per output entry,
+ * each part rounded up to 256 bytes: <= 12 * max(2^24, nq * topk) + 4 * nq * topk + 768 bytes. */
+size_t ise_binary_knn_workspace_bytes(ise_ctx* ctx, int64_t nq, int64_t ntotal, int code_size, int topk);
+int ise_binary_knn(ise_ctx* ctx, const uint8_t* q, int64_t nq, const uint8_t* codes, int64_t ntotal, int code_size,
+                   int64_t pitch, int topk, int32_t* out_dis, int64_t* out_idx, void* workspace, size_t workspace_bytes,
+                   void* stream);
+/* Range search (hamming_range_search): every code with distance < radius (strict).  Results of query i are
+ * out[lims[i] .. lims[i + 1]) in ascending id, with the same int32 distances ise_binary_knn returns.  Two calls on the
+ * same stream with the same arguments and the same workspace, untouched in between:
+ *   ise_binary_range_count  counts the hits of every (query, column chunk) segment, scans them into int64 offsets
+ *                           (totals above 2^31 are fine) and writes lims[nq + 1] (lims[0] = 0 for nq == 0);
+ *   ise_binary_range_fill   re-scans the chunks that have hits and writes out_dis / out_ids[lims[nq]] (warp ballots and
+ *                           popc prefixes give the slots in id order, no sort).
+ * The caller reads lims[nq] to size the outputs.  Workspace (ise_binary_range_workspace_bytes) is 16 bytes per segment
+ * (count, offset) for the nq * S segments, S <= 256 chosen so that there are at most max(2^22, nq) of them, plus the
+ * offsets scan's scratch (ise_range_lims_workspace_bytes). */
+size_t ise_binary_range_workspace_bytes(ise_ctx* ctx, int64_t nq, int64_t ntotal, int code_size);
+int ise_binary_range_count(ise_ctx* ctx, const uint8_t* q, int64_t nq, const uint8_t* codes, int64_t ntotal,
+                           int code_size, int64_t pitch, int radius, int64_t* lims, void* workspace,
+                           size_t workspace_bytes, void* stream);
+int ise_binary_range_fill(ise_ctx* ctx, const uint8_t* q, int64_t nq, const uint8_t* codes, int64_t ntotal,
+                          int code_size, int64_t pitch, int radius, int32_t* out_dis, int64_t* out_ids,
+                          void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- collectives for a single-process multi-GPU host (NCCL over NVLink, resolved with dlopen at run time) ----------
  * The two exchange steps of the sharded path (SURVEY section 8e): the per-iteration all-reduce of the k-means
  * [k*d sums | k counts] buffer and the all-gather of per-shard top-k lists before ise_topk_merge.  The Python host
