@@ -120,6 +120,16 @@ PROTOTYPES = {
                                       _c_void_p, _size, _c_void_p]),
     "ise_binary_range_fill": (_int, [_c_void_p, _c_void_p, _i64, _c_void_p, _i64, _int, _i64, _int, _c_void_p,
                                      _c_void_p, _c_void_p, _size, _c_void_p]),
+    "ise_binary_ivf_search_workspace_bytes": (_size, [_c_void_p, _i64, _int, _i64, _i64, _int, _int]),
+    "ise_binary_ivf_search": (_int, [_c_void_p, _c_void_p, _i64, _c_void_p, _c_void_p, _c_void_p, _i64, _i64, _int, _i64,
+                                     _c_void_p, _int, _int, _c_void_p, _c_void_p, _c_void_p, _size, _c_void_p]),
+    "ise_binary_ivf_range_workspace_bytes": (_size, [_c_void_p, _i64, _int, _i64, _i64, _int]),
+    "ise_binary_ivf_range_count": (_int, [_c_void_p, _c_void_p, _i64, _c_void_p, _c_void_p, _c_void_p, _i64, _i64, _int,
+                                          _i64, _c_void_p, _int, _int, _c_void_p, _c_void_p, _size, _c_void_p]),
+    "ise_binary_ivf_range_fill": (_int, [_c_void_p, _c_void_p, _i64, _c_void_p, _c_void_p, _c_void_p, _i64, _i64, _int,
+                                         _i64, _int, _int, _c_void_p, _c_void_p, _c_void_p, _size, _c_void_p]),
+    "ise_binary_to_real": (_int, [_c_void_p, _c_void_p, _i64, _int, _i64, _c_void_p, _c_void_p]),
+    "ise_real_to_binary": (_int, [_c_void_p, _c_void_p, _i64, _int, _i64, _c_void_p, _c_void_p]),
     "ise_okapi_csr": (_int, [_c_void_p, _c_void_p, _c_void_p, _c_void_p, _i64, _f64, _f64, _f64, _f64, _c_void_p, _int,
                              _c_void_p, _c_void_p]),
     "ise_tfidf_finish": (_int, [_c_void_p, _c_void_p, _int, _i64, _int, _c_void_p, _int, _c_void_p]),

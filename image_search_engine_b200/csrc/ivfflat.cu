@@ -1,10 +1,8 @@
 // IndexIVFFlat search: exact FP32 scan of the probed inverted lists (faiss/IndexIVFFlat.cpp IVFFlatScanner,
 // faiss/utils/distances.cpp fvec_inner_product / fvec_L2sqr) without an [nq, ntotal] score matrix.
 //
-//   ivf_probe_keys / radix sort  the nq * nprobe (query, probe slot) pairs sorted by list id (stable: the queries
-//                                of a list stay in ascending pair order);
-//   ivf_list_items / scan        per list: its first sorted pair and its number of work items
-//                                ceil(queries / kQB) * chunks; exclusive scan -> item offsets;
+//   grouping (ivf_grouping.cuh)  the nq * nprobe (query, probe slot) pairs sorted by list id, and per list
+//                                ceil(queries / kQB) * chunks work items of chunks of kCB-row granules;
 //   ivfflat_scan_kernel          one work item = (list, block of <= kQB of its queries, chunk of its vectors).  The
 //                                block's queries and kCB vectors at a time go through shared memory kDK dimensions at
 //                                a time; each thread accumulates a 4 x 4 piece of the kQB x kCB score tile with the
@@ -25,71 +23,17 @@
 //   ivfflat_range_fill_kernel    re-runs the items with hits and writes each segment's hits in list order.
 // Every kernel scores through score_tile, so search and range search return bit-identical distances.  S is capped at
 // 256 / nprobe and so that the segment table holds at most max(2^22, nq * nprobe) entries.
-#include <cub/device/device_radix_sort.cuh>
-#include <cub/device/device_scan.cuh>
-
-#include <algorithm>
-
 #include "common.cuh"
+#include "ivf_grouping.cuh"
 #include "topk_list.cuh"
 
 namespace {
 
+using ivf::kThreads;                // 16 x 8 threads, 4 x 4 scores each
 constexpr int kQB = 32;             // queries per work item
-constexpr int kCB = 64;             // vectors per score tile
+constexpr int kCB = 64;             // vectors per score tile (the chunk granule)
 constexpr int kDK = 32;             // dimensions per shared-memory slice
-constexpr int kThreads = 128;       // 16 x 8 threads, 4 x 4 scores each
-constexpr int kMergeFanIn = 256;    // ise_topk_merge: at most 256 lists per row
 constexpr int kWarps = kThreads / 32;
-constexpr int64_t kPartialBudget = int64_t(1) << 24;
-constexpr int64_t kSegmentBudget = int64_t(1) << 22;   // range search: (pair, chunk) segments
-
-static inline size_t align256(size_t b) { return (b + 255) & ~size_t(255); }
-
-__host__ __device__ __forceinline__ int64_t list_chunks(int64_t len, int S) {
-    return len == 0 ? 1 : (int64_t)min((int64_t)S, (len + kCB - 1) / kCB);
-}
-
-// a pair without a list (probe -1) sorts after every list and gets no work item: its partial slots are marked empty
-__global__ void ivf_probe_keys_kernel(const int64_t* __restrict__ probes, int64_t nq, int nprobe, int64_t nlist, int S,
-                                      int topk, int32_t* __restrict__ keys, int32_t* __restrict__ vals,
-                                      int64_t* __restrict__ part_idx) {
-    const int64_t npairs = nq * nprobe;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < npairs; i += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t l = probes[i];
-        const bool ok = l >= 0 && l < nlist;
-        keys[i] = ok ? (int32_t)l : (int32_t)nlist;
-        vals[i] = (int32_t)i;
-        if (!ok && part_idx)
-            for (int c = 0; c < S; ++c) part_idx[(((i % nprobe) * S + c) * nq + i / nprobe) * topk] = -1;
-    }
-}
-
-__device__ __forceinline__ int64_t lower_bound_i32(const int32_t* __restrict__ a, int64_t n, int32_t key) {
-    int64_t lo = 0, hi = n;
-    while (lo < hi) {
-        const int64_t mid = (lo + hi) >> 1;
-        if (a[mid] < key) lo = mid + 1;
-        else hi = mid;
-    }
-    return lo;
-}
-
-// qoff[l] = first sorted pair of list l (qoff[nlist] = number of valid pairs); items[l] = work items of list l
-__global__ void ivf_list_items_kernel(const int32_t* __restrict__ keys_sorted, int64_t npairs,
-                                      const int64_t* __restrict__ list_off, int64_t nlist, int S,
-                                      int32_t* __restrict__ qoff, int64_t* __restrict__ items) {
-    for (int64_t l = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; l <= nlist; l += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t lo = lower_bound_i32(keys_sorted, npairs, (int32_t)l);
-        qoff[l] = (int32_t)lo;
-        if (l == nlist) {
-            items[l] = 0;
-        } else {
-            const int64_t nql = lower_bound_i32(keys_sorted, npairs, (int32_t)(l + 1)) - lo;
-            items[l] = nql ? (nql + kQB - 1) / kQB * list_chunks(list_off[l + 1] - list_off[l], S) : 0;
-        }
-    }
-}
 
 // four consecutive columns c .. c+3 of a row (zeros past d or for a missing row); vec: d % 4 == 0, 16-byte rows
 __device__ __forceinline__ float4 load4(const float* __restrict__ row, int c, int d, bool vec) {
@@ -101,40 +45,6 @@ __device__ __forceinline__ float4 load4(const float* __restrict__ row, int c, in
     if (c + 2 < d) v.z = __ldg(row + c + 2);
     if (c + 3 < d) v.w = __ldg(row + c + 3);
     return v;
-}
-
-struct Item {
-    int64_t lbase, nch, c;              // first row of the list, its chunks, this item's chunk
-    int64_t v_begin, v_end;             // the chunk's vectors, in list positions
-};
-
-// work item w of the persistent loop: its list (item_off[l] <= w < item_off[l + 1]), query block and vector chunk; the
-// block's pairs go to s_pair (-1 past the block).  The caller synchronises before reading s_pair.
-__device__ __forceinline__ Item decode_item(int64_t w, const int64_t* __restrict__ list_off, int64_t nlist,
-                                            const int32_t* __restrict__ pairs_sorted, const int32_t* __restrict__ qoff,
-                                            const int64_t* __restrict__ item_off, int S, int tid, int* s_pair) {
-    int64_t lo = 0, hi = nlist;
-    while (hi - lo > 1) {
-        const int64_t mid = (lo + hi) >> 1;
-        if (item_off[mid] <= w) lo = mid;
-        else hi = mid;
-    }
-    const int64_t l = lo;
-    Item it;
-    it.lbase = list_off[l];
-    const int64_t len = list_off[l + 1] - it.lbase;
-    const int64_t nch = list_chunks(len, S);
-    const int64_t local = w - item_off[l];
-    const int64_t qb = local / nch;
-    it.nch = nch;
-    it.c = local % nch;
-    const int64_t p0 = qoff[l] + qb * kQB;
-    const int nqb = (int)min((int64_t)kQB, (int64_t)qoff[l + 1] - p0);
-    if (tid < kQB) s_pair[tid] = tid < nqb ? pairs_sorted[p0 + tid] : -1;
-    const int64_t cl = (len + nch - 1) / nch;
-    it.v_begin = min(len, it.c * cl);
-    it.v_end = min(len, it.v_begin + cl);
-    return it;
 }
 
 // s_s[r][j] = score of pair s_pair[r] against list vector t0 + j (r < kQB, j < nv) with the direct formulas: one
@@ -214,7 +124,7 @@ __global__ void __launch_bounds__(kThreads) ivfflat_scan_kernel(
         __syncthreads();
         const int64_t w = s_item;
         if (w >= total) break;
-        const Item it = decode_item(w, list_off, nlist, pairs_sorted, qoff, item_off, S, tid, s_pair);
+        const ivf::Item it = ivf::decode_item(w, list_off, nlist, pairs_sorted, qoff, item_off, S, kCB, kQB, tid, s_pair);
         const int64_t lbase = it.lbase, c = it.c;
         const float* xl = xs + lbase * (int64_t)d;
         __syncthreads();
@@ -285,7 +195,7 @@ __global__ void __launch_bounds__(kThreads) ivfflat_range_count_kernel(
         __syncthreads();
         const int64_t w = s_item;
         if (w >= total) break;
-        const Item it = decode_item(w, list_off, nlist, pairs_sorted, qoff, item_off, S, tid, s_pair);
+        const ivf::Item it = ivf::decode_item(w, list_off, nlist, pairs_sorted, qoff, item_off, S, kCB, kQB, tid, s_pair);
         const float* xl = xs + it.lbase * (int64_t)d;
         __syncthreads();
         int hits[kQB / kWarps];
@@ -341,7 +251,7 @@ __global__ void __launch_bounds__(kThreads) ivfflat_range_fill_kernel(
         __syncthreads();
         const int64_t w = s_item;
         if (w >= total) break;
-        const Item it = decode_item(w, list_off, nlist, pairs_sorted, qoff, item_off, S, tid, s_pair);
+        const ivf::Item it = ivf::decode_item(w, list_off, nlist, pairs_sorted, qoff, item_off, S, kCB, kQB, tid, s_pair);
         const float* xl = xs + it.lbase * (int64_t)d;
         const int64_t* il = ids + it.lbase;
         __syncthreads();
@@ -388,117 +298,6 @@ __global__ void __launch_bounds__(kThreads) ivfflat_range_fill_kernel(
     }
 }
 
-struct Plan {
-    int S;                 // chunks per list (partial-list / segment slots per probe)
-    int64_t npairs, g;     // nq * nprobe; slots per query = nprobe * S
-    int end_bit;           // radix-sort key bits (list ids 0 .. nlist)
-    size_t sort_tmp, scan_tmp, pairs, lists, grouping;
-    size_t parts, level;   // search: partial lists and merge levels
-    int64_t segs;          // range: nq * nprobe * S (pair, chunk) segments
-    size_t seg, lims_tmp;  // range: one int64 per segment + 1 (counts, offsets); ise_range_lims scratch
-};
-
-// the (query, probe) grouping both searches share; S covers the longest list, stays <= 256 / nprobe and <= room
-static Plan make_plan(int64_t nq, int nprobe, int64_t nlist, int64_t max_list_len, int64_t room) {
-    Plan p{};
-    const int64_t need = std::max<int64_t>(1, ceil_div64(max_list_len, kCB));
-    // a query's nprobe * S partial lists fit one merge while nprobe <= 256: beyond 256 / nprobe chunks per list the
-    // (list, query block) items already fill the machine and more chunks only add merge levels
-    const int64_t one_merge = std::max<int64_t>(1, kMergeFanIn / nprobe);
-    p.S = (int)std::min({need, std::max<int64_t>(1, room), one_merge});
-    p.npairs = nq * nprobe;
-    p.g = (int64_t)nprobe * p.S;
-    p.end_bit = 1;
-    while (p.end_bit < 31 && ((int64_t)1 << p.end_bit) <= nlist) ++p.end_bit;
-    cub::DeviceRadixSort::SortPairs(nullptr, p.sort_tmp, (const int32_t*)nullptr, (int32_t*)nullptr,
-                                    (const int32_t*)nullptr, (int32_t*)nullptr, (int)p.npairs, 0, p.end_bit);
-    cub::DeviceScan::ExclusiveSum(nullptr, p.scan_tmp, (const int64_t*)nullptr, (int64_t*)nullptr, (int)(nlist + 1));
-    p.pairs = align256((size_t)p.npairs * sizeof(int32_t));
-    p.lists = align256((size_t)(nlist + 1) * sizeof(int64_t));
-    p.grouping = 4 * p.pairs + align256(p.sort_tmp) + 3 * p.lists + align256(p.scan_tmp) + 256;
-    return p;
-}
-
-static Plan search_plan(int64_t nq, int nprobe, int64_t nlist, int64_t max_list_len, int topk) {
-    Plan p = make_plan(nq, nprobe, nlist, max_list_len, kPartialBudget / std::max<int64_t>(1, nq * nprobe * (int64_t)topk));
-    const size_t entries = (size_t)p.g * nq * topk;
-    p.parts = align256(entries * sizeof(float)) + align256(entries * sizeof(int64_t));
-    const size_t lv = p.g > kMergeFanIn ? (size_t)ceil_div64(p.g, kMergeFanIn) * nq * topk : 0;
-    p.level = align256(lv * sizeof(float)) + align256(lv * sizeof(int64_t));
-    return p;
-}
-
-static Plan range_plan(ise_ctx* ctx, int64_t nq, int nprobe, int64_t nlist, int64_t max_list_len) {
-    Plan p = make_plan(nq, nprobe, nlist, max_list_len, kSegmentBudget / std::max<int64_t>(1, nq * nprobe));
-    p.segs = p.g * nq;
-    p.seg = align256((size_t)(p.segs + 1) * sizeof(int64_t));
-    p.lims_tmp = align256(ise_range_lims_workspace_bytes(ctx, p.segs));
-    return p;
-}
-
-static bool plan_args_ok(int64_t nq, int nprobe, int64_t nlist, int64_t max_list_len, int topk) {
-    return nq > 0 && nprobe >= 1 && nlist >= 1 && nlist < ((int64_t)1 << 30) && max_list_len >= 0 && topk >= 1 &&
-           topk <= 128 && nq * nprobe < ((int64_t)1 << 31);
-}
-
-struct Grouping {
-    int32_t *keys, *keys_sorted, *vals, *pairs_sorted, *qoff;
-    int64_t *items, *item_off;
-    void *sort_tmp, *scan_tmp;
-    unsigned long long* counter;   // next work item of the persistent kernels
-};
-
-static uint8_t* take(uint8_t*& w, size_t bytes) {
-    uint8_t* r = w;
-    w += bytes;
-    return r;
-}
-
-// the first p.grouping bytes of a workspace
-static Grouping carve_grouping(uint8_t*& w, const Plan& p) {
-    Grouping g;
-    g.keys = reinterpret_cast<int32_t*>(take(w, p.pairs));
-    g.keys_sorted = reinterpret_cast<int32_t*>(take(w, p.pairs));
-    g.vals = reinterpret_cast<int32_t*>(take(w, p.pairs));
-    g.pairs_sorted = reinterpret_cast<int32_t*>(take(w, p.pairs));
-    g.sort_tmp = take(w, align256(p.sort_tmp));
-    g.qoff = reinterpret_cast<int32_t*>(take(w, p.lists));
-    g.items = reinterpret_cast<int64_t*>(take(w, p.lists));
-    g.item_off = reinterpret_cast<int64_t*>(take(w, p.lists));
-    g.scan_tmp = take(w, align256(p.scan_tmp));
-    g.counter = reinterpret_cast<unsigned long long*>(take(w, 256));
-    return g;
-}
-
-// groups the (query, probe slot) pairs by list and numbers the work items; zeroes the item counter.  part_idx (search
-// only, else null): the partial lists of pairs without a list are marked empty.
-static int group_pairs(ise_ctx* ctx, const Plan& p, const Grouping& g, const int64_t* probes, int64_t nq, int nprobe,
-                       int64_t nlist, const int64_t* list_off, int topk, int64_t* part_idx, cudaStream_t st) {
-    ISE_CUDA(cudaMemsetAsync(g.counter, 0, sizeof(unsigned long long), st));
-    const int grid_pairs = (int)std::min<int64_t>(ceil_div64(p.npairs, 256), (int64_t)ctx->sm_count * 8);
-    ivf_probe_keys_kernel<<<grid_pairs, 256, 0, st>>>(probes, nq, nprobe, nlist, p.S, topk, g.keys, g.vals, part_idx);
-    ISE_LAUNCH_CHECK();
-    size_t sort_bytes = p.sort_tmp;
-    ISE_CUDA(cub::DeviceRadixSort::SortPairs(g.sort_tmp, sort_bytes, g.keys, g.keys_sorted, g.vals, g.pairs_sorted,
-                                             (int)p.npairs, 0, p.end_bit, st));
-    const int grid_lists = (int)std::min<int64_t>(ceil_div64(nlist + 1, 256), (int64_t)ctx->sm_count * 8);
-    ivf_list_items_kernel<<<grid_lists, 256, 0, st>>>(g.keys_sorted, p.npairs, list_off, nlist, p.S, g.qoff, g.items);
-    ISE_LAUNCH_CHECK();
-    size_t scan_bytes = p.scan_tmp;
-    ISE_CUDA(cub::DeviceScan::ExclusiveSum(g.scan_tmp, scan_bytes, g.items, g.item_off, (int)(nlist + 1), st));
-    return 0;
-}
-
-// persistent CTAs (as many as fit) that take work items from the counter: the item count stays on the device
-template <typename Kernel, typename... Args>
-static int launch_persistent(ise_ctx* ctx, cudaStream_t st, Kernel kernel, Args... args) {
-    int per_sm = 0;
-    ISE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, 0));
-    kernel<<<ctx->sm_count * std::max(per_sm, 1), kThreads, 0, st>>>(args...);
-    ISE_LAUNCH_CHECK();
-    return 0;
-}
-
 static bool vec_rows(const float* q, const float* xs, int d) {
     return (d % 4 == 0) && ((reinterpret_cast<uintptr_t>(q) | reinterpret_cast<uintptr_t>(xs)) & 15) == 0;
 }
@@ -507,8 +306,8 @@ static bool vec_rows(const float* q, const float* xs, int d) {
 
 ISE_EXPORT size_t ise_ivfflat_search_workspace_bytes(ise_ctx* ctx, int64_t nq, int nprobe, int64_t nlist,
                                                      int64_t max_list_len, int topk) {
-    if (!ctx || !plan_args_ok(nq, nprobe, nlist, max_list_len, topk)) return 0;
-    const Plan p = search_plan(nq, nprobe, nlist, max_list_len, topk);
+    if (!ctx || !ivf::plan_args_ok(nq, nprobe, nlist, max_list_len, topk)) return 0;
+    const ivf::Plan p = ivf::search_plan(nq, nprobe, nlist, max_list_len, topk, kCB, kQB);
     return p.grouping + p.parts + p.level;
 }
 
@@ -517,6 +316,7 @@ ISE_EXPORT int ise_ivfflat_search(ise_ctx* ctx, const float* q, int64_t nq, int 
                                   int64_t max_list_len, const int64_t* probes, int nprobe, int metric, int topk,
                                   float* out_val, int64_t* out_idx, void* workspace, size_t workspace_bytes,
                                   void* stream) {
+    using namespace ivf;
     ISE_CHECK_ARG(ctx != nullptr);
     ISE_CHECK_ARG(metric == ISE_METRIC_IP || metric == ISE_METRIC_L2);
     ISE_CHECK_ARG(nq >= 0 && d > 0 && topk >= 1 && topk <= 128);
@@ -528,14 +328,14 @@ ISE_EXPORT int ise_ivfflat_search(ise_ctx* ctx, const float* q, int64_t nq, int 
     if (workspace_bytes < need) ISE_FAIL("workspace too small: need " + std::to_string(need));
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
-    const Plan p = search_plan(nq, nprobe, nlist, max_list_len, topk);
+    const Plan p = search_plan(nq, nprobe, nlist, max_list_len, topk, kCB, kQB);
 
     uint8_t* w = reinterpret_cast<uint8_t*>(workspace);
     const Grouping gr = carve_grouping(w, p);
     const size_t entries = (size_t)p.g * nq * topk;
     float* part_val = reinterpret_cast<float*>(take(w, align256(entries * sizeof(float))));
     int64_t* part_idx = reinterpret_cast<int64_t*>(take(w, align256(entries * sizeof(int64_t))));
-    const size_t lv = p.g > kMergeFanIn ? (size_t)ceil_div64(p.g, kMergeFanIn) * nq * topk : 0;
+    const size_t lv = level_entries(p, nq, topk);
     float* lvl_val = reinterpret_cast<float*>(take(w, align256(lv * sizeof(float))));
     int64_t* lvl_idx = reinterpret_cast<int64_t*>(take(w, align256(lv * sizeof(int64_t))));
 
@@ -558,61 +358,27 @@ ISE_EXPORT int ise_ivfflat_search(ise_ctx* ctx, const float* q, int64_t nq, int 
     if (rc) return rc;
 
     // 3. merge the nprobe * S partial lists of every query, at most kMergeFanIn at a time
-    float* src_val = part_val;
-    int64_t* src_idx = part_idx;
-    float* dst_val = lvl_val;
-    int64_t* dst_idx = lvl_idx;
-    int64_t g = p.g;
-    const size_t list_stride = (size_t)nq * topk;
-    while (g > kMergeFanIn) {
-        const int64_t g2 = ceil_div64(g, kMergeFanIn);
-        for (int64_t j = 0; j < g2; ++j) {
-            const int n = (int)std::min<int64_t>(kMergeFanIn, g - j * kMergeFanIn);
-            const size_t in = (size_t)j * kMergeFanIn * list_stride, out = (size_t)j * list_stride;
-            rc = ise_topk_merge(ctx, src_val + in, src_idx + in, n, nq, topk, metric, dst_val + out, dst_idx + out, stream);
-            if (rc) return rc;
-        }
-        std::swap(src_val, dst_val);
-        std::swap(src_idx, dst_idx);
-        g = g2;
-    }
-    return ise_topk_merge(ctx, src_val, src_idx, (int)g, nq, topk, metric, out_val, out_idx, stream);
+    return merge_levels(ctx, p, nq, topk, metric, part_val, part_idx, lvl_val, lvl_idx, out_val, out_idx, stream);
 }
 
 ISE_EXPORT size_t ise_ivfflat_range_workspace_bytes(ise_ctx* ctx, int64_t nq, int nprobe, int64_t nlist,
                                                     int64_t max_list_len) {
-    if (!ctx || !plan_args_ok(nq, nprobe, nlist, max_list_len, 1)) return 0;
-    const Plan p = range_plan(ctx, nq, nprobe, nlist, max_list_len);
-    return p.grouping + 2 * p.seg + p.lims_tmp;
+    if (!ctx || !ivf::plan_args_ok(nq, nprobe, nlist, max_list_len, 1)) return 0;
+    return ivf::range_workspace(ivf::range_plan(ctx, nq, nprobe, nlist, max_list_len, kCB, kQB));
 }
-
-int ise_internal_range_offsets(const int64_t* cnt, int64_t rows, int64_t per_row, int64_t base,
-                               int64_t* offs, int64_t* lims, void* tmp, size_t tmp_bytes, void* stream);   // range.cu
 
 namespace {
 
-struct RangeWork {
-    Plan p;
-    Grouping gr;
-    int64_t *cnt, *offs;   // per (pair, chunk) segment: hits, output offset (offs[segs] = total)
-    void* lims_tmp;
-};
-
 static int range_setup(ise_ctx* ctx, const float* q, int64_t nq, int d, const float* xs_sorted,
                        const int64_t* ids_sorted, const int64_t* list_off, int64_t nlist, int64_t max_list_len,
-                       int nprobe, int metric, void* workspace, size_t workspace_bytes, RangeWork* rw) {
-    ISE_CHECK_ARG(plan_args_ok(nq, nprobe, nlist, max_list_len, 1));
+                       int nprobe, int metric, void* workspace, size_t workspace_bytes, ivf::RangeWork* rw) {
+    ISE_CHECK_ARG(ivf::plan_args_ok(nq, nprobe, nlist, max_list_len, 1));
     ISE_CHECK_ARG(metric == ISE_METRIC_IP || metric == ISE_METRIC_L2);
     ISE_CHECK_ARG(d > 0 && q && list_off && workspace);
     ISE_CHECK_ARG(max_list_len == 0 || (xs_sorted && ids_sorted));
     const size_t need = ise_ivfflat_range_workspace_bytes(ctx, nq, nprobe, nlist, max_list_len);
     if (workspace_bytes < need) ISE_FAIL("workspace too small: need " + std::to_string(need));
-    rw->p = range_plan(ctx, nq, nprobe, nlist, max_list_len);
-    uint8_t* w = reinterpret_cast<uint8_t*>(workspace);
-    rw->gr = carve_grouping(w, rw->p);
-    rw->cnt = reinterpret_cast<int64_t*>(take(w, rw->p.seg));
-    rw->offs = reinterpret_cast<int64_t*>(take(w, rw->p.seg));
-    rw->lims_tmp = take(w, rw->p.lims_tmp);
+    *rw = ivf::carve_range(workspace, ivf::range_plan(ctx, nq, nprobe, nlist, max_list_len, kCB, kQB));
     return 0;
 }
 
@@ -631,20 +397,20 @@ ISE_EXPORT int ise_ivfflat_range_count(ise_ctx* ctx, const float* q, int64_t nq,
         return 0;
     }
     ISE_CHECK_ARG(probes != nullptr);
-    RangeWork rw;
+    ivf::RangeWork rw;
     int rc = range_setup(ctx, q, nq, d, xs_sorted, ids_sorted, list_off, nlist, max_list_len, nprobe, metric,
                          workspace, workspace_bytes, &rw);
     if (rc) return rc;
-    const Plan& p = rw.p;
+    const ivf::Plan& p = rw.p;
     // segments no item writes (probe -1, chunk slots a list does not use) count 0; cnt[segs] = 0 ends the scan
     ISE_CUDA(cudaMemsetAsync(rw.cnt, 0, (size_t)(p.segs + 1) * sizeof(int64_t), st));
-    rc = group_pairs(ctx, p, rw.gr, probes, nq, nprobe, nlist, list_off, 0, nullptr, st);
+    rc = ivf::group_pairs(ctx, p, rw.gr, probes, nq, nprobe, nlist, list_off, 0, nullptr, st);
     if (rc) return rc;
     const bool vec = vec_rows(q, xs_sorted, d);
 #define ISE_COUNT_ARGS q, d, vec, xs_sorted, list_off, nlist, rw.gr.pairs_sorted, rw.gr.qoff, rw.gr.item_off, nprobe, \
                        p.S, radius, rw.gr.counter, rw.cnt
-    rc = metric == ISE_METRIC_L2 ? launch_persistent(ctx, st, ivfflat_range_count_kernel<true>, ISE_COUNT_ARGS)
-                                 : launch_persistent(ctx, st, ivfflat_range_count_kernel<false>, ISE_COUNT_ARGS);
+    rc = metric == ISE_METRIC_L2 ? ivf::launch_persistent(ctx, st, ivfflat_range_count_kernel<true>, ISE_COUNT_ARGS)
+                                 : ivf::launch_persistent(ctx, st, ivfflat_range_count_kernel<false>, ISE_COUNT_ARGS);
 #undef ISE_COUNT_ARGS
     if (rc) return rc;
     return ise_internal_range_offsets(rw.cnt, nq, p.g, 0, rw.offs, lims, rw.lims_tmp, p.lims_tmp, stream);
@@ -659,7 +425,7 @@ ISE_EXPORT int ise_ivfflat_range_fill(ise_ctx* ctx, const float* q, int64_t nq, 
     ISE_CHECK_ARG(out_dis && out_ids);
     DeviceGuard guard(ctx->device);
     cudaStream_t st = (cudaStream_t)stream;
-    RangeWork rw;
+    ivf::RangeWork rw;
     int rc = range_setup(ctx, q, nq, d, xs_sorted, ids_sorted, list_off, nlist, max_list_len, nprobe, metric,
                          workspace, workspace_bytes, &rw);
     if (rc) return rc;
@@ -667,8 +433,8 @@ ISE_EXPORT int ise_ivfflat_range_fill(ise_ctx* ctx, const float* q, int64_t nq, 
     const bool vec = vec_rows(q, xs_sorted, d);
 #define ISE_FILL_ARGS q, d, vec, xs_sorted, ids_sorted, list_off, nlist, rw.gr.pairs_sorted, rw.gr.qoff, \
                       rw.gr.item_off, nprobe, rw.p.S, radius, rw.gr.counter, rw.offs, out_dis, out_ids
-    rc = metric == ISE_METRIC_L2 ? launch_persistent(ctx, st, ivfflat_range_fill_kernel<true>, ISE_FILL_ARGS)
-                                 : launch_persistent(ctx, st, ivfflat_range_fill_kernel<false>, ISE_FILL_ARGS);
+    rc = metric == ISE_METRIC_L2 ? ivf::launch_persistent(ctx, st, ivfflat_range_fill_kernel<true>, ISE_FILL_ARGS)
+                                 : ivf::launch_persistent(ctx, st, ivfflat_range_fill_kernel<false>, ISE_FILL_ARGS);
 #undef ISE_FILL_ARGS
     return rc;
 }

@@ -371,7 +371,91 @@ class IndexIVFPQ:
                 f"ntotal={self.ntotal} (HBM resident)>")
 
 
-class IndexIVFFlat:
+class _InvertedLists:
+    """The list-sorted storage of the IVF indexes (IndexIVFFlat: FP32 vectors, IndexBinaryIVF: padded code rows): one
+    device copy of the rows grouped by list with their ids and list offsets; rows added since the last search are merged
+    into it lazily at the next search.  Subclasses set ``nlist`` and ``_lock`` and call ``_clear`` in __init__."""
+
+    def _clear(self) -> None:
+        self._rows = self._ids = self._off = None   # list-sorted rows, their ids, list offsets [nlist + 1] (device)
+        self._sizes = np.zeros(self.nlist, np.int64)   # host copy of the list sizes
+        self._pending = []                              # (rows, list numbers, ids) added since the last search
+        self._ntotal = 0
+
+    @property
+    def ntotal(self) -> int:
+        return self._ntotal
+
+    def _list_numbers(self, list_nos, n: int, device) -> torch.Tensor:
+        lists = torch.as_tensor(np.asarray(list_nos) if not isinstance(list_nos, torch.Tensor) else list_nos)
+        lists = lists.to(device=device, dtype=torch.int64).reshape(-1)
+        if lists.shape[0] != n:
+            raise AssertionError("add_preassigned: one list number per vector")
+        if lists.shape[0] and not (0 <= int(lists.min()) and int(lists.max()) < self.nlist):
+            raise AssertionError(f"add_preassigned: list numbers must lie in [0, {self.nlist})")
+        return lists
+
+    def _append(self, rows: torch.Tensor, lists: torch.Tensor) -> None:
+        """Appends device rows (ids ntotal + i) to the given lists, in order."""
+        sizes = torch.bincount(lists, minlength=self.nlist).cpu().numpy()
+        with self._lock:
+            ids = torch.arange(self._ntotal, self._ntotal + rows.shape[0], dtype=torch.int64, device=rows.device)
+            self._pending.append((rows.contiguous(), lists, ids))
+            self._sizes += sizes
+            self._ntotal += rows.shape[0]
+
+    def _lists(self):
+        """Merges the pending rows into the list-sorted storage (stable by list: ids keep ascending in every list)."""
+        with self._lock:
+            if self._pending:
+                first = self._pending[0][0]
+                dev = first.device
+                old = self._rows is not None
+                parts_l = [torch.repeat_interleave(torch.arange(self.nlist, device=dev), torch.diff(self._off))] if old else []
+                parts_l += [p[1] for p in self._pending]
+                order = torch.argsort(torch.cat(parts_l), stable=True)
+                dest = torch.empty_like(order)
+                dest[order] = torch.arange(order.shape[0], device=dev)
+                rows_all = torch.empty((self._ntotal,) + tuple(first.shape[1:]), dtype=first.dtype, device=dev)
+                ids = torch.empty((self._ntotal,), dtype=torch.int64, device=dev)
+                r0 = 0
+                for rows, row_ids in ([(self._rows, self._ids)] if old else []) + [(p[0], p[2]) for p in self._pending]:
+                    pos = dest[r0:r0 + rows.shape[0]]
+                    rows_all.index_copy_(0, pos, rows)
+                    ids.index_copy_(0, pos, row_ids)
+                    r0 += rows.shape[0]
+                off = np.zeros(self.nlist + 1, np.int64)
+                np.cumsum(self._sizes, out=off[1:])
+                self._rows, self._ids, self._off = rows_all, ids, torch.from_numpy(off).to(dev)
+                self._pending = []
+            return self._rows, self._ids, self._off
+
+    def _insertion_order(self):
+        """(rows, list numbers) in insertion order (ids 0 .. ntotal - 1), on the device: what pickling stores."""
+        rows, ids, off = self._lists()
+        xb = torch.empty_like(rows)
+        xb[ids] = rows
+        assign = torch.empty_like(ids)
+        assign[ids] = torch.repeat_interleave(torch.arange(self.nlist, device=ids.device), torch.diff(off))
+        return xb, assign
+
+    def reset(self) -> None:
+        with self._lock:
+            self._clear()
+
+    def get_list_size(self, list_no: int) -> int:
+        return int(self._sizes[int(list_no)])
+
+    def get_list_ids(self, list_no: int) -> np.ndarray:
+        """Ids stored in one list, in list order (InvertedLists::get_ids)."""
+        _, ids, off = self._lists() if self._ntotal else (None, None, None)
+        if ids is None:
+            return np.zeros(0, np.int64)
+        l = int(list_no)
+        return ids[int(off[l]):int(off[l + 1])].cpu().numpy()
+
+
+class IndexIVFFlat(_InvertedLists):
     """faiss.IndexIVFFlat (faiss/IndexIVFFlat.cpp, ~1.7.4): an inverted file whose lists hold the raw FP32 vectors, so
     a search scans only the ``nprobe`` probed lists yet returns exact FP32 distances.  ``range_search`` filters the
     same lists by a radius (``ise_ivfflat_range_count`` / ``_fill``) and returns its results in Faiss's probe order.
@@ -398,16 +482,6 @@ class IndexIVFFlat:
         self.is_trained = quantizer.ntotal == self.nlist
         self._lock = threading.RLock()
         self._clear()
-
-    def _clear(self) -> None:
-        self._xs = self._ids = self._off = None     # list-sorted vectors, their ids, list offsets [nlist + 1] (device)
-        self._sizes = np.zeros(self.nlist, np.int64)   # host copy of the list sizes
-        self._pending = []                              # (vectors, list numbers, ids) added since the last search
-        self._ntotal = 0
-
-    @property
-    def ntotal(self) -> int:
-        return self._ntotal
 
     def train(self, x) -> None:
         """Level1Quantizer::train_q1: k-means (niter 10, seed 1234, <= 256 points per centroid, spherical for inner
@@ -443,43 +517,7 @@ class IndexIVFFlat:
         xd = xd.to(torch.float32)
         if was_cuda and xd.data_ptr() == x.data_ptr():
             xd = xd.clone()
-        lists = torch.as_tensor(np.asarray(list_nos) if not isinstance(list_nos, torch.Tensor) else list_nos)
-        lists = lists.to(device=xd.device, dtype=torch.int64).reshape(-1)
-        if lists.shape[0] != xd.shape[0]:
-            raise AssertionError("add_preassigned: one list number per vector")
-        if lists.shape[0] and not (0 <= int(lists.min()) and int(lists.max()) < self.nlist):
-            raise AssertionError(f"add_preassigned: list numbers must lie in [0, {self.nlist})")
-        sizes = torch.bincount(lists, minlength=self.nlist).cpu().numpy()
-        with self._lock:
-            ids = torch.arange(self._ntotal, self._ntotal + xd.shape[0], dtype=torch.int64, device=xd.device)
-            self._pending.append((xd.contiguous(), lists, ids))
-            self._sizes += sizes
-            self._ntotal += xd.shape[0]
-
-    def _lists(self):
-        """Merges the pending rows into the list-sorted storage (stable by list: ids keep ascending in every list)."""
-        with self._lock:
-            if self._pending:
-                dev = self._pending[0][0].device
-                old = self._xs is not None
-                parts_l = [torch.repeat_interleave(torch.arange(self.nlist, device=dev), torch.diff(self._off))] if old else []
-                parts_l += [p[1] for p in self._pending]
-                order = torch.argsort(torch.cat(parts_l), stable=True)
-                dest = torch.empty_like(order)
-                dest[order] = torch.arange(order.shape[0], device=dev)
-                xs = torch.empty((self._ntotal, self.d), dtype=torch.float32, device=dev)
-                ids = torch.empty((self._ntotal,), dtype=torch.int64, device=dev)
-                r0 = 0
-                for rows, row_ids in ([(self._xs, self._ids)] if old else []) + [(p[0], p[2]) for p in self._pending]:
-                    pos = dest[r0:r0 + rows.shape[0]]
-                    xs.index_copy_(0, pos, rows)
-                    ids.index_copy_(0, pos, row_ids)
-                    r0 += rows.shape[0]
-                off = np.zeros(self.nlist + 1, np.int64)
-                np.cumsum(self._sizes, out=off[1:])
-                self._xs, self._ids, self._off = xs, ids, torch.from_numpy(off).to(dev)
-                self._pending = []
-            return self._xs, self._ids, self._off
+        self._append(xd, self._list_numbers(list_nos, xd.shape[0], xd.device))
 
     def search(self, x, k: int):
         """IndexIVF::search: probe min(nprobe, nlist) lists, exact FP32 scan (IVFFlatScanner: fvec_inner_product /
@@ -528,32 +566,13 @@ class IndexIVFFlat:
             return lims, D, I
         return lims.cpu().numpy().astype(np.uint64), D.cpu().numpy(), I.cpu().numpy()
 
-    def reset(self) -> None:
-        with self._lock:
-            self._clear()
-
-    def get_list_size(self, list_no: int) -> int:
-        return int(self._sizes[int(list_no)])
-
-    def get_list_ids(self, list_no: int) -> np.ndarray:
-        """Ids stored in one list, in list order (InvertedLists::get_ids)."""
-        _, ids, off = self._lists() if self._ntotal else (None, None, None)
-        if ids is None:
-            return np.zeros(0, np.int64)
-        l = int(list_no)
-        return ids[int(off[l]):int(off[l + 1])].cpu().numpy()
-
     # joblib / pickle: trained state, vectors and list numbers in insertion order (host arrays)
     def __getstate__(self):
         st = dict(d=self.d, nlist=self.nlist, metric_type=self.metric_type, nprobe=self.nprobe,
                   quantizer_metric=self.quantizer.metric_type, is_trained=self.is_trained,
                   coarse=self.quantizer.reconstruct_n(), xb=None, assign=None)
         if self._ntotal:
-            xs, ids, off = self._lists()
-            xb = torch.empty_like(xs)
-            xb[ids] = xs
-            assign = torch.empty_like(ids)
-            assign[ids] = torch.repeat_interleave(torch.arange(self.nlist, device=ids.device), torch.diff(off))
+            xb, assign = self._insertion_order()
             st["xb"], st["assign"] = xb.cpu().numpy(), assign.cpu().numpy()
         return st
 
@@ -699,13 +718,156 @@ class IndexBinaryFlat:
             self.add(st["codes"])
 
 
+class IndexBinaryIVF(_InvertedLists):
+    """faiss.IndexBinaryIVF (faiss/IndexBinaryIVF.cpp, ~1.7.4, recalled rather than checked against Faiss, like the rest
+    of the Faiss semantics here; tests/_binary_ivf_oracle.py): an inverted file of binary codes whose probed lists are
+    scanned by exact Hamming distance, for collections where IndexBinaryFlat's exhaustive scan is too slow.
+
+    ``quantizer`` is an IndexBinaryFlat of the same ``d`` (bits, a multiple of 8, at most 2048) holding the nlist list
+    codes.  ``train`` decodes a sample of the codes to +-1 floats, runs the L2 k-means of IndexIVFFlat (niter 10, seed
+    1234, <= 256 points per centroid) and thresholds the centroids back to bits.  A code goes to the quantizer's Hamming
+    top-1 (lowest list id on ties).  ``search`` probes ``min(nprobe, nlist)`` lists through the quantizer and returns
+    (D int32, I int64) in the canonical (distance, id) order over their codes (``ise_binary_ivf_search``); as in
+    IndexIVFFlat, this deliberately differs from Faiss's heap, which can keep a higher id from an earlier-probed list
+    when a tie falls on the k-th place.  ``range_search`` keeps every code of the same lists with distance < radius, in
+    Faiss's scan order: by probe rank, then by position in the list.  Codes live in HBM grouped by list, rows
+    zero-padded to a multiple of 16 bytes."""
+
+    def __init__(self, quantizer: IndexBinaryFlat, d: int, nlist: int):
+        d = int(d)
+        if d <= 0 or d % 8 != 0:
+            raise RuntimeError("Error: 'd % 8 == 0' failed")
+        if d // 8 > ops.BINARY_MAX_CODE_SIZE:
+            raise NotImplementedError(f"IndexBinaryIVF supports d <= {8 * ops.BINARY_MAX_CODE_SIZE} bits")
+        if quantizer.d != d:
+            raise RuntimeError(f"quantizer dimension {quantizer.d} differs from the index dimension {d}")
+        self.quantizer, self.d, self.code_size, self.nlist = quantizer, d, d // 8, int(nlist)
+        self.nprobe = 1
+        self.is_trained = quantizer.ntotal == self.nlist
+        self.verbose = False
+        self._lock = threading.RLock()
+        self._clear()
+
+    def train(self, x) -> None:
+        """IndexBinaryIVF::train: unless the quantizer already holds nlist codes, k-means (L2, niter 10, seed 1234) on the
+        codes decoded to +-1 floats, centroids thresholded back to bits (> 0 -> 1).  Only the <= 256 * nlist sampled
+        codes are decoded, the sample Kmeans would draw (rand_perm prefix), which gives the result of decoding all."""
+        a = _binary_rows(x, self.code_size, "train")
+        if self.quantizer.ntotal != self.nlist:
+            codes, _ = self.quantizer._device_rows(a)
+            n, nmax = codes.shape[0], self.nlist * ClusteringParameters().max_points_per_centroid
+            if n < self.nlist:
+                raise RuntimeError("Number of training points (%d) should be at least as large as number of "
+                                   "clusters (%d)" % (n, self.nlist))
+            if n > nmax:
+                perm = ops.rand_perm_prefix(n, 1234, nmax)
+                codes = codes.index_select(0, torch.from_numpy(perm).to(codes.device))
+            km = Kmeans(self.d, self.nlist, niter=10, seed=1234)
+            km.train(ops.binary_to_real(codes, self.code_size))
+            self.quantizer.reset()
+            self.quantizer.add(ops.real_to_binary(km.index._database().contiguous(), self.code_size))
+        self.is_trained = True
+
+    def _assign(self, rows: torch.Tensor) -> torch.Tensor:
+        """Quantizer Hamming top-1 of padded device rows (lowest list id on ties)."""
+        return ops.binary_knn(rows, self.quantizer._database(), self.code_size, 1)[1].reshape(-1)
+
+    def add(self, x) -> None:
+        """IndexBinaryIVF::add_with_ids(n, x, nullptr): ids ntotal + i, list = the quantizer's top-1."""
+        if not self.is_trained:
+            raise RuntimeError("Error: 'is_trained' failed")
+        rows, _ = self.quantizer._device_rows(_binary_rows(x, self.code_size, "add"))
+        self._append(rows, self._assign(rows))
+
+    def add_preassigned(self, x, list_nos) -> None:
+        """IndexBinaryIVF::add_core with precomputed_idx: appends x (ids ntotal + i) to the given lists, in order."""
+        if not self.is_trained:
+            raise RuntimeError("Error: 'is_trained' failed")
+        rows, _ = self.quantizer._device_rows(_binary_rows(x, self.code_size, "add"))
+        self._append(rows, self._list_numbers(list_nos, rows.shape[0], rows.device))
+
+    def _probes(self, q: torch.Tensor) -> torch.Tensor:
+        nprobe = min(self.nprobe, self.nlist)
+        return ops.binary_knn(q, self.quantizer._database(), self.code_size, nprobe)[1]
+
+    def _check_nprobe(self) -> None:
+        if min(self.nprobe, self.nlist) > ops.MAX_TOPK:
+            raise NotImplementedError(f"IndexBinaryIVF probes at most {ops.MAX_TOPK} lists")
+
+    def search(self, x, k: int):
+        """IndexBinaryIVF::search: the k nearest codes of the min(nprobe, nlist) probed lists, (D int32 [nq, k], I int64
+        [nq, k]) in the canonical (distance, id) order; fewer than k results leave id -1 / 2^31 - 1.  1 <= k <= 128."""
+        k = int(k)
+        if k <= 0:
+            raise AssertionError("k must be positive")
+        if k > ops.MAX_TOPK:
+            raise NotImplementedError(f"IndexBinaryIVF.search supports k <= {ops.MAX_TOPK}")
+        a = _binary_rows(x, self.code_size, "search")
+        self._check_nprobe()
+        q, was_cuda = self.quantizer._device_rows(a)
+        nq = q.shape[0]
+        if nq and self._ntotal and self.is_trained:
+            codes, ids, off = self._lists()
+            D, I = ops.binary_ivf_search(q, codes, ids, off, int(self._sizes.max()), self._probes(q), self.code_size, k)
+        else:
+            D = torch.full((nq, k), 2**31 - 1, dtype=torch.int32, device=q.device)
+            I = torch.full((nq, k), -1, dtype=torch.int64, device=q.device)
+        if was_cuda:
+            return D, I
+        return D.cpu().numpy(), I.cpu().numpy()
+
+    def range_search(self, x, radius: int):
+        """IndexBinaryIVF::range_search: every code of the probed lists with Hamming distance < radius (strict), with the
+        distances ``search`` returns.  Returns (lims [nq + 1], D int32, I int64); the results of query i are
+        D[lims[i]:lims[i+1]] / I[...] by probe rank, then by position in the list (ids ascend inside a list).  NumPy
+        input gives NumPy output (lims uint64); CUDA tensors give CUDA tensors (lims int64)."""
+        radius = operator.index(radius)
+        a = _binary_rows(x, self.code_size, "range_search")
+        self._check_nprobe()
+        q, was_cuda = self.quantizer._device_rows(a)
+        nq = q.shape[0]
+        if nq and self._ntotal and self.is_trained:
+            codes, ids, off = self._lists()
+            lims, D, I = ops.binary_ivf_range_search(q, codes, ids, off, int(self._sizes.max()), self._probes(q),
+                                                     self.code_size, radius)
+        else:
+            lims, D, I = ops.range_empty(nq, q.device)
+            D = D.to(torch.int32)
+        if was_cuda:
+            return lims, D, I
+        return lims.cpu().numpy().astype(np.uint64), D.cpu().numpy(), I.cpu().numpy()
+
+    # joblib / pickle: quantizer codes, nprobe, codes and list numbers in insertion order (host arrays)
+    def __getstate__(self):
+        st = dict(d=self.d, nlist=self.nlist, nprobe=self.nprobe, is_trained=self.is_trained,
+                  coarse=self.quantizer.__getstate__()["codes"], codes=None, assign=None)
+        if self._ntotal:
+            rows, assign = self._insertion_order()
+            st["codes"], st["assign"] = rows[:, :self.code_size].cpu().numpy(), assign.cpu().numpy()
+        return st
+
+    def __setstate__(self, st):
+        quantizer = IndexBinaryFlat(st["d"])
+        if st["coarse"].shape[0]:
+            quantizer.add(st["coarse"])
+        self.__init__(quantizer, st["d"], st["nlist"])
+        self.nprobe, self.is_trained = st["nprobe"], st["is_trained"]
+        if st["codes"] is not None:
+            self.add_preassigned(st["codes"], st["assign"])
+
+    def __repr__(self):
+        return (f"<image_search_engine_b200.IndexBinaryIVF d={self.d} nlist={self.nlist} nprobe={self.nprobe} "
+                f"ntotal={self.ntotal} (HBM resident)>")
+
+
 # ------------------------------------------------------------------------------------------
 # flat index file format (faiss/impl/index_write.cpp), so existing models/*.faiss files open
 # ------------------------------------------------------------------------------------------
 def write_index(index: IndexFlat, fname) -> None:
-    if isinstance(index, IndexBinaryFlat):
-        raise NotImplementedError("Faiss writes binary indexes with write_index_binary (IBxF), which is not provided; "
-                                  "an IndexBinaryFlat can be pickled")
+    if isinstance(index, (IndexBinaryFlat, IndexBinaryIVF)):
+        name = type(index).__name__
+        raise NotImplementedError("Faiss writes binary indexes with write_index_binary (IBxF / IBwF), which is not "
+                                  f"provided; an {name} can be pickled")
     if isinstance(index, (IndexIVFPQ, IndexIVFFlat)):
         name = type(index).__name__
         raise NotImplementedError(f"only flat indexes are written in Faiss's file format; an {name} can be pickled")

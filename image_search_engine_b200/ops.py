@@ -1034,6 +1034,115 @@ def binary_range_search(q: torch.Tensor, codes: torch.Tensor, code_size: int, ra
 
 
 # ------------------------------------------------------------------------------------------
+# binary IVF (IndexBinaryIVF)
+# ------------------------------------------------------------------------------------------
+def _binary_ivf_args(q: torch.Tensor, codes: torch.Tensor, ids: torch.Tensor, list_off: torch.Tensor,
+                     probes: torch.Tensor, code_size: int):
+    pitch = _binary_args(q, codes, code_size)
+    if ids.dtype != torch.int64 or list_off.dtype != torch.int64 or probes.dtype != torch.int64:
+        raise IseError("binary IVF search: ids, list offsets and probes are int64")
+    if probes.dim() != 2 or probes.shape[0] != q.shape[0] or ids.shape[0] != codes.shape[0]:
+        raise IseError("binary IVF search: inconsistent shapes")
+    return pitch, probes.contiguous(), list_off.contiguous(), ids.contiguous()
+
+
+def binary_ivf_search_workspace_bytes(nq: int, nprobe: int, nlist: int, max_list_len: int, code_size: int,
+                                      topk: int) -> int:
+    """Device scratch of one binary_ivf_search call (the bound is in include/ise.h)."""
+    return int(_lib.load().ise_binary_ivf_search_workspace_bytes(_lib.ctx(torch.cuda.current_device()), int(nq),
+                                                                   int(nprobe), int(nlist), int(max_list_len),
+                                                                   int(code_size), int(topk)))
+
+
+def binary_ivf_search(q: torch.Tensor, codes: torch.Tensor, ids: torch.Tensor, list_off: torch.Tensor,
+                      max_list_len: int, probes: torch.Tensor, code_size: int, topk: int):
+    """Exact Hamming top-k of every query over the codes of its probed lists (IndexBinaryIVF.search): q [nq, pitch] and
+    codes [ntotal, pitch] uint8 as binary_knn's, codes / ids grouped by list (list l = rows list_off[l] ..
+    list_off[l + 1], ids ascending inside a list), probes [nq, nprobe] int64.  Returns (D int32, I int64) [nq, topk]
+    sorted by (distance, id); padding is id -1 / 2^31 - 1."""
+    pitch, probes, list_off, ids = _binary_ivf_args(q, codes, ids, list_off, probes, code_size)
+    if not 1 <= topk <= MAX_TOPK:
+        raise IseError(f"topk must be in [1, {MAX_TOPK}]")
+    nq, nprobe, nlist = q.shape[0], probes.shape[1], list_off.shape[0] - 1
+    D = torch.empty((nq, topk), dtype=torch.int32, device=q.device)
+    I = torch.empty((nq, topk), dtype=torch.int64, device=q.device)
+    if nq == 0:
+        return D, I
+    lib, ctx = _lib.load(), _lib.ctx(_dev(q))
+    ws_bytes = lib.ise_binary_ivf_search_workspace_bytes(ctx, nq, nprobe, nlist, int(max_list_len), int(code_size),
+                                                         int(topk))
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=q.device)
+    _lib.check(lib.ise_binary_ivf_search(ctx, _ptr(q), nq, _ptr(codes), _ptr(ids), _ptr(list_off), nlist,
+                                         int(max_list_len), int(code_size), pitch, _ptr(probes), nprobe, int(topk),
+                                         _ptr(D), _ptr(I), _ptr(ws), ws_bytes, _stream()))
+    _count(7)                                 # probe keys, sort, list items, scan, scan kernel, merge, distances
+    return D, I
+
+
+def binary_ivf_range_workspace_bytes(nq: int, nprobe: int, nlist: int, max_list_len: int, code_size: int) -> int:
+    """Device scratch of one binary_ivf_range_search call (the bound is in include/ise.h)."""
+    return int(_lib.load().ise_binary_ivf_range_workspace_bytes(_lib.ctx(torch.cuda.current_device()), int(nq),
+                                                                  int(nprobe), int(nlist), int(max_list_len),
+                                                                  int(code_size)))
+
+
+def binary_ivf_range_search(q: torch.Tensor, codes: torch.Tensor, ids: torch.Tensor, list_off: torch.Tensor,
+                            max_list_len: int, probes: torch.Tensor, code_size: int, radius: int):
+    """Every code of a query's probed lists within Hamming distance < radius (IndexBinaryIVF.range_search).  Inputs as
+    binary_ivf_search.  Returns (lims int64 [nq + 1], D int32, I int64) on the device; the results of query i are
+    D / I[lims[i]:lims[i+1]] by probe rank, then list position (Faiss's order).  One readback: the total, lims[nq]."""
+    pitch, probes, list_off, ids = _binary_ivf_args(q, codes, ids, list_off, probes, code_size)
+    nq, nprobe, nlist = q.shape[0], probes.shape[1], list_off.shape[0] - 1
+    if nq == 0:
+        lims, D, I = range_empty(0, q.device)
+        return lims, D.to(torch.int32), I
+    radius = min(max(int(radius), 0), 1 << 30)           # every distance is in [0, 2048]: the result is the same
+    lib, ctx = _lib.load(), _lib.ctx(_dev(q))
+    ws_bytes = lib.ise_binary_ivf_range_workspace_bytes(ctx, nq, nprobe, nlist, int(max_list_len), int(code_size))
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=q.device)
+    lims = torch.empty((nq + 1,), dtype=torch.int64, device=q.device)
+    _lib.check(lib.ise_binary_ivf_range_count(ctx, _ptr(q), nq, _ptr(codes), _ptr(ids), _ptr(list_off), nlist,
+                                              int(max_list_len), int(code_size), pitch, _ptr(probes), nprobe, radius,
+                                              _ptr(lims), _ptr(ws), ws_bytes, _stream()))
+    total = int(lims[nq].item())                          # the one readback: sizes D / I
+    D = torch.empty((total,), dtype=torch.int32, device=q.device)
+    I = torch.empty((total,), dtype=torch.int64, device=q.device)
+    if total:
+        _lib.check(lib.ise_binary_ivf_range_fill(ctx, _ptr(q), nq, _ptr(codes), _ptr(ids), _ptr(list_off), nlist,
+                                                 int(max_list_len), int(code_size), pitch, nprobe, radius, _ptr(D),
+                                                 _ptr(I), _ptr(ws), ws_bytes, _stream()))
+    _count(9 if total else 8)
+    return lims, D, I
+
+
+def binary_to_real(codes: torch.Tensor, code_size: int) -> torch.Tensor:
+    """uint8 rows [n, >= code_size] -> float32 [n, 8 * code_size]: bit j of byte i (LSB first) -> coordinate 8 i + j,
+    1 -> +1, 0 -> -1 (IndexBinaryIVF::train's decoding)."""
+    if codes.dtype != torch.uint8 or codes.dim() != 2 or codes.stride(1) != 1 or codes.shape[1] < code_size:
+        raise IseError("binary_to_real needs uint8 rows of at least code_size bytes")
+    n = codes.shape[0]
+    out = torch.empty((n, 8 * int(code_size)), dtype=torch.float32, device=codes.device)
+    if n:
+        _lib.check(_lib.load().ise_binary_to_real(_lib.ctx(_dev(codes)), _ptr(codes), n, int(code_size),
+                                                  codes.stride(0), _ptr(out), _stream()))
+        _count()
+    return out
+
+
+def real_to_binary(x: torch.Tensor, code_size: int) -> torch.Tensor:
+    """float32 [n, 8 * code_size] -> uint8 rows [n, code_size]: bit = 1 iff the coordinate is > 0."""
+    if x.dtype != torch.float32 or x.dim() != 2 or not x.is_contiguous() or x.shape[1] != 8 * int(code_size):
+        raise IseError("real_to_binary needs contiguous float32 rows of 8 * code_size")
+    n = x.shape[0]
+    out = torch.empty((n, int(code_size)), dtype=torch.uint8, device=x.device)
+    if n:
+        _lib.check(_lib.load().ise_real_to_binary(_lib.ctx(_dev(x)), _ptr(x), n, int(code_size), int(code_size),
+                                                  _ptr(out), _stream()))
+        _count()
+    return out
+
+
+# ------------------------------------------------------------------------------------------
 # k-means update
 # ------------------------------------------------------------------------------------------
 def kmeans_accumulate(x: torch.Tensor, assign: torch.Tensor, dis: torch.Tensor | None, sums: torch.Tensor,

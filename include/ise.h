@@ -466,6 +466,55 @@ int ise_binary_range_fill(ise_ctx* ctx, const uint8_t* q, int64_t nq, const uint
                           int code_size, int64_t pitch, int radius, int32_t* out_dis, int64_t* out_ids,
                           void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- binary IVF index (faiss/IndexBinaryIVF.cpp) ----------------------------------------------------------------
+ * Exact Hamming distances over the codes of the probed inverted lists; no [nq, ntotal] matrix and no host
+ * synchronisation.  q[nq] uint8 rows of `pitch` bytes (as ise_binary_knn, zero past code_size, 16-byte aligned);
+ * codes_sorted[ntotal] the codes grouped by list with the same pitch, list l = rows list_off[l] .. list_off[l + 1]
+ * (list_off: int64[nlist + 1]) with ids ids_sorted[] ascending inside every list; max_list_len = the longest list (host
+ * value, sizes the workspace, < 2^31); probes[nq, nprobe] int64 list ids (-1 = none).  The (query, probe) pairs are
+ * grouped by list as in ise_ivfflat_search; a work item scans a chunk of a list for 4, 32 or 128 of its queries (32, 4
+ * or 1 threads each), chosen from the average number of queries per probed list, nq * nprobe / nlist.
+ *
+ * ise_binary_ivf_search: out_dis[nq, topk] int32 and out_idx[nq, topk] int64 sorted by (distance, id) over the scanned
+ * codes (among equal distances the lowest ids win), padded with id -1 / 2^31 - 1.  1 <= topk <= 128, nq * nprobe <
+ * 2^31.  Workspace (ise_binary_ivf_search_workspace_bytes) is O(nq * nprobe * topk + nlist): 12 bytes per
+ * partial-list entry, at most max(2^24, nq nprobe topk) entries, plus 1/256 of that for the merge levels, 4 bytes per
+ * output entry, 16 bytes per (query, probe) pair and 24 per list for the grouping, and CUB's sort / scan scratch. */
+size_t ise_binary_ivf_search_workspace_bytes(ise_ctx* ctx, int64_t nq, int nprobe, int64_t nlist, int64_t max_list_len,
+                                             int code_size, int topk);
+int ise_binary_ivf_search(ise_ctx* ctx, const uint8_t* q, int64_t nq, const uint8_t* codes_sorted,
+                          const int64_t* ids_sorted, const int64_t* list_off, int64_t nlist, int64_t max_list_len,
+                          int code_size, int64_t pitch, const int64_t* probes, int nprobe, int topk, int32_t* out_dis,
+                          int64_t* out_idx, void* workspace, size_t workspace_bytes, void* stream);
+/* Range search (faiss/IndexIVF.cpp range_search_preassigned, scan_codes_range): every code of a probed list with
+ * distance < radius (strict), with the distances ise_binary_ivf_search returns.  Results of query i are
+ * out[lims[i] .. lims[i + 1]) by probe rank (probes[i, 0] first; -1 skipped), then by position in the list.  Two calls
+ * on the same stream with the same arguments and the same workspace, untouched in between:
+ *   ise_binary_ivf_range_count  groups the pairs, counts the hits of every (pair, chunk) segment, scans them into int64
+ *                               offsets and writes lims[nq + 1] (lims[0] = 0 for nq == 0);
+ *   ise_binary_ivf_range_fill   re-scans the work items that have hits and writes out_dis / out_ids[lims[nq]].
+ * The caller reads lims[nq] to size the outputs.  Workspace (ise_binary_ivf_range_workspace_bytes) is
+ * O(nq * nprobe * S + nlist): 16 bytes per (pair, chunk) segment, at most max(2^22, nq * nprobe) segments, the offsets
+ * scan's scratch (ise_range_lims_workspace_bytes), and the grouping as for the search. */
+size_t ise_binary_ivf_range_workspace_bytes(ise_ctx* ctx, int64_t nq, int nprobe, int64_t nlist, int64_t max_list_len,
+                                            int code_size);
+int ise_binary_ivf_range_count(ise_ctx* ctx, const uint8_t* q, int64_t nq, const uint8_t* codes_sorted,
+                               const int64_t* ids_sorted, const int64_t* list_off, int64_t nlist, int64_t max_list_len,
+                               int code_size, int64_t pitch, const int64_t* probes, int nprobe, int radius,
+                               int64_t* lims, void* workspace, size_t workspace_bytes, void* stream);
+int ise_binary_ivf_range_fill(ise_ctx* ctx, const uint8_t* q, int64_t nq, const uint8_t* codes_sorted,
+                              const int64_t* ids_sorted, const int64_t* list_off, int64_t nlist, int64_t max_list_len,
+                              int code_size, int64_t pitch, int nprobe, int radius, int32_t* out_dis, int64_t* out_ids,
+                              void* workspace, size_t workspace_bytes, void* stream);
+/* IndexBinaryIVF::train's conversions, no workspace.  ise_binary_to_real: out[n, 8 * code_size] float32, coordinate
+ * 8 i + j = +1 if bit j (LSB first) of byte i of the row is set, else -1; rows of codes are `pitch` bytes apart.
+ * ise_real_to_binary: codes[n, pitch], bit j of byte i = (x[8 i + j] > 0) (an exact 0 gives 0), zero bytes past
+ * code_size; x rows are 8 * code_size floats. */
+int ise_binary_to_real(ise_ctx* ctx, const uint8_t* codes, int64_t n, int code_size, int64_t pitch, float* out,
+                       void* stream);
+int ise_real_to_binary(ise_ctx* ctx, const float* x, int64_t n, int code_size, int64_t pitch, uint8_t* codes,
+                       void* stream);
+
 /* ---- collectives for a single-process multi-GPU host (NCCL over NVLink, resolved with dlopen at run time) ----------
  * The two exchange steps of the sharded path (SURVEY section 8e): the per-iteration all-reduce of the k-means
  * [k*d sums | k counts] buffer and the all-gather of per-shard top-k lists before ise_topk_merge.  The Python host
