@@ -95,7 +95,8 @@ PROTOTYPES = {
     "ise_kmeans_mean": (_int, [_c_void_p, _c_void_p, _c_void_p, _i64, _int, _c_void_p, _c_void_p, _c_void_p]),
     "ise_kmeans_apply_splits": (_int, [_c_void_p, _c_void_p, _i64, _int, _c_void_p, C.c_int32, _c_void_p]),
     "ise_bovw_histogram": (_int, [_c_void_p, _c_void_p, _i64, _c_void_p, _i64, _int, _int, _int, _c_void_p, _int,
-                                  _f64, _f64, _f64, _f64, _c_void_p]),
+                                  _f64, _f64, _f64, _f64, _int, _c_void_p]),
+    "ise_clear": (_int, [_c_void_p, _c_void_p, _size, _f64, _c_void_p]),
     "ise_bovw_histogram_csr": (_int, [_c_void_p, _c_void_p, _c_void_p, _i64, _int, _int, _int, _c_void_p, _c_void_p,
                                       _c_void_p, _c_void_p, _int, _f64, _f64, _f64, _f64, _c_void_p]),
     "ise_scores_topk_workspace_bytes": (_size, [_c_void_p, _i64, _i64, _int]),

@@ -30,6 +30,11 @@ from .kmeans_faiss import FaissKMeans
 from .utils import OkapiTransformer, create_search_index
 
 _HIST_MODES = {"numpy_compat": HIST_NUMPY_COMPAT, "bincount": HIST_BINCOUNT}
+# Rate of the clear that runs beside the assign in histograms_device.  Any HBM stream beside the assign slows it: on a
+# B200 (1000 W) at C2, 328 MB written unpaced cost the assign ~40-49 us and paced to 1-2 TB/s ~17-22 us (measured,
+# profiles/microbench_hist_zeroed.py has the step-level A/B).  At 2 TB/s the clear lasts ~170 us, under a fifth of the
+# C2 assign (100 descriptors of d = 128 per image).
+_CLEAR_GB_PER_S = 2000.0
 
 
 def describe_dataset(describer, X, prediction=False):
@@ -280,7 +285,8 @@ class BOVW(BaseEstimator):
         # copy first: on Python >= 3.11 BaseEstimator.__getstate__ hands back the LIVE __dict__, and popping from it
         # would drop the caches of the estimator being pickled
         state = dict(super().__getstate__())
-        for key in ("_pipe_cache", "_csr_cache", "_csr_bufs", "_pipe_lock", "_pack_bufs", "_last_transfer"):   # CUDA streams / events / staging buffers / locks are not persisted
+        for key in ("_pipe_cache", "_csr_cache", "_csr_bufs", "_pipe_lock", "_pack_bufs", "_last_transfer",
+                    "_clear_streams"):   # CUDA streams / events / staging buffers / locks are not persisted
             state.pop(key, None)
         return state
 
@@ -622,20 +628,36 @@ class BOVW(BaseEstimator):
 
     def histograms_device(self, descriptions, *, okapi: OkapiTransformer | None = None,
                           out_dtype=torch.float64) -> torch.Tensor:
-        """One assign launch + one histogram launch for all images; optional fused Okapi weighting."""
+        """One assign launch + one histogram launch for all images; optional fused Okapi weighting.  The result matrix
+        is cleared on a side stream while the assign runs, and the histogram then writes only the non-zero bins."""
         if self.hist_mode not in _HIST_MODES:
             raise ValueError(f"hist_mode must be one of {sorted(_HIST_MODES)}")
         dev = ops.require_cuda()
         mat, offsets = pack_descriptions(descriptions)
         xd = mat.to(dev, non_blocking=True) if isinstance(mat, torch.Tensor) else \
             torch.from_numpy(mat).to(dev, non_blocking=True)
-        off = torch.from_numpy(offsets).to(dev, non_blocking=True)
+        off = torch.empty((len(offsets),), dtype=torch.int64, device=dev)
+        out = torch.empty((len(offsets) - 1, int(self.n_clusters)), dtype=out_dtype, device=dev)
+        main = torch.cuda.current_stream()
+        allocated = main.record_event()
+        side = self.__dict__.setdefault("_clear_streams", {}).get(dev.index)
+        if side is None:
+            side = self.__dict__["_clear_streams"].setdefault(dev.index, torch.cuda.Stream(device=dev))
+        # the assign is enqueued first; the clear's blocks fit beside its CTAs on every SM (csrc/bovw.cu, clear_kernel).
+        # Only the histogram reads the offsets, so their upload goes to the side stream too, off the assign's path.
         words = self.clusterer.transform_device(xd)
+        side.wait_event(allocated)
+        with torch.cuda.stream(side):
+            off.copy_(torch.from_numpy(offsets), non_blocking=True)
+            ops.clear_(out, _CLEAR_GB_PER_S)
+        # the current stream waits for the side stream before `off` / `out` are used, returned or freed: the caching
+        # allocator only orders them on the current stream
+        main.wait_stream(side)
         kw = {}
         if okapi is not None:
             kw = dict(okapi=True, k1=okapi.k1, k2=okapi.k2, b=okapi.b)
         return ops.bovw_histogram(words, off, int(self.n_clusters), mode=_HIST_MODES[self.hist_mode],
-                                  out_dtype=out_dtype, **kw)
+                                  out_dtype=out_dtype, out=out, zeroed=True, **kw)
 
     def fit_transform(self, X, y=None):
         self.fit(X)

@@ -62,10 +62,43 @@ __device__ __forceinline__ void store4(double* p, double a, double b, double c, 
     reinterpret_cast<double2*>(p)[1] = make_double2(c, d);
 }
 
+// Zero fill sized to run BESIDE the verified assign (one 512-thread CTA per SM, 95 registers, 205.8 KB of shared
+// memory): 128 threads, no shared memory and at most 32 registers per thread (the 16 of __launch_bounds__ cap them),
+// so its blocks fit in what the assign's CTA leaves of an SM.  ise_clear gives it the max-shared carveout: with the
+// default, an SM that holds clear blocks is configured for little shared memory and cannot take the assign's CTA
+// until they drain (measured on a B200: the two kernels then ran one after the other).  The assign also slows under
+// a concurrent full-rate HBM stream, so ns_per_sweep > 0 paces the stores against %globaltimer: each thread stores
+// 16 bytes per sweep and starts sweep s no earlier than s * ns_per_sweep after it began.  Evict-first stores: the
+// cleared rows are not read again before the histogram's scattered writes.
+constexpr int kClearThreads = 128;
+
+__device__ __forceinline__ uint64_t global_ns() {
+    uint64_t t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+
+__global__ void __launch_bounds__(kClearThreads, 16)
+clear_kernel(uint4* __restrict__ p, int64_t n16, unsigned char* __restrict__ tail, int tail_bytes,
+             unsigned ns_per_sweep) {
+    const int64_t stride = (int64_t)gridDim.x * kClearThreads;
+    const uint64_t t0 = ns_per_sweep ? global_ns() : 0;
+    uint64_t due = t0;
+    for (int64_t i = (int64_t)blockIdx.x * kClearThreads + threadIdx.x; i < n16; i += stride) {
+        __stcs(p + i, make_uint4(0u, 0u, 0u, 0u));
+        if (ns_per_sweep) {
+            due += ns_per_sweep;
+            while (global_ns() < due) __nanosleep(64);
+        }
+    }
+    if (blockIdx.x == 0 && threadIdx.x < tail_bytes) tail[threadIdx.x] = 0;
+}
+
 // One CTA walks images (grid-stride).  Per image: the ids are read ONCE into registers (up to WPT per thread;
 // longer images re-read the tail from L2), min/max for the numpy-compat edges (32-bit redux), shared-memory atomic
 // counts, then the row is written with 128-bit stores while the counters are cleared in the same sweep (no
-// separate zeroing phase); the NEXT image's ids are already in flight during the write-out.  The Okapi weight
+// separate zeroing phase); the NEXT image's ids are already in flight during the write-out.  ZEROED (the row was
+// cleared beforehand): only the image's distinct bins are written, see write_distinct_bins.  The Okapi weight
 // depends only on (tf, dl): the weights of tf = 1..kTfTable are computed once per image by 32 threads and the
 // write-out looks them up -- with the FP64 divisions inlined in the write-out the first version was
 // instruction-bound (6.1 k warp instructions per image, 0.44 of HBM peak; profiles/r01_findings.md section 9).
@@ -78,11 +111,57 @@ __device__ __noinline__ double okapi_weight_rare(double tf, double k1, double k2
     return okapi_weight(tf, k1, k2, b, ratio);
 }
 
-template <typename OutT, bool SMEM>
+// Write-out of one image into a row that was cleared beforehand: at BoVW sizes ~97 % of a row is zeros, so writing
+// only the image's distinct bins saves nearly all of the row's bytes.  The nt threads of the group (warp or CTA)
+// walk their own ids, not the k counters.  A held id (bins[i], -1 = none) whose atomicAdd saw 0 (bit i of `first`)
+// was its bin's first hit: that thread writes the bin, and after `sync` resets its counter, so only touched counters
+// are reset.  With `whole` (k a multiple of the bins per 32-byte sector, 32-byte aligned rows) the owner writes the
+// whole aligned sector around its bin, every value taken from the final counts: a scattered 8-byte store into a row
+// that is not in L2 is a partial sector, which the memory side has to read, merge and write back.  Two owners in one
+// sector write the same bytes.  Ids past the WPT * nt held ones were re-read and kept no flags: once the held owners
+// are done, an atomicExch picks one writer for each bin still counted.
+template <int WPT, typename OutT, typename BinOf, typename Weight, typename Sync>
+__device__ __forceinline__ void write_distinct_bins(const int (&bins)[WPT], unsigned first, int* s_cnt, OutT* orow,
+                                                    bool whole, const int64_t* __restrict__ words, int64_t lo,
+                                                    int64_t hi, int t, int nt, BinOf bin_of, Weight weight, Sync sync) {
+    constexpr int G = 32 / (int)sizeof(OutT);   // bins per 32-byte sector
+#pragma unroll
+    for (int i = 0; i < WPT; ++i)
+        if (first & (1u << i)) {
+            if (whole) {
+                const int g = bins[i] & ~(G - 1);
+                auto val = [&](int u) -> double {
+                    const int c = s_cnt[g + u];
+                    return c ? weight(c) : 0.0;
+                };
+#pragma unroll
+                for (int u = 0; u < G; u += 4) store4(orow + g + u, val(u), val(u + 1), val(u + 2), val(u + 3));
+            } else {
+                orow[bins[i]] = (OutT)weight(s_cnt[bins[i]]);
+            }
+        }
+    sync();
+#pragma unroll
+    for (int i = 0; i < WPT; ++i)
+        if (first & (1u << i)) s_cnt[bins[i]] = 0;
+    if (lo + WPT * nt < hi) {
+        sync();
+        for (int64_t j = lo + t + WPT * nt; j < hi; j += nt) {
+            const int bin = bin_of((int)__ldg(words + j));
+            if (bin >= 0) {
+                const int c = atomicExch(&s_cnt[bin], 0);
+                if (c) orow[bin] = (OutT)weight(c);
+            }
+        }
+    }
+}
+
+template <typename OutT, bool SMEM, bool ZEROED>
 __global__ void __launch_bounds__(kThreads, 8)
 histogram_kernel(const int64_t* __restrict__ words, const int64_t* __restrict__ off, int64_t n_img, int k, int mode,
                  OutT* __restrict__ out, int okapi, double k1, double k2, double b, double avgdl_in) {
-    constexpr int WPT = 4;                       // ids held in registers per thread (covers 1024 per image)
+    static_assert(SMEM || !ZEROED, "without shared-memory counters the counts are added into the cleared row itself");
+    constexpr int WPT = 4;                       // ids held in registers per thread (covers 512 per image)
     extern __shared__ int s_cnt[];
     __shared__ int s_mn, s_mx;
     __shared__ double s_w[kTfTable + 1];
@@ -106,6 +185,7 @@ histogram_kernel(const int64_t* __restrict__ words, const int64_t* __restrict__ 
     if (blockIdx.x < n_img) fetch(blockIdx.x);
     __syncthreads();
     const bool vec_ok = (k % 4 == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
+    const bool whole = ZEROED && k % (32 / (int)sizeof(OutT)) == 0 && (reinterpret_cast<uintptr_t>(out) & 31) == 0;
     for (int64_t img = blockIdx.x; img < n_img; img += gridDim.x) {
         const int64_t cnt = hi - lo;
         OutT* orow = out + img * (int64_t)k;
@@ -129,19 +209,31 @@ histogram_kernel(const int64_t* __restrict__ words, const int64_t* __restrict__ 
             __syncthreads();
             nb.setup(s_mn, s_mx, k);
         }
-        auto count = [&](int v) {
+        auto bin_of = [&](int v) -> int {
             int bin;
             if (mode == ISE_HIST_NUMPY_COMPAT) bin = nb.bin(v);
             else bin = (v >= 0 && v < k) ? v : -1;
-            if (bin >= 0 && bin < k) {
-                if (SMEM) atomicAdd(&s_cnt[bin], 1);
-                else atomicAdd(orow + bin, (OutT)1);  // row was zeroed by the caller's memset
-            }
+            return bin >= 0 && bin < k ? bin : -1;
         };
+        auto count = [&](int bin) {
+            if (SMEM) atomicAdd(&s_cnt[bin], 1);
+            else atomicAdd(orow + bin, (OutT)1);  // row was zeroed beforehand (memset or the caller's clear)
+        };
+        int bins[WPT];
+        unsigned first = 0;    // ZEROED: bit i = bins[i] saw its first hit here
 #pragma unroll
-        for (int i = 0; i < WPT; ++i)
-            if (lo + threadIdx.x + i * kThreads < hi) count(w[i]);
-        for (int64_t j = lo + threadIdx.x + WPT * kThreads; j < hi; j += kThreads) count((int)words[j]);
+        for (int i = 0; i < WPT; ++i) {
+            bins[i] = lo + threadIdx.x + i * kThreads < hi ? bin_of(w[i]) : -1;
+            if (bins[i] >= 0) {
+                if (ZEROED) first |= atomicAdd(&s_cnt[bins[i]], 1) == 0 ? 1u << i : 0u;
+                else count(bins[i]);
+            }
+        }
+        for (int64_t j = lo + threadIdx.x + WPT * kThreads; j < hi; j += kThreads) {
+            const int bin = bin_of((int)words[j]);
+            if (bin >= 0) count(bin);
+        }
+        const int64_t img_lo = lo, img_hi = hi;   // fetch() moves lo / hi on to the next image
         // ids of the next image: in flight while this row is written
         if (img + gridDim.x < n_img) fetch(img + gridDim.x);
         __syncthreads();
@@ -151,7 +243,10 @@ histogram_kernel(const int64_t* __restrict__ words, const int64_t* __restrict__ 
             if (c <= kTfTable) return s_w[c];
             return okapi_weight_rare((double)c, k1, k2, b, ratio);
         };
-        if (SMEM) {
+        if (ZEROED) {
+            write_distinct_bins<WPT>(bins, first, s_cnt, orow, whole, words, img_lo, img_hi, threadIdx.x, kThreads,
+                                     bin_of, weight, [] { __syncthreads(); });
+        } else if (SMEM) {
             if (vec_ok) {
                 for (int j = threadIdx.x * 4; j < k; j += kThreads * 4) {
                     const int4 c = *reinterpret_cast<const int4*>(s_cnt + j);
@@ -193,7 +288,7 @@ histogram_kernel(const int64_t* __restrict__ words, const int64_t* __restrict__ 
 constexpr int kWarpHistWarps = 4;          // warps per CTA; k * 4 B of counters each
 constexpr int kWarpHistMaxBins = 4096;
 
-template <typename OutT>
+template <typename OutT, bool ZEROED>
 __global__ void __launch_bounds__(kWarpHistWarps * 32)
 histogram_warp_kernel(const int64_t* __restrict__ words, const int64_t* __restrict__ off, int64_t n_img, int k, int mode,
                       OutT* __restrict__ out, int okapi, double k1, double k2, double b, double avgdl_in) {
@@ -207,6 +302,7 @@ histogram_warp_kernel(const int64_t* __restrict__ words, const int64_t* __restri
     for (int j = lane; j < k; j += 32) s_cnt[j] = 0;
     __syncwarp();
     const bool vec_ok = (k % 4 == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
+    const bool whole = ZEROED && k % (32 / (int)sizeof(OutT)) == 0 && (reinterpret_cast<uintptr_t>(out) & 31) == 0;
     const int64_t warp = (int64_t)blockIdx.x * kWarpHistWarps + wib, nwarps = (int64_t)gridDim.x * kWarpHistWarps;
     for (int64_t img = warp; img < n_img; img += nwarps) {
         const int64_t lo = __ldg(off + img), hi = __ldg(off + img + 1);
@@ -235,23 +331,36 @@ histogram_warp_kernel(const int64_t* __restrict__ words, const int64_t* __restri
             mx = __reduce_max_sync(0xffffffffu, mx);
             nb.setup(mn, mx, k);
         }
-        auto count = [&](int v) {
+        auto bin_of = [&](int v) -> int {
             int bin;
             if (mode == ISE_HIST_NUMPY_COMPAT) bin = nb.bin(v);
             else bin = (v >= 0 && v < k) ? v : -1;
-            if (bin >= 0 && bin < k) atomicAdd(&s_cnt[bin], 1);
+            return bin >= 0 && bin < k ? bin : -1;
         };
+        int bins[WPT];
+        unsigned first = 0;    // ZEROED: bit i = bins[i] saw its first hit here
 #pragma unroll
-        for (int i = 0; i < WPT; ++i)
-            if (lo + lane + i * 32 < hi) count(w[i]);
-        for (int64_t j = lo + lane + WPT * 32; j < hi; j += 32) count((int)__ldg(words + j));
+        for (int i = 0; i < WPT; ++i) {
+            bins[i] = lo + lane + i * 32 < hi ? bin_of(w[i]) : -1;
+            if (bins[i] >= 0) {
+                if (ZEROED) first |= atomicAdd(&s_cnt[bins[i]], 1) == 0 ? 1u << i : 0u;
+                else atomicAdd(&s_cnt[bins[i]], 1);
+            }
+        }
+        for (int64_t j = lo + lane + WPT * 32; j < hi; j += 32) {
+            const int bin = bin_of((int)__ldg(words + j));
+            if (bin >= 0) atomicAdd(&s_cnt[bin], 1);
+        }
         __syncwarp();
         auto weight = [&](int c) -> double {
             if (!okapi) return (double)c;
             if (c <= kTfTable) return s_w[c];
             return okapi_weight_rare((double)c, k1, k2, b, ratio);
         };
-        if (vec_ok) {
+        if (ZEROED) {
+            write_distinct_bins<WPT>(bins, first, s_cnt, orow, whole, words, lo, hi, lane, 32, bin_of, weight,
+                                     [] { __syncwarp(); });
+        } else if (vec_ok) {
             for (int j = lane * 4; j < k; j += 128) {
                 const int4 c = *reinterpret_cast<const int4*>(s_cnt + j);
                 double v0 = 0.0, v1 = 0.0, v2 = 0.0, v3 = 0.0;
@@ -551,9 +660,25 @@ __global__ void tfidf_finish_kernel(T* __restrict__ h, int64_t n_img, int k, con
 
 }  // namespace
 
+ISE_EXPORT int ise_clear(ise_ctx* ctx, void* p, size_t bytes, double gb_per_s, void* stream) {
+    ISE_CHECK_ARG(ctx && gb_per_s >= 0.0);
+    if (bytes == 0) return 0;
+    ISE_CHECK_ARG(p && (reinterpret_cast<uintptr_t>(p) & 15) == 0);
+    DeviceGuard guard(ctx->device);
+    // one sweep = every thread of the grid stores 16 bytes; 1 GB/s = 1 byte per ns
+    const double sweep_bytes = (double)ctx->sm_count * kClearThreads * 16;
+    const unsigned ns_per_sweep = gb_per_s > 0.0 ? (unsigned)std::min(1e9, std::max(1.0, sweep_bytes / gb_per_s)) : 0u;
+    ISE_CUDA(cudaFuncSetAttribute(clear_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                  cudaSharedmemCarveoutMaxShared));
+    clear_kernel<<<ctx->sm_count, kClearThreads, 0, (cudaStream_t)stream>>>(
+        (uint4*)p, (int64_t)(bytes / 16), (unsigned char*)p + bytes / 16 * 16, (int)(bytes % 16), ns_per_sweep);
+    ISE_LAUNCH_CHECK();
+    return 0;
+}
+
 ISE_EXPORT int ise_bovw_histogram(ise_ctx* ctx, const int64_t* words, int64_t n_words, const int64_t* img_offsets,
                                   int64_t n_img, int k, int mode, int out_dtype, void* out, int okapi, double k1,
-                                  double k2, double b, double avgdl, void* stream) {
+                                  double k2, double b, double avgdl, int zeroed, void* stream) {
     ISE_CHECK_ARG(ctx && n_img >= 0 && k >= 1);   // ids are handled as int32 (k is an int)
     ISE_CHECK_ARG(mode == ISE_HIST_NUMPY_COMPAT || mode == ISE_HIST_BINCOUNT);
     ISE_CHECK_ARG(out_dtype == ISE_OUT_F32 || out_dtype == ISE_OUT_F64);
@@ -572,34 +697,25 @@ ISE_EXPORT int ise_bovw_histogram(ise_ctx* ctx, const int64_t* words, int64_t n_
         const size_t shm_w = (size_t)kWarpHistWarps * k * sizeof(int);
         const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(16, (200 * 1024) / (shm_w + 2048)));
         const int grid_w = (int)std::min<int64_t>(ceil_div64(n_img, kWarpHistWarps), (int64_t)ctx->sm_count * per_sm);
-        if (out_dtype == ISE_OUT_F64) {
-            auto kern = histogram_warp_kernel<double>;
-            ISE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shm_w));
-            kern<<<grid_w, kWarpHistWarps * 32, shm_w, st>>>(words, img_offsets, n_img, k, mode, (double*)out, okapi, k1,
-                                                            k2, b, avgdl);
-        } else {
-            auto kern = histogram_warp_kernel<float>;
-            ISE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shm_w));
-            kern<<<grid_w, kWarpHistWarps * 32, shm_w, st>>>(words, img_offsets, n_img, k, mode, (float*)out, okapi, k1,
-                                                            k2, b, avgdl);
-        }
+        auto kern = zeroed ? histogram_warp_kernel<double, true> : histogram_warp_kernel<double, false>;
+        ISE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shm_w));
+        kern<<<grid_w, kWarpHistWarps * 32, shm_w, st>>>(words, img_offsets, n_img, k, mode, (double*)out, okapi, k1,
+                                                        k2, b, avgdl);
         ISE_LAUNCH_CHECK();
         return 0;
     }
     const int grid = (int)std::min<int64_t>(n_img, (int64_t)ctx->sm_count * 16);
     const size_t elt = out_dtype == ISE_OUT_F64 ? 8 : 4;
-    if (!smem) ISE_CUDA(cudaMemsetAsync(out, 0, (size_t)n_img * k * elt, st));
+    if (!smem && !zeroed) ISE_CUDA(cudaMemsetAsync(out, 0, (size_t)n_img * k * elt, st));
     const size_t shm = smem ? (size_t)k * sizeof(int) : 0;
     if (out_dtype == ISE_OUT_F64) {
-        if (smem) histogram_kernel<double, true><<<grid, kThreads, shm, st>>>(words, img_offsets, n_img, k, mode,
-                                                                              (double*)out, okapi, k1, k2, b, avgdl);
-        else histogram_kernel<double, false><<<grid, kThreads, 0, st>>>(words, img_offsets, n_img, k, mode,
-                                                                        (double*)out, okapi, k1, k2, b, avgdl);
+        auto kern = !smem ? histogram_kernel<double, false, false>
+                          : zeroed ? histogram_kernel<double, true, true> : histogram_kernel<double, true, false>;
+        kern<<<grid, kThreads, shm, st>>>(words, img_offsets, n_img, k, mode, (double*)out, okapi, k1, k2, b, avgdl);
     } else {
-        if (smem) histogram_kernel<float, true><<<grid, kThreads, shm, st>>>(words, img_offsets, n_img, k, mode,
-                                                                             (float*)out, okapi, k1, k2, b, avgdl);
-        else histogram_kernel<float, false><<<grid, kThreads, 0, st>>>(words, img_offsets, n_img, k, mode,
-                                                                       (float*)out, okapi, k1, k2, b, avgdl);
+        auto kern = !smem ? histogram_kernel<float, false, false>
+                          : zeroed ? histogram_kernel<float, true, true> : histogram_kernel<float, true, false>;
+        kern<<<grid, kThreads, shm, st>>>(words, img_offsets, n_img, k, mode, (float*)out, okapi, k1, k2, b, avgdl);
     }
     ISE_LAUNCH_CHECK();
     return 0;

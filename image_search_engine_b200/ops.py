@@ -1210,7 +1210,9 @@ def kmeans_apply_splits(centroids: torch.Tensor, pairs: torch.Tensor):
 # ------------------------------------------------------------------------------------------
 def bovw_histogram(words: torch.Tensor, img_offsets: torch.Tensor, k: int, *, mode: int = HIST_NUMPY_COMPAT,
                    out_dtype: torch.dtype = torch.float64, okapi: bool = False, k1: float = 1.0, k2: float = 1.0,
-                   b: float = 0.75, avgdl: float = -1.0, out: torch.Tensor | None = None) -> torch.Tensor:
+                   b: float = 0.75, avgdl: float = -1.0, out: torch.Tensor | None = None,
+                   zeroed: bool = False) -> torch.Tensor:
+    """``zeroed=True``: ``out`` is already all zeros (``clear_``) and only the non-zero bins are written."""
     if words.dtype != torch.int64 or img_offsets.dtype != torch.int64:
         raise IseError("bovw_histogram: words and img_offsets must be int64")
     words = words.reshape(-1).contiguous()
@@ -1219,14 +1221,27 @@ def bovw_histogram(words: torch.Tensor, img_offsets: torch.Tensor, k: int, *, mo
     if out_dtype not in (torch.float32, torch.float64):
         raise IseError("bovw_histogram: float32 or float64 output")
     if out is None:
+        if zeroed:
+            raise IseError("bovw_histogram: zeroed=True needs a cleared out=")
         out = torch.empty((n_img, k), dtype=out_dtype, device=words.device)
     elif tuple(out.shape) != (n_img, k) or out.dtype != out_dtype or not out.is_contiguous():
         raise IseError("bovw_histogram: out must be a contiguous [n_img, k] tensor of out_dtype")
     _lib.check(_lib.load().ise_bovw_histogram(
         _lib.ctx(_dev(img_offsets)), _ptr(words), int(words.numel()), _ptr(img_offsets), n_img, int(k), int(mode), od,
-        _ptr(out), 1 if okapi else 0, float(k1), float(k2), float(b), float(avgdl), _stream()))
+        _ptr(out), 1 if okapi else 0, float(k1), float(k2), float(b), float(avgdl), 1 if zeroed else 0, _stream()))
     _count()
     return out
+
+
+def clear_(t: torch.Tensor, gb_per_s: float = 0.0) -> torch.Tensor:
+    """Zero-fills a contiguous CUDA tensor in place with the project's clear kernel (one 128-thread block per SM, sized
+    to run beside the assign kernel on another stream); ``gb_per_s`` > 0 paces the stores to about that rate."""
+    if not t.is_contiguous():
+        raise IseError("clear_: contiguous tensor expected")
+    _lib.check(_lib.load().ise_clear(_lib.ctx(_dev(t)), _ptr(t), t.numel() * t.element_size(), float(gb_per_s),
+                                      _stream()))
+    _count()
+    return t
 
 
 def bovw_histogram_csr(words: torch.Tensor, img_offsets: torch.Tensor, k: int, *, mode: int = HIST_NUMPY_COMPAT,

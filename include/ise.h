@@ -337,10 +337,16 @@ int ise_kmeans_apply_splits(ise_ctx* ctx, float* centroids, int64_t k, int d,
  * okapi != 0 fuses OkapiTransformer.transform: tf*k1/(tf*k1 + k2*(1-b+b*dl/avgdl)) with
  * dl = row sum, avgdl = mean dl over this batch when the argument is < 0, else the given value (a batch
  * fed in several launches passes the whole batch's mean); zeros stay zero.  n_words = length of words[] (its
- * ratio to n_img picks the warp-per-image kernel for short images); 0 = unknown. */
+ * ratio to n_img picks the warp-per-image kernel for short images); 0 = unknown.  zeroed != 0: out is already all
+ * zeros (e.g. from ise_clear) and only each image's non-zero bins are written; zeroed = 0 writes every cell. */
 int ise_bovw_histogram(ise_ctx* ctx, const int64_t* words, int64_t n_words, const int64_t* img_offsets, int64_t n_img,
                        int k, int mode, int out_dtype, void* out,
-                       int okapi, double k1, double k2, double b, double avgdl, void* stream);
+                       int okapi, double k1, double k2, double b, double avgdl, int zeroed, void* stream);
+/* zero-fill bytes at p (device, 16-byte aligned) with one small CTA per SM, sized to run beside the assign kernel on
+ * another stream: clears a histogram matrix for ise_bovw_histogram(..., zeroed = 1) while the ids are computed.
+ * gb_per_s > 0 paces the stores to about that rate (the assign slows down under a concurrent full-rate HBM stream);
+ * 0 = as fast as the stores go. */
+int ise_clear(ise_ctx* ctx, void* p, size_t bytes, double gb_per_s, void* stream);
 /* Same histogram (+ fused Okapi), as a CSR matrix with sorted column indices -- what
  * OkapiTransformer.transform returns (scipy CSR, utils.py:153-202) and what
  * `pipeline.transform(...)` hands to its caller (engine.py:96, bag_of_visual_words.py:181-183): the dense
