@@ -105,6 +105,16 @@ PROTOTYPES = {
     "ise_ivfpq_residual": (_int, [_c_void_p, _c_void_p, _i64, _i64, _int, _c_void_p, _c_void_p, _c_void_p, _c_void_p]),
     "ise_ivfpq_scan": (_int, [_c_void_p, _c_void_p, _i64, _int, _c_void_p, _i64, _c_void_p, _int, _c_void_p, _int, _int,
                               _c_void_p, _c_void_p, _i64, _c_void_p, _c_void_p]),
+    "ise_ivfpq_search_workspace_bytes": (_size, [_c_void_p, _i64, _int, _i64, _i64, _int, _int, _int]),
+    "ise_ivfpq_search": (_int, [_c_void_p, _c_void_p, _i64, _int, _c_void_p, _i64, _c_void_p, _int, _int, _c_void_p,
+                                _c_void_p, _c_void_p, _i64, _c_void_p, _int, _int, _c_void_p, _c_void_p, _c_void_p,
+                                _size, _c_void_p]),
+    "ise_ivfpq_range_workspace_bytes": (_size, [_c_void_p, _i64, _int, _i64, _i64, _int, _int]),
+    "ise_ivfpq_range_count": (_int, [_c_void_p, _c_void_p, _i64, _int, _c_void_p, _i64, _c_void_p, _int, _int,
+                                     _c_void_p, _c_void_p, _c_void_p, _i64, _c_void_p, _int, C.c_float, _c_void_p,
+                                     _c_void_p, _size, _c_void_p]),
+    "ise_ivfpq_range_fill": (_int, [_c_void_p, _i64, _int, _i64, _int, _int, _c_void_p, _c_void_p, _c_void_p, _i64,
+                                    _int, C.c_float, _c_void_p, _c_void_p, _c_void_p, _size, _c_void_p]),
     "ise_ivfflat_search_workspace_bytes": (_size, [_c_void_p, _i64, _int, _i64, _i64, _int]),
     "ise_ivfflat_search": (_int, [_c_void_p, _c_void_p, _i64, _int, _c_void_p, _c_void_p, _c_void_p, _i64, _i64,
                                   _c_void_p, _int, _int, _int, _c_void_p, _c_void_p, _c_void_p, _size, _c_void_p]),

@@ -1,4 +1,4 @@
-// The (query, probe) grouping of the IVF scans (ivfflat.cu, binary.cu): the nq * nprobe pairs sorted by list, work
+// The (query, probe) grouping of the IVF scans (ivfflat.cu, binary.cu, ivfpq.cu): the nq * nprobe pairs sorted by list, work
 // items (list, block of <= qb of its queries, chunk of its rows) taken by persistent CTAs from a device counter, and the
 // merge levels of the partial lists.
 //
@@ -222,14 +222,20 @@ static int group_pairs(ise_ctx* ctx, const Plan& p, const Grouping& g, const int
     return 0;
 }
 
-// persistent CTAs (as many as fit) that take work items from the counter: the item count stays on the device
+// persistent CTAs (as many as fit with shm bytes of dynamic shared memory each) that take work items from the counter:
+// the item count stays on the device
 template <typename Kernel, typename... Args>
-static int launch_persistent(ise_ctx* ctx, cudaStream_t st, Kernel kernel, Args... args) {
+static int launch_persistent_shm(ise_ctx* ctx, cudaStream_t st, size_t shm, Kernel kernel, Args... args) {
     int per_sm = 0;
-    ISE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, 0));
-    kernel<<<ctx->sm_count * std::max(per_sm, 1), kThreads, 0, st>>>(args...);
+    ISE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, shm));
+    kernel<<<ctx->sm_count * std::max(per_sm, 1), kThreads, shm, st>>>(args...);
     ISE_LAUNCH_CHECK();
     return 0;
+}
+
+template <typename Kernel, typename... Args>
+static int launch_persistent(ise_ctx* ctx, cudaStream_t st, Kernel kernel, Args... args) {
+    return launch_persistent_shm(ctx, st, 0, kernel, args...);
 }
 
 // merges the nprobe * S partial lists of every query (part_*, list-major [g][nq][topk]) into out_*, at most kMergeFanIn

@@ -216,9 +216,13 @@ class IndexIVFPQ:
     Training is the hot path's own machinery: level-1 clustering (nlist centroids, niter = 10) and one k-means
     per sub-quantizer (256 centroids on d/M-dimensional residual slices, niter = 25, seed 1234, at most 65 536
     training rows) run on the tensor-core assign + update kernels; vectors are encoded with the fused top-1
-    assign; search probes the ``nprobe`` nearest lists and scans their codes with a shared-memory look-up table
-    (``ise_ivfpq_scan``) followed by the canonical top-k selection.  Approximate by construction (8-bit codes):
-    returned distances are sum_m |(q - c_list)_m - pq_m[code_m]|^2 like Faiss's.
+    assign; search probes the ``nprobe`` nearest lists and scans only their codes: the (query, probe) pairs are
+    grouped by list, each pair gets one look-up table, and the partial top-k lists are merged (``ise_ivfpq_search``),
+    so time and memory follow the probed lists.  For k > 128 (or M * ksub > 8192) the search scans into a
+    [min(nq, 4096), ntotal] distance matrix (``ise_ivfpq_scan``) followed by the top-k selection instead.  Both return
+    the same distances, sum_m |(q - c_list)_m - pq_m[code_m]|^2 like Faiss's; approximate by construction (8-bit
+    codes).  Results are in the canonical (distance, id) order: among equal distances the lowest ids win.
+    ``range_search`` filters the same lists by a radius (``ise_ivfpq_range_count`` / ``_fill``) in Faiss's probe order.
     """
 
     def __init__(self, quantizer, d, nlist, M, nbits_per_idx, metric=METRIC_L2):
@@ -312,14 +316,23 @@ class IndexIVFPQ:
             self._sorted = None
 
     def _lists(self):
+        """(codes, ids, list offsets, host list sizes): the codes grouped by list, rebuilt after add / reset."""
         with self._lock:
             if self._sorted is None:
-                order = torch.argsort(self._assign, stable=True)           # lists keep insertion order
+                order = torch.argsort(self._assign, stable=True)           # lists keep insertion order (= ascending id)
                 counts = torch.bincount(self._assign, minlength=self.nlist)
                 off = torch.zeros((self.nlist + 1,), dtype=torch.int64, device=counts.device)
                 off[1:] = torch.cumsum(counts, 0)
-                self._sorted = (self._codes.index_select(0, order).contiguous(), self._ids.index_select(0, order), off)
+                self._sorted = (self._codes.index_select(0, order).contiguous(), self._ids.index_select(0, order), off,
+                                counts.cpu().numpy())
             return self._sorted
+
+    def _probes(self, q: torch.Tensor) -> torch.Tensor:
+        return self.quantizer._search_device(q, min(self.nprobe, self.nlist), need_distances=False)[1]
+
+    def _grouped(self, k: int) -> bool:
+        """search scans the probed lists grouped by list; otherwise into a dense [min(nq, 4096), ntotal] matrix"""
+        return k <= ops.MAX_TOPK and self.M * self.ksub <= ops.IVFPQ_MAX_TABLE
 
     def search(self, x, k: int):
         k = int(k)
@@ -330,10 +343,16 @@ class IndexIVFPQ:
         if q.shape[1] != self.d:
             raise AssertionError(f"search: expected (n, {self.d}) array")
         nq = q.shape[0]
-        D, I = ops.topk_padding(nq, k, METRIC_L2, q.device)
-        if nq and self.ntotal:
-            codes, ids, off = self._lists()
-            _, probes = self.quantizer._search_device(q, min(self.nprobe, self.nlist), need_distances=False)
+        if not (nq and self.ntotal):
+            D, I = ops.topk_padding(nq, k, METRIC_L2, q.device)
+        elif self._grouped(k):
+            codes, ids, off, sizes = self._lists()
+            D, I = ops.ivfpq_search(q.contiguous(), self.quantizer._database(), self.pq_centroids, codes, ids, off,
+                                    int(sizes.max()), self._probes(q), k)
+        else:
+            D, I = ops.topk_padding(nq, k, METRIC_L2, q.device)
+            codes, ids, off, _ = self._lists()
+            probes = self._probes(q)
             for q0 in range(0, nq, 4096):                                  # bounds the [nq, ntotal] distance matrix
                 qs = q[q0:q0 + 4096].contiguous()
                 dist = ops.ivfpq_scan(qs, self.quantizer._database(), probes[q0:q0 + 4096], self.pq_centroids, codes, off)
@@ -344,6 +363,41 @@ class IndexIVFPQ:
         if was_cuda:
             return D, I
         return D.cpu().numpy(), I.cpu().numpy()
+
+    def range_search(self, x, radius: float):
+        """IndexIVF::range_search: probe min(nprobe, nlist) lists as ``search`` does and return every stored code of
+        them whose distance (the one ``search`` returns) is below ``radius``: strict, radius cast to float32.  Returns
+        (lims [nq + 1], D, I); the results of query i are D[lims[i]:lims[i+1]] / I[...] in Faiss's scan order: by probe
+        rank (nearest list first), then by position in the list (ids ascend inside a list).  NumPy input gives NumPy
+        output (lims uint64); CUDA tensors give CUDA tensors (lims int64).  An untrained or empty index returns no
+        results."""
+        radius = float(radius)
+        q, was_cuda = _to_device(x)
+        if q.shape[1] != self.d:
+            raise AssertionError(f"range_search: expected (n, {self.d}) array")
+        q = q.to(torch.float32).contiguous()
+        nq = q.shape[0]
+        if nq and self.ntotal and self.is_trained:
+            codes, ids, off, sizes = self._lists()
+            lims, D, I = ops.ivfpq_range_search(q, self.quantizer._database(), self.pq_centroids, codes, ids, off,
+                                                int(sizes.max()), self._probes(q), radius)
+        else:
+            lims, D, I = ops.range_empty(nq, q.device)
+        if was_cuda:
+            return lims, D, I
+        return lims.cpu().numpy().astype(np.uint64), D.cpu().numpy(), I.cpu().numpy()
+
+    def get_list_size(self, list_no: int) -> int:
+        sizes = self._lists()[3] if self.ntotal else np.zeros(self.nlist, np.int64)
+        return int(sizes[int(list_no)])
+
+    def get_list_ids(self, list_no: int) -> np.ndarray:
+        """Ids stored in one list, in list order (InvertedLists::get_ids)."""
+        if not self.ntotal:
+            return np.zeros(0, np.int64)
+        _, ids, off, _ = self._lists()
+        l = int(list_no)
+        return ids[int(off[l]):int(off[l + 1])].cpu().numpy()
 
     def reset(self) -> None:
         with self._lock:

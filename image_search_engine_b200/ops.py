@@ -871,6 +871,130 @@ def ivfpq_scan(q: torch.Tensor, coarse: torch.Tensor, probes: torch.Tensor, pq_c
     return dist
 
 
+IVFPQ_MAX_TABLE = 8192          # M * ksub: a work item of ise_ivfpq_search stages four look-up tables in shared memory
+# bytes of look-up tables (4 * M * ksub per query and probe) one ise_ivfpq_* call may build: ivfpq_search and
+# ivfpq_range_search split the queries into batches that stay below it
+IVFPQ_LUT_BUDGET = 1 << 30
+
+
+def ivfpq_batch(nprobe: int, M: int, ksub: int) -> int:
+    """Queries per ise_ivfpq_* call: as many as keep their tables within IVFPQ_LUT_BUDGET (at least one)."""
+    return max(1, IVFPQ_LUT_BUDGET // (4 * int(nprobe) * int(M) * int(ksub)))
+
+
+def ivfpq_search_workspace_bytes(nq: int, nprobe: int, nlist: int, max_list_len: int, M: int, ksub: int,
+                                 topk: int) -> int:
+    """Device scratch of one ise_ivfpq_search call over nq queries (the formula is in include/ise.h)."""
+    return int(_lib.load().ise_ivfpq_search_workspace_bytes(_lib.ctx(torch.cuda.current_device()), int(nq), int(nprobe),
+                                                              int(nlist), int(max_list_len), int(M), int(ksub),
+                                                              int(topk)))
+
+
+def ivfpq_range_workspace_bytes(nq: int, nprobe: int, nlist: int, max_list_len: int, M: int, ksub: int) -> int:
+    """Device scratch of one ise_ivfpq_range_count / _fill pair over nq queries (the formula is in include/ise.h)."""
+    return int(_lib.load().ise_ivfpq_range_workspace_bytes(_lib.ctx(torch.cuda.current_device()), int(nq), int(nprobe),
+                                                             int(nlist), int(max_list_len), int(M), int(ksub)))
+
+
+def _ivfpq_args(name: str, q, coarse, pq_centroids, codes, ids, list_off, probes):
+    if q.dtype != torch.float32 or coarse.dtype != torch.float32 or pq_centroids.dtype != torch.float32:
+        raise IseError(f"{name}: float32 queries and centroids")
+    if codes.dtype != torch.uint8 or ids.dtype != torch.int64 or list_off.dtype != torch.int64 or probes.dtype != torch.int64:
+        raise IseError(f"{name}: uint8 codes; int64 ids, list offsets and probes")
+    nq, d = q.shape
+    M, ksub, dsub = pq_centroids.shape
+    if (M * dsub != d or coarse.dim() != 2 or coarse.shape[1] != d or codes.dim() != 2 or codes.shape[1] != M
+            or ids.shape[0] != codes.shape[0] or probes.shape[0] != nq or list_off.shape[0] != coarse.shape[0] + 1):
+        raise IseError(f"{name}: inconsistent shapes")
+    if M * ksub > IVFPQ_MAX_TABLE:
+        raise IseError(f"{name}: M * ksub must be at most {IVFPQ_MAX_TABLE}")
+    return (q.contiguous(), coarse.contiguous(), pq_centroids.contiguous(), codes.contiguous(), ids.contiguous(),
+            list_off.contiguous(), probes.contiguous())
+
+
+def _ivfpq_batches(nq: int, nprobe: int, M: int, ksub: int):
+    nb = ivfpq_batch(nprobe, M, ksub)
+    return [(q0, min(nb, nq - q0)) for q0 in range(0, nq, nb)]
+
+
+def ivfpq_search(q: torch.Tensor, coarse: torch.Tensor, pq_centroids: torch.Tensor, codes: torch.Tensor,
+                 ids: torch.Tensor, list_off: torch.Tensor, max_list_len: int, probes: torch.Tensor, topk: int):
+    """L2 top-k of every query over the PQ codes of its probed lists (IndexIVFPQ.search, by_residual) without an
+    [nq, ntotal] matrix: codes [ntotal, M] uint8 / ids grouped by list (list l = rows list_off[l] .. list_off[l + 1],
+    ids ascending inside a list), pq_centroids [M, ksub, d / M], probes [nq, nprobe] int64.  Distances have the bits of
+    ivfpq_scan's; the order is the canonical (distance, id), padded with id -1 / FLT_MAX.  The queries go in batches of
+    ivfpq_batch(nprobe, M, ksub), which bounds the look-up tables."""
+    if not 1 <= topk <= MAX_TOPK:
+        raise IseError(f"topk must be in [1, {MAX_TOPK}]")
+    q, coarse, pq_centroids, codes, ids, list_off, probes = _ivfpq_args("ivfpq_search", q, coarse, pq_centroids, codes,
+                                                                        ids, list_off, probes)
+    nq, d = q.shape
+    M, ksub, _ = pq_centroids.shape
+    nprobe, nlist = probes.shape[1], coarse.shape[0]
+    val = torch.empty((nq, topk), dtype=torch.float32, device=q.device)
+    idx = torch.empty((nq, topk), dtype=torch.int64, device=q.device)
+    if nq == 0:
+        return val, idx
+    lib, ctx = _lib.load(), _lib.ctx(_dev(q))
+    batches = _ivfpq_batches(nq, nprobe, M, ksub)
+    ws_bytes = max(lib.ise_ivfpq_search_workspace_bytes(ctx, n, nprobe, nlist, int(max_list_len), M, ksub, int(topk))
+                   for n in {batches[0][1], batches[-1][1]})
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=q.device)
+    for q0, n in batches:
+        _lib.check(lib.ise_ivfpq_search(ctx, _ptr(q[q0:]), n, d, _ptr(coarse), nlist, _ptr(pq_centroids), M, ksub,
+                                        _ptr(codes), _ptr(ids), _ptr(list_off), int(max_list_len), _ptr(probes[q0:]),
+                                        nprobe, int(topk), _ptr(val[q0:]), _ptr(idx[q0:]), _ptr(ws), ws_bytes,
+                                        _stream()))
+        _count(7)
+    return val, idx
+
+
+def ivfpq_range_search(q: torch.Tensor, coarse: torch.Tensor, pq_centroids: torch.Tensor, codes: torch.Tensor,
+                       ids: torch.Tensor, list_off: torch.Tensor, max_list_len: int, probes: torch.Tensor,
+                       radius: float):
+    """Every code of a query's probed lists with dis < radius (IndexIVFPQ.range_search; strict, radius cast to
+    float32), with the distances ivfpq_search returns.  Inputs as ivfpq_search.  Returns (lims int64 [nq + 1],
+    D float32, I int64) on the device; the results of query i are D / I[lims[i]:lims[i+1]] in probe rank order, then
+    list order (Faiss's order).  One readback per batch of ivfpq_batch(nprobe, M, ksub) queries: its total."""
+    q, coarse, pq_centroids, codes, ids, list_off, probes = _ivfpq_args("ivfpq_range_search", q, coarse, pq_centroids,
+                                                                        codes, ids, list_off, probes)
+    nq, d = q.shape
+    M, ksub, _ = pq_centroids.shape
+    nprobe, nlist = probes.shape[1], coarse.shape[0]
+    radius = float(np.float32(radius))
+    if nq == 0:
+        last_search_stats.update(mode="ivfpq-range", rows=0, pairs=0, results=0, fallback_rows=0)
+        return range_empty(0, q.device)
+    lib, ctx = _lib.load(), _lib.ctx(_dev(q))
+    batches = _ivfpq_batches(nq, nprobe, M, ksub)
+    ws_bytes = max(lib.ise_ivfpq_range_workspace_bytes(ctx, n, nprobe, nlist, int(max_list_len), M, ksub)
+                   for n in {batches[0][1], batches[-1][1]})
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=q.device)
+    lims = torch.empty((nq + 1,), dtype=torch.int64, device=q.device)
+    Ds, Is, base = [], [], 0
+    for q0, n in batches:
+        _lib.check(lib.ise_ivfpq_range_count(ctx, _ptr(q[q0:]), n, d, _ptr(coarse), nlist, _ptr(pq_centroids), M, ksub,
+                                             _ptr(codes), _ptr(ids), _ptr(list_off), int(max_list_len),
+                                             _ptr(probes[q0:]), nprobe, radius, _ptr(lims[q0:]), _ptr(ws), ws_bytes,
+                                             _stream()))
+        total = int(lims[q0 + n].item())                  # the batch's readback: sizes its D / I
+        D = torch.empty((total,), dtype=torch.float32, device=q.device)
+        I = torch.empty((total,), dtype=torch.int64, device=q.device)
+        if total:
+            _lib.check(lib.ise_ivfpq_range_fill(ctx, n, d, nlist, M, ksub, _ptr(codes), _ptr(ids), _ptr(list_off),
+                                                int(max_list_len), nprobe, radius, _ptr(D), _ptr(I), _ptr(ws),
+                                                ws_bytes, _stream()))
+        _count(10 if total else 9)
+        if base:
+            lims[q0:q0 + n + 1] += base                   # count wrote the batch's offsets from 0
+        Ds.append(D)
+        Is.append(I)
+        base += total
+    D, I = (Ds[0], Is[0]) if len(Ds) == 1 else (torch.cat(Ds), torch.cat(Is))
+    last_search_stats.update(mode="ivfpq-range", rows=nq, pairs=nq * nprobe, results=base, fallback_rows=0)
+    return lims, D, I
+
+
 # ------------------------------------------------------------------------------------------
 # IVFFlat
 # ------------------------------------------------------------------------------------------

@@ -391,6 +391,51 @@ int ise_ivfpq_residual(ise_ctx* ctx, const float* x, int64_t ldx, int64_t n, int
 int ise_ivfpq_scan(ise_ctx* ctx, const float* q, int64_t nq, int d, const float* coarse_centroids, int64_t nlist,
                    const int64_t* probes, int nprobe, const float* pq_centroids, int M, int ksub,
                    const uint8_t* codes, const int64_t* list_offsets, int64_t ntotal, float* dist, void* stream);
+/* L2 top-k over the codes of the probed lists without an [nq, ntotal] matrix (faiss/IndexIVFPQ.cpp IVFPQScanner,
+ * by_residual, no precomputed tables).  q[nq, d] float32; coarse_centroids[nlist, d]; pq_centroids[M, ksub, d / M];
+ * codes[ntotal, M] uint8 grouped by list, list l = rows list_off[l] .. list_off[l + 1], with ids ids_sorted[]
+ * ascending inside every list; max_list_len = the longest list (host value); probes[nq, nprobe] int64 (-1 = none).
+ * Every distance has the bits of ise_ivfpq_scan's: one table entry per (pair, m, code) as one fmaf chain over
+ * j = 0 .. d/M - 1 of t = (q - c_list)[m d/M + j] - pq[m][code][j], then dis = 0; dis += tab[m][code_m] for m = 0 ..
+ * M-1.  out[nq, topk] sorted in the canonical (distance, id) order, padded with id -1 / FLT_MAX.  One table per
+ * (query, probe) pair and call; pairs grouped by list on the device and scanned in (list, block of 4 queries, chunk of
+ * codes) work items whose tables are staged in shared memory; the partial lists merged with ise_topk_merge; no host
+ * synchronisation.  Workspace (ise_ivfpq_search_workspace_bytes) is O(nq * nprobe * (topk * S + M * ksub) + nlist):
+ * 4 * nq * nprobe * M * ksub bytes of tables (callers bound them by searching the queries in batches); 12 bytes per
+ * partial-list entry for the nq * nprobe * S * topk entries, S = min(ceil(max_list_len / 1024), max(1, 256 / nprobe),
+ * max(1, 2^24 / (nq * nprobe * topk))) chunks per list, plus 1/256 of that for the merge levels; 16 bytes per
+ * (query, probe) pair and 24 per list for the grouping, and CUB's sort / scan scratch.  d % M == 0,
+ * 1 <= ksub <= 256, M * ksub <= 8192 (4 tables in shared memory), d <= 51200, topk <= 128, nq * nprobe < 2^31. */
+size_t ise_ivfpq_search_workspace_bytes(ise_ctx* ctx, int64_t nq, int nprobe, int64_t nlist, int64_t max_list_len,
+                                        int M, int ksub, int topk);
+int ise_ivfpq_search(ise_ctx* ctx, const float* q, int64_t nq, int d, const float* coarse_centroids, int64_t nlist,
+                     const float* pq_centroids, int M, int ksub, const uint8_t* codes, const int64_t* ids_sorted,
+                     const int64_t* list_off, int64_t max_list_len, const int64_t* probes, int nprobe, int topk,
+                     float* out_val, int64_t* out_idx, void* workspace, size_t workspace_bytes, void* stream);
+/* Range search over the probed lists (faiss/IndexIVF.cpp range_search_preassigned, IVFPQScanner::scan_codes_range):
+ * every code of a probed list with dis < radius (strict; the distances are bit-identical to ise_ivfpq_search's).
+ * Same inputs as ise_ivfpq_search.  Results of query i are out[lims[i] .. lims[i + 1]) in Faiss's order: probe rank
+ * (probes[i, 0] first; -1 skipped), then position inside the list (= ascending id).
+ * Two calls on the same stream with the same arguments and the same workspace, untouched in between:
+ *   ise_ivfpq_range_count  groups the pairs, builds their tables, counts the hits of every (pair, chunk) segment,
+ *                          scans them into int64 offsets and writes lims[nq + 1] (lims[nq] = total; lims[0] = 0 for
+ *                          nq == 0).  The workspace then carries the grouping, the tables and the segment offsets;
+ *   ise_ivfpq_range_fill   re-scans the work items that have hits and writes out_dis / out_ids[lims[nq]].
+ * No host synchronisation inside; the caller reads lims[nq] to size the outputs.  Workspace
+ * (ise_ivfpq_range_workspace_bytes) is O(nq * nprobe * (S + M * ksub) + nlist): 4 * nq * nprobe * M * ksub bytes of
+ * tables; 16 bytes per segment (count, offset) for the nq * nprobe * S segments, with S = min(ceil(max_list_len / 1024),
+ * max(1, 256 / nprobe), max(1, 2^22 / (nq * nprobe))) chunks per list; 16 bytes per (query, probe) pair and 24 per
+ * list for the grouping; CUB's sort / scan scratch.  Limits as ise_ivfpq_search. */
+size_t ise_ivfpq_range_workspace_bytes(ise_ctx* ctx, int64_t nq, int nprobe, int64_t nlist, int64_t max_list_len,
+                                       int M, int ksub);
+int ise_ivfpq_range_count(ise_ctx* ctx, const float* q, int64_t nq, int d, const float* coarse_centroids, int64_t nlist,
+                          const float* pq_centroids, int M, int ksub, const uint8_t* codes, const int64_t* ids_sorted,
+                          const int64_t* list_off, int64_t max_list_len, const int64_t* probes, int nprobe,
+                          float radius, int64_t* lims, void* workspace, size_t workspace_bytes, void* stream);
+int ise_ivfpq_range_fill(ise_ctx* ctx, int64_t nq, int d, int64_t nlist, int M, int ksub, const uint8_t* codes,
+                         const int64_t* ids_sorted, const int64_t* list_off, int64_t max_list_len, int nprobe,
+                         float radius, float* out_dis, int64_t* out_ids, void* workspace, size_t workspace_bytes,
+                         void* stream);
 
 /* ---- IVFFlat index (faiss/IndexIVFFlat.cpp IndexIVFFlat::search_preassigned, IVFFlatScanner) ----------------------
  * Exact FP32 top-k over the vectors of the probed inverted lists, scored with Faiss's scanner formulas (IP: sum x*y,
